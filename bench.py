@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference algorithm's CPU path (oracle port) on the host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's predictions to DIR/pred.npy
 
 Workload ("step"): cfg3 of BASELINE.json -- MixSTE s2s h36m_gt config, F=243 frames, 9 DDIM steps, flip
 test-time augmentation, 256 clips per GPU (weak scaling): one step = DDIM-sample the 256 clips and their 256
@@ -24,11 +25,13 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree, which may be read-only
 
 import torch  # noqa: E402
 
 F_FRAMES, J, S_STEPS = 243, 17, 9
 METRIC, UNIT = "denoised_pose_frames_per_s", "pose-frames/s"
+DUMP_BYTES = 60 * 2 ** 20           # --dump-outputs: keeps the files under 64 MB
 
 # BASELINE.json configs.  cfg3 is the configuration the metric is quoted on (the default, and what the driver runs);
 # the others are selectable with --config so that their lines come from the same harness (profiles/).
@@ -215,6 +218,18 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------ our arm
+def dump_outputs(out_dir, pred):
+    """Writes pred [clips, F, J, 3] as out_dir/pred.npy (float32).  Beyond DUMP_BYTES it keeps a sample of clips drawn
+    with a fixed seed, in clip order, so two builds run with the same arguments dump the same clips."""
+    import numpy as np
+    keep = DUMP_BYTES // (pred[0].numel() * 4)
+    if pred.shape[0] > keep:
+        idx = torch.randperm(pred.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        pred = pred[idx.to(pred.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pred.npy"), pred.detach().to("cpu", torch.float32).numpy())
+
+
 def run_ours(args):
     import torch.distributed as dist
     from diff3dhpe_b200 import _lib, evaluate, synthetic
@@ -333,6 +348,8 @@ def run_ours(args):
     timed_check = {"clips_resampled_alone": picks, "bit_equal": not mismatched, "mismatched": mismatched,
                    "batch_clips": n0, "tokens": n0 * F * J}
     assert not mismatched, f"timed batch disagrees with single-clip runs at clips {mismatched}"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch.cat(outs))
 
     # ---- e2e: the public API with HOST buffers: pinned x2d/gt -> device, flip, sampler (noise drawn on the device in the
     #      reference's order), un-flip/average, MPJPE, then the ONE exchange step of the sharded path -- all-gather of the
@@ -493,9 +510,15 @@ def main():
                          "units), f8c (fp16 main + e5m2 correction products, 2 units), split3 (3 fp16 passes), fp16 (1 pass, "
                          "outside the parity bar)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the predictions of the last timed step (rank 0's clips; flip-TTA merged) to DIR/pred.npy")
     ap.add_argument("--lean", action="store_true",
                     help="scaling exhibits (tools/gpu_scaling.sh): no e2e warm-up pass, per-class profile on the first batch only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the CUDA path's outputs; it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -108,6 +108,25 @@ def test_window_rule():
         evaluate.window_starts(100, 243)
 
 
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: the whole prediction tensor as float32 when it fits, otherwise the same seeded sample of
+    clips, in clip order, on every call."""
+    import numpy as np
+    monkeypatch.setattr(sys, "dont_write_bytecode", sys.dont_write_bytecode)     # importing bench sets it
+    import bench
+    pred = torch.randn(10, 3, 17, 3, generator=torch.Generator().manual_seed(0))
+    bench.dump_outputs(str(tmp_path / "all"), pred)
+    got = np.load(tmp_path / "all" / "pred.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, pred.numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4 * pred[0].numel() * 4)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), pred)
+    a, b = np.load(tmp_path / "a" / "pred.npy"), np.load(tmp_path / "b" / "pred.npy")
+    assert a.shape == (4, 3, 17, 3) and np.array_equal(a, b)
+    rows = [next(i for i in range(10) if np.array_equal(r, pred[i].numpy())) for r in a]
+    assert rows == sorted(set(rows))
+
+
 _WORKER = r'''
 import os, sys, torch, torch.distributed as dist
 sys.path.insert(0, sys.argv[1])
