@@ -15,6 +15,7 @@ LIB_PATH = Path(os.environ.get("D3D_LIB", _PKG / "libdiff3d_b200.so"))
 GEMM_TC_SPLIT3, GEMM_TC_FP16, GEMM_SIMT_FP32, GEMM_TC_F8C, GEMM_SIMT_F8C, GEMM_TC_F4C, GEMM_SIMT_F4C = 0, 1, 2, 3, 4, 5, 6
 GEMM_DEFAULT = GEMM_TC_F4C      # shipped precision mode of the drop-in modules (DESIGN.md section 2)
 ATTN_DEFAULT, ATTN_SIMT, ATTN_MMA_SYNC = 0, 1, 2
+ROWWISE_LIFT, ROWWISE_POSTNORM, ROWWISE_NORM2, ROWWISE_HEAD = 0, 1, 2, 3     # d3d_debug_rowwise
 PROF_CLASSES = ("gemm", "attn_spatial", "attn_temporal", "ln", "lift", "head_ddim")
 
 
@@ -72,6 +73,8 @@ PROTOTYPES = {
                                               C.c_int32, C.c_void_p]),
     "d3d_debug_forward_blocks": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p,
                                            C.c_void_p]),
+    "d3d_debug_rowwise": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
+                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
 }
 
 _lib = None

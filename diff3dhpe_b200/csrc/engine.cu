@@ -437,15 +437,41 @@ int compute_time_table(d3d_handle* h, const float* t_dev, int R, float* table, c
   return 0;
 }
 
+// The row-wise launches of a denoiser call with the parameters they read (shared by run_blocks and d3d_debug_rowwise).
+// tv: time table of the call ([rows][nblk][512], block 0 first) or null; tv_stride: its row stride (0 = one row for
+// every clip).
+// lift: X = fusion_layer(input) + Spatial_pos_embed + time vector of block 0;  A = norm1 of block 0 (X)
+int lift_launch(d3d_handle* h, const float* x2d, const float* y, const float* x5, const float* tv, int64_t tv_stride,
+                int64_t T, cudaStream_t st) {
+  KLP(D3D_PROF_LIFT, st, launch_lift_ln(x2d, y, x5, h->wf_t, h->bf, h->spos, tv, tv_stride,
+                                        LnParams{h->blk[0].n1g, h->blk[0].n1b}, h->X, h->A.hi, h->A.lo, h->A.sf, h->fmt, T, h->J,
+                                        h->F * h->J, st));
+  return 0;
+}
+// into block b (1 <= b < nblk): X = Spatial_norm (b - 1 even) / Temporal_norm (b - 1 odd) of X (+ Temporal_pos_embed
+// when b == 1) + time vector of block b;  A = norm1 of block b (X)
+int postnorm_launch(d3d_handle* h, int b, const float* tv, int64_t tv_stride, int64_t T, cudaStream_t st) {
+  const LnParams post = ((b - 1) % 2 == 0) ? LnParams{h->sn_g, h->sn_b} : LnParams{h->tn_g, h->tn_b};
+  const Blk& nx = h->blk[b];
+  KLP(D3D_PROF_LN, st,
+      launch_postnorm_add_ln(h->X, post, (b == 1) ? h->tpos : nullptr, tv ? tv + b * kC : nullptr, tv_stride,
+                             LnParams{nx.n1g, nx.n1b}, h->A.hi, h->A.lo, h->A.sf, h->fmt, T, h->J, h->F, st));
+  return 0;
+}
+// A = norm2 of block b (X)
+int norm2_launch(d3d_handle* h, int b, int64_t T, cudaStream_t st) {
+  KLP(D3D_PROF_LN, st, launch_ln_split(h->X, LnParams{h->blk[b].n2g, h->blk[b].n2b}, 1e-6f, h->A.hi, h->A.lo, h->A.sf, h->fmt,
+                                       T, st));
+  return 0;
+}
+
 // One denoiser evaluation up to (excluding) the final post-norm + head: leaves the residual stream in h->X.
 int run_blocks(d3d_handle* h, const float* x2d, const float* y, const float* x5, const float* tv, int64_t tv_stride,
                int B, int n_blocks, cudaStream_t st) {
   const int64_t T = static_cast<int64_t>(B) * h->F * h->J;
   const int gm = h->cfg.gemm_mode, am = h->cfg.attn_mode;
   int r;
-  KLP(D3D_PROF_LIFT, st, launch_lift_ln(x2d, y, x5, h->wf_t, h->bf, h->spos, tv, tv_stride,
-                                        LnParams{h->blk[0].n1g, h->blk[0].n1b}, h->X, h->A.hi, h->A.lo, h->A.sf, h->fmt, T, h->J,
-                                        h->F * h->J, st));
+  if ((r = lift_launch(h, x2d, y, x5, tv, tv_stride, T, st))) return r;
   for (int b = 0; b < n_blocks; ++b) {
     const Blk& k = h->blk[b];
     const bool spatial = (b % 2) == 0;
@@ -461,19 +487,13 @@ int run_blocks(d3d_handle* h, const float* x2d, const float* y, const float* x5,
     } else {
       if ((r = run_gemm(h, h->ATT, k.proj, T, EPI_F32, h->X, h->X, nullptr, nullptr, nullptr, gm, st, nullptr, nullptr, nullptr,
                         h->have_m_x ? &h->m_x : nullptr))) return r;
-      KLP(D3D_PROF_LN, st, launch_ln_split(h->X, LnParams{k.n2g, k.n2b}, 1e-6f, h->A.hi, h->A.lo, h->A.sf, h->fmt, T, st));
+      if ((r = norm2_launch(h, b, T, st))) return r;
     }
     if (!h->defer_ln2 &&
         (r = run_gemm(h, h->A, k.fc1, T, EPI_GELU_SPLIT, nullptr, nullptr, h->H.hi, h->H.lo, nullptr, gm, st, nullptr, h->H.sf))) return r;
     if ((r = run_gemm(h, h->H, k.fc2, T, EPI_F32, h->X, h->X, nullptr, nullptr, nullptr, gm, st, nullptr, nullptr, nullptr,
                       h->have_m_x ? &h->m_x : nullptr))) return r;
-    if (b + 1 < n_blocks) {
-      const LnParams post = spatial ? LnParams{h->sn_g, h->sn_b} : LnParams{h->tn_g, h->tn_b};
-      const Blk& nx = h->blk[b + 1];
-      KLP(D3D_PROF_LN, st,
-          launch_postnorm_add_ln(h->X, post, (b + 1 == 1) ? h->tpos : nullptr, tv ? tv + (b + 1) * kC : nullptr,
-                                 tv_stride, LnParams{nx.n1g, nx.n1b}, h->A.hi, h->A.lo, h->A.sf, h->fmt, T, h->J, h->F, st));
-    }
+    if (b + 1 < n_blocks && (r = postnorm_launch(h, b + 1, tv, tv_stride, T, st))) return r;
   }
   return 0;
 }
@@ -1128,6 +1148,20 @@ int d3d_op_attention(d3d_handle* h, const float* qkv, float* out, int32_t B, int
   return run_attention(h, h->QKV, nullptr, nullptr, out, B, spatial != 0, attn_mode, st);
 }
 
+// rows [0, T) of a [tok_cap, 512] workspace operand -> raw arrays (layout: include/diff3d_b200.h,
+// d3d_debug_attention_operand)
+static int copy_operand_out(d3d_handle* h, const OperandBuf& o, int64_t T, void* hi_out, void* second_out, cudaStream_t st) {
+  CK(cudaMemcpyAsync(hi_out, o.hi, static_cast<size_t>(T) * kC * 2, cudaMemcpyDeviceToDevice, st));
+  if (h->fmt == FMT_F4C) {
+    // second_out: [T][512] c4 bytes (256 B of P nibbles | 256 B of Q nibbles), then [T][32] scale bytes, row-major
+    CK(cudaMemcpyAsync(second_out, o.lo, static_cast<size_t>(T) * kC, cudaMemcpyDeviceToDevice, st));
+    KL(launch_sf_rows(o.sf, static_cast<uint8_t*>(second_out) + static_cast<size_t>(T) * kC, T, kC, st));
+  } else {
+    CK(cudaMemcpyAsync(second_out, o.lo, static_cast<size_t>(T) * kC * 2, cudaMemcpyDeviceToDevice, st));
+  }
+  return 0;
+}
+
 int d3d_debug_attention_operand(d3d_handle* h, const float* qkv, void* hi_out, void* second_out, int32_t B,
                                 int32_t spatial, int32_t attn_mode, void* stream) {
   if (!h || !qkv || !hi_out || !second_out) return -1;
@@ -1139,15 +1173,59 @@ int d3d_debug_attention_operand(d3d_handle* h, const float* qkv, void* hi_out, v
   KL(launch_pack_qkv16(qkv, h->QKV, T, st));
   int r = run_attention(h, h->QKV, h->ATT.hi, h->ATT.lo, nullptr, B, spatial != 0, attn_mode, st);
   if (r) return r;
-  CK(cudaMemcpyAsync(hi_out, h->ATT.hi, static_cast<size_t>(T) * kC * 2, cudaMemcpyDeviceToDevice, st));
-  if (h->fmt == FMT_F4C) {
-    // second_out: [T][512] c4 bytes (256 B of P nibbles | 256 B of Q nibbles), then [T][32] scale bytes, row-major
-    CK(cudaMemcpyAsync(second_out, h->ATT.lo, static_cast<size_t>(T) * kC, cudaMemcpyDeviceToDevice, st));
-    KL(launch_sf_rows(h->ATT.sf, static_cast<uint8_t*>(second_out) + static_cast<size_t>(T) * kC, T, kC, st));
-  } else {
-    CK(cudaMemcpyAsync(second_out, h->ATT.lo, static_cast<size_t>(T) * kC * 2, cudaMemcpyDeviceToDevice, st));
+  return copy_operand_out(h, h->ATT, T, hi_out, second_out, st);
+}
+
+int d3d_debug_rowwise(d3d_handle* h, int32_t op, int32_t block, const float* in, const int64_t* t_dev, int32_t shared_t,
+                      int32_t B, float* out, void* hi_out, void* second_out, void* stream) {
+  int r = check_ready(h, B);
+  if (r) return r;
+  if (op < D3D_ROWWISE_LIFT || op > D3D_ROWWISE_HEAD) return fail(h, -2, "op out of range");
+  const bool operand = op != D3D_ROWWISE_HEAD, timed = op == D3D_ROWWISE_LIFT || op == D3D_ROWWISE_POSTNORM;
+  if (!in || (op != D3D_ROWWISE_NORM2 && !out) || (operand && (!hi_out || !second_out)) ||
+      (timed && h->cfg.with_time_emb && !t_dev))
+    return fail(h, -1, "null argument");
+  if (op == D3D_ROWWISE_POSTNORM && (block < 1 || block >= h->nblk)) return fail(h, -2, "block out of range [1, 2 depth)");
+  if (op == D3D_ROWWISE_NORM2 && (block < 0 || block >= h->nblk)) return fail(h, -2, "block out of range [0, 2 depth)");
+  DeviceGuard guard(h->cfg.device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int64_t T = static_cast<int64_t>(B) * h->F * h->J;
+  const size_t x_bytes = static_cast<size_t>(T) * kC * sizeof(float);
+  const float* tv = nullptr;
+  int64_t tv_stride = 0;
+  if (timed && h->cfg.with_time_emb) {
+    if ((r = general_time_table(h, t_dev, B, st))) return r;
+    tv = h->tv_general;
+    tv_stride = shared_t ? 0 : static_cast<int64_t>(h->nblk) * kC;
   }
-  return 0;
+  if (operand) {
+    // rows the launch does not write come back as NaN halves / 0xff bytes; the scale atoms (which interleave the
+    // padding rows of the last tile) get byte 1, a scale of 2^-126 that no LayerNorm block produces
+    CK(cudaMemsetAsync(h->A.hi, 0xff, static_cast<size_t>(T) * kC * 2, st));
+    CK(cudaMemsetAsync(h->A.lo, 0xff, static_cast<size_t>(T) * (h->fmt == FMT_F4C ? kC : 2 * kC), st));
+    if (h->fmt == FMT_F4C)
+      CK(cudaMemsetAsync(h->A.sf, 1, static_cast<size_t>((T + 127) / 128) * 128 * (kC / 16), st));
+  }
+  if (op == D3D_ROWWISE_LIFT) {
+    CK(cudaMemsetAsync(h->X, 0xff, x_bytes, st));
+    if (shared_t) {        // the sampler's form: 2D keypoints and the noisy pose in two arrays
+      CK(cudaMemcpy2DAsync(h->in_x2d, 2 * sizeof(float), in, 5 * sizeof(float), 2 * sizeof(float), static_cast<size_t>(T),
+                           cudaMemcpyDeviceToDevice, st));
+      CK(cudaMemcpy2DAsync(h->y, 3 * sizeof(float), in + 2, 5 * sizeof(float), 3 * sizeof(float), static_cast<size_t>(T),
+                           cudaMemcpyDeviceToDevice, st));
+      r = lift_launch(h, h->in_x2d, h->y, nullptr, tv, tv_stride, T, st);
+    } else {               // forward_denoise's form: x5 [T, 5]
+      r = lift_launch(h, nullptr, nullptr, in, tv, tv_stride, T, st);
+    }
+  } else {
+    CK(cudaMemcpyAsync(h->X, in, x_bytes, cudaMemcpyDeviceToDevice, st));
+    if (op == D3D_ROWWISE_POSTNORM) r = postnorm_launch(h, block, tv, tv_stride, T, st);
+    else if (op == D3D_ROWWISE_NORM2) r = norm2_launch(h, block, T, st);
+    else r = run_head(h, DdimStep{}, nullptr, nullptr, out, nullptr, nullptr, 0, B, st);
+  }
+  if (r) return r;
+  if (op == D3D_ROWWISE_LIFT || op == D3D_ROWWISE_POSTNORM) CK(cudaMemcpyAsync(out, h->X, x_bytes, cudaMemcpyDeviceToDevice, st));
+  return operand ? copy_operand_out(h, h->A, T, hi_out, second_out, st) : 0;
 }
 
 int d3d_op_time_table(d3d_handle* h, const float* t_host, int32_t R, float* out, void* stream) {

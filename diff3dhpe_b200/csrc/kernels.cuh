@@ -131,7 +131,7 @@ cudaError_t launch_postnorm_add_ln(float* X, LnParams post, const float* tpos /*
 // A = LN(X; ln)  (MODEL:128 norm2)
 cudaError_t launch_ln_split(const float* X, LnParams ln, float eps, __half* a_hi, __half* a_lo, uint8_t* a_sf, int fmt,
                             int64_t T, cudaStream_t st);
-// out = LN(x) fp32 (stand-alone exhibit / op test)
+// out = LN(x) fp32, the per-row arithmetic of the kernels above (d3d_op_layernorm: reference of their operands)
 cudaError_t launch_ln_f32(const float* x, LnParams ln, float eps, float* out, int64_t T, cudaStream_t st);
 
 struct DdimStep {      // DIFF:287-297 scalars; last != 0 -> y_next = x0 (DIFF:283-285)

@@ -296,6 +296,28 @@ class Engine:
                    "d3d_debug_attention_operand")
         return hi, second
 
+    def debug_rowwise(self, op, inp, t=None, shared_t=False, block=0):
+        """One row-wise kernel launch in isolation (d3d_debug_rowwise; op = _lib.ROWWISE_*).  inp: x5 [T,5] (LIFT) or the
+        residual stream X [T,C]; t: [B] timesteps (LIFT / POSTNORM).  Returns (out, hi, second): out = X after the launch
+        [T,C] (LIFT / POSTNORM), the head output [T,3] (HEAD) or None (NORM2); hi fp16 [T,C] and second uint8 [T,2C] = the
+        A operand written (None for HEAD), in the layout of debug_attention_operand."""
+        T = inp.shape[0]
+        B = T // (self.F * self.J)
+        _check_dev(inp, self.device, (B * self.F * self.J, 5 if op == _lib.ROWWISE_LIFT else self.C), name="inp")
+        if t is not None:
+            t = t.to(device=self.device, dtype=torch.int64).contiguous()
+            if t.numel() != B:
+                raise ValueError("t must have one entry per clip")
+        out = hi = second = None
+        if op != _lib.ROWWISE_NORM2:
+            out = torch.empty((T, 3 if op == _lib.ROWWISE_HEAD else self.C), device=self.device, dtype=torch.float32)
+        if op != _lib.ROWWISE_HEAD:
+            hi = torch.empty((T, self.C), device=self.device, dtype=torch.float16)
+            second = torch.empty((T, 2 * self.C), device=self.device, dtype=torch.uint8)
+        _lib.check(self.lib.d3d_debug_rowwise(self.h, op, block, _ptr(inp), _ptr(t), int(bool(shared_t)), B, _ptr(out),
+                                              _ptr(hi), _ptr(second), self._stream()), self.h, "d3d_debug_rowwise")
+        return out, hi, second
+
     def op_time_table(self, t_host: Sequence[float]):
         R = len(t_host)
         arr = (C.c_float * R)(*[float(v) for v in t_host])

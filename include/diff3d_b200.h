@@ -203,7 +203,9 @@ D3D_API int d3d_op_linear(d3d_handle* h, const float* a_dev, const float* w_dev,
 D3D_API int d3d_op_linear_bench(d3d_handle* h, int64_t M, int32_t N, int32_t K, int32_t act, int32_t gemm_mode,
                         int32_t iters, float* ms_per_launch);
 
-/* LayerNorm over the last dim (512): out = (x-mean)*rstd*gamma+beta (MODEL:184,218). */
+/* LayerNorm over the last dim (512): out = (x-mean)*rstd*gamma+beta (MODEL:184,218).  The per-row arithmetic is the
+ * one of the hot path's row-wise kernels (two-pass variance, rsqrt + one Newton step, packed fp32 pairs), so `out` is
+ * bit for bit the fp32 LayerNorm those kernels quantise into a GEMM operand. */
 D3D_API int d3d_op_layernorm(d3d_handle* h, const float* x_dev, const float* gamma_dev, const float* beta_dev, float eps,
                      float* out_dev, int64_t rows, void* stream);
 
@@ -245,6 +247,33 @@ D3D_API int d3d_op_linear_dln_linear(d3d_handle* h, const float* a_dev, const fl
  * row (k-blocks of 32 elements: 16 of the first part, then 16 of the second), element 2i in the low nibble of byte i). */
 D3D_API int d3d_debug_attention_operand(d3d_handle* h, const float* qkv_dev, void* hi_out_dev, void* second_out_dev,
                                 int32_t B, int32_t spatial, int32_t attn_mode, void* stream);
+
+/* One row-wise kernel of the hot path in isolation: exactly one launch through the production launcher, on the
+ * handle's weights and its own X / A workspace, with the arguments the denoiser call passes.  T = B*F*J rows.
+ *   D3D_ROWWISE_LIFT      in_dev x5 [T,5]; out_dev X [T,C] = fusion_layer(x5) + Spatial_pos_embed + time vector of
+ *                         block 0; operand = norm1 of block 0 (X)                          (MODEL:250, 230-233, 113-116, 127)
+ *   D3D_ROWWISE_POSTNORM  in_dev X [T,C] leaving block `block`-1 (1 <= block < 2*depth); out_dev X entering `block` =
+ *                         Spatial_norm (block-1 even) / Temporal_norm (block-1 odd) of X (+ Temporal_pos_embed when
+ *                         block == 1) + time vector of `block`; operand = norm1 of `block` (X)  (MODEL:236/245, 239-242)
+ *   D3D_ROWWISE_NORM2     in_dev X [T,C]; operand = norm2 of `block` (X), eps 1e-6; out_dev unused (may be NULL)
+ *                                                                                                          (MODEL:128)
+ *   D3D_ROWWISE_HEAD      in_dev X [T,C] leaving the last block; out_dev [T,3] = head.1(head.0 LN (1e-5) of
+ *                         Temporal_norm(X)), the forward_denoise form (MODEL:245, 255-257); no operand
+ * Time vectors (LIFT / POSTNORM, handles with with_time_emb): t_dev [B] int64.  shared_t != 0 adds clip 0's vector to
+ * every row, as the DDIM loop does (one t per step): with the default D3D_LN_ROWS this selects the two-rows-per-warp
+ * kernels, and LIFT reads x5 de-interleaved into the sampler's x2d / y arrays.  shared_t == 0 adds each clip's own
+ * vector, as forward_denoise does: one row per warp.  D3D_LN_ROWS=1 selects the one-row kernels throughout.  The
+ * operand comes back in the layout of d3d_debug_attention_operand (hi_out_dev [T,C] fp16, second_out_dev [T,2*C]
+ * bytes); rows the launch leaves unwritten read back as NaN halves / 0xff bytes. */
+enum {
+  D3D_ROWWISE_LIFT = 0,
+  D3D_ROWWISE_POSTNORM = 1,
+  D3D_ROWWISE_NORM2 = 2,
+  D3D_ROWWISE_HEAD = 3
+};
+D3D_API int d3d_debug_rowwise(d3d_handle* h, int32_t op, int32_t block, const float* in_dev, const int64_t* t_dev,
+                              int32_t shared_t, int32_t B, float* out_dev, void* hi_out_dev, void* second_out_dev,
+                              void* stream);
 
 #ifdef __cplusplus
 }
