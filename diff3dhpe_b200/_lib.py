@@ -7,6 +7,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import threading
 from pathlib import Path
 
 _PKG = Path(__file__).resolve().parent
@@ -78,13 +79,22 @@ PROTOTYPES = {
 }
 
 _lib = None
+_load_lock = threading.Lock()     # nn.DataParallel creates its engines from one thread per device
 
 
 def load():
-    """Load (once) and return the ctypes library with prototypes applied."""
+    """Load (once, also when several threads ask at the same time) and return the ctypes library with prototypes
+    applied."""
     global _lib
     if _lib is not None:
         return _lib
+    with _load_lock:
+        if _lib is None:
+            _lib = _load()
+    return _lib
+
+
+def _load():
     if not LIB_PATH.exists():
         raise RuntimeError(
             f"{LIB_PATH} not found: build it with `python -m diff3dhpe_b200.build` "
@@ -96,7 +106,6 @@ def load():
         fn.argtypes = args
     if lib.d3d_abi_version() != 1:
         raise RuntimeError("libdiff3d_b200.so ABI version mismatch")
-    _lib = lib
     return lib
 
 

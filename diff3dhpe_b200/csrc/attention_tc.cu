@@ -1053,16 +1053,18 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
+static EncodeTiledFn query_encode_tiled() {
+  void* fn = nullptr;
+  cudaDriverEntryPointQueryResult qres;
+  cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
+  return (e == cudaSuccess && qres == cudaDriverEntryPointSuccess) ? reinterpret_cast<EncodeTiledFn>(fn) : nullptr;
+}
+
 int encode_rank4(CUtensorMap* out, void* base, CUtensorMapDataType dt, const cuuint64_t (&dims)[4],
                  const cuuint64_t (&strides)[3], const cuuint32_t (&box)[4], CUtensorMapSwizzle swz) {
-  static EncodeTiledFn encode = nullptr;
-  if (!encode) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
-    if (e != cudaSuccess || qres != cudaDriverEntryPointSuccess || !fn) return -1;
-    encode = reinterpret_cast<EncodeTiledFn>(fn);
-  }
+  // fetched once; a function-local static is initialised thread-safely when handles are created concurrently
+  static const EncodeTiledFn encode = query_encode_tiled();
+  if (!encode) return -1;
   cuuint32_t estr[4] = {1, 1, 1, 1};
   CUresult r = encode(out, dt, 4, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
                       CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);

@@ -21,7 +21,8 @@ using namespace d3d;
 
 namespace {
 
-std::string g_create_error;
+// message of the calling thread's last failed d3d_create: handles may be created from several threads at once
+thread_local std::string g_create_error;
 
 struct Lin {
   int N = 0, K = 0;
@@ -402,9 +403,9 @@ int run_attention(d3d_handle* h, const __half* qkv, __half* o_hi, __half* o_lo, 
 }
 
 int check_weights(d3d_handle* h) {
-  static const char* per_blk[] = {"norm1.weight", "norm1.bias", "attn.qkv.weight", "attn.proj.weight", "attn.proj.bias",
-                                  "norm2.weight", "norm2.bias", "mlp.fc1.weight", "mlp.fc1.bias", "mlp.fc2.weight",
-                                  "mlp.fc2.bias"};
+  static const char* const per_blk[] = {"norm1.weight", "norm1.bias", "attn.qkv.weight", "attn.proj.weight",
+                                        "attn.proj.bias", "norm2.weight", "norm2.bias", "mlp.fc1.weight", "mlp.fc1.bias",
+                                        "mlp.fc2.weight", "mlp.fc2.bias"};
   std::vector<std::string> need = {"fusion_layer.weight", "fusion_layer.bias", "Spatial_pos_embed", "Temporal_pos_embed",
                                    "Spatial_norm.weight", "Spatial_norm.bias", "Temporal_norm.weight", "Temporal_norm.bias",
                                    "head.0.weight", "head.0.bias", "head.1.weight", "head.1.bias"};

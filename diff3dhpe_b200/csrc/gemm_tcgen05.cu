@@ -1144,11 +1144,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constan
   }
 }
 
-// Clusters of 4 cannot straddle a GPC, so fewer than 148/4 of them may be co-resident: ask the runtime (once).
+// Clusters of 4 cannot straddle a GPC, so fewer than 148/4 of them may be co-resident: ask the runtime.
 template <int CG, int BN, int PASSES, int EPI, int CS, int EW = 8>
-int max_clusters(int num_sms) {
-  static int cached = -1;
-  if (cached >= 0) return cached;
+int query_max_clusters(int num_sms) {
   int n = num_sms / (CG * CS);
   if (CG * CS > 2) {
     cudaLaunchConfig_t cfg{};
@@ -1167,8 +1165,15 @@ int max_clusters(int num_sms) {
       n = q;
     (void)cudaGetLastError();
   }
-  cached = n;
   return n;
+}
+
+// Asked once per kernel instance.  A function-local static is initialised exactly once even when handles are created
+// from several threads at the same time (C++11 thread-safe initialisation).
+template <int CG, int BN, int PASSES, int EPI, int CS, int EW = 8>
+int max_clusters(int num_sms) {
+  static const int cached = query_max_clusters<CG, BN, PASSES, EPI, CS, EW>(num_sms);
+  return cached;
 }
 
 template <int CG, int BN, int PASSES, int EPI, int CS = 1, int EW = 8>
@@ -1312,15 +1317,22 @@ static CUtensorMapL2promotion l2_promotion() {
        : k == 2 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
 }
 
+static EncodeTiledFn query_encode_tiled() {
+  void* fn = nullptr;
+  cudaDriverEntryPointQueryResult qres;
+  cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
+  return (e == cudaSuccess && qres == cudaDriverEntryPointSuccess) ? reinterpret_cast<EncodeTiledFn>(fn) : nullptr;
+}
+
+// The driver's cuTensorMapEncodeTiled, fetched once (thread-safe initialisation of a function-local static).
+static EncodeTiledFn encode_tiled() {
+  static const EncodeTiledFn fn = query_encode_tiled();
+  return fn;
+}
+
 int make_operand_map(CUtensorMap* out, const __half* base, int64_t rows, int64_t K, int box_rows) {
-  static EncodeTiledFn encode = nullptr;
-  if (!encode) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
-    if (e != cudaSuccess || qres != cudaDriverEntryPointSuccess || !fn) return -1;
-    encode = reinterpret_cast<EncodeTiledFn>(fn);
-  }
+  const EncodeTiledFn encode = encode_tiled();
+  if (!encode) return -1;
   cuuint64_t dims[2] = {static_cast<cuuint64_t>(K), static_cast<cuuint64_t>(rows)};
   cuuint64_t strides[1] = {static_cast<cuuint64_t>(K) * 2};
   cuuint32_t box[2] = {BK, static_cast<cuuint32_t>(box_rows)};
@@ -1334,11 +1346,8 @@ int make_operand_map(CUtensorMap* out, const __half* base, int64_t rows, int64_t
 
 // uint8 [rows, row_bytes] row-major array (the c8 arrays of FMT_F8C): {128 bytes x 128 rows} boxes, SWIZZLE_128B
 int make_operand_map_u8(CUtensorMap* out, const void* base, int64_t rows, int64_t row_bytes, int box_rows) {
-  void* fn = nullptr;
-  cudaDriverEntryPointQueryResult qres;
-  cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
-  if (e != cudaSuccess || qres != cudaDriverEntryPointSuccess || !fn) return -1;
-  EncodeTiledFn encode = reinterpret_cast<EncodeTiledFn>(fn);
+  const EncodeTiledFn encode = encode_tiled();
+  if (!encode) return -1;
   cuuint64_t dims[2] = {static_cast<cuuint64_t>(row_bytes), static_cast<cuuint64_t>(rows)};
   cuuint64_t strides[1] = {static_cast<cuuint64_t>(row_bytes)};
   cuuint32_t box[2] = {128, static_cast<cuuint32_t>(box_rows)};

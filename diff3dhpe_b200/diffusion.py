@@ -9,10 +9,13 @@ noise in the reference's order and hands raw device pointers across the C ABI.
 from __future__ import annotations
 
 import math
+from contextlib import contextmanager
 
 import torch
 import torch.nn.functional as F
 from torch import nn
+
+from .model import _MasterRef, _SharedWithReplicas
 
 
 def _betas(name: str, timesteps: int) -> torch.Tensor:
@@ -34,7 +37,7 @@ def _betas(name: str, timesteps: int) -> torch.Tensor:
     return torch.clip(1 - (ac[1:] / ac[:-1]), 0, 0.999)
 
 
-class GaussianDiffusion(nn.Module):
+class GaussianDiffusion(_SharedWithReplicas, nn.Module):
     def __init__(self, model, timesteps=100, sampling_timesteps=20, loss_type='l1', conditional=True,
                  clip_denoised=False, beta_schedule='cosine', p2_loss_weight_gamma=0., p2_loss_weight_k=1,
                  ddim_sampling_eta=0., clipLoss=False):
@@ -73,7 +76,7 @@ class GaussianDiffusion(nn.Module):
         }
         for k, v in bufs.items():
             self.register_buffer(k, v.to(torch.float32))
-        self._schedule_key = None
+        self._shared = _MasterRef(self)      # nn.DataParallel replicas read the schedule's identity from the master
 
     # ------------------------------------------------------------------ schedule / engine plumbing
     def ddim_times(self):
@@ -81,15 +84,26 @@ class GaussianDiffusion(nn.Module):
         t = torch.linspace(-1, self.num_timesteps - 1, steps=self.sampling_timesteps + 1)
         return list(reversed(t.int().tolist()))
 
+    @contextmanager
+    def _locked_engine(self, batch):
+        """The model's engine for this device, locked for the caller, with this sampler's schedule set.  The schedule key
+        lives in the engine's record, so it survives nn.DataParallel's per-call replicas, and is built from the master's
+        `alphas_cumprod` (a replica's copy is a new tensor on every call): an unchanged schedule is never set again,
+        which would drop the engine's captured graphs."""
+        with self.model._engine_record(batch) as rec:
+            master = self._shared.master(self)
+            ac = master.alphas_cumprod
+            key = (self._shared, self.sampling_timesteps, float(self.ddim_sampling_eta), bool(self.clip_denoised),
+                   ac.data_ptr(), ac._version)
+            if rec.schedule_key != key:
+                rec.engine.set_schedule(self.ddim_times(), ac, master.sqrt_one_minus_alphas_cumprod,
+                                        self.ddim_sampling_eta, self.clip_denoised)
+                rec.schedule_key = key
+            yield rec.engine
+
     def _engine(self, batch):
-        eng = self.model.engine(batch)
-        key = (id(eng), eng.h.value, self.sampling_timesteps, float(self.ddim_sampling_eta), bool(self.clip_denoised),
-               self.alphas_cumprod.data_ptr(), self.alphas_cumprod._version)
-        if self._schedule_key != key:
-            eng.set_schedule(self.ddim_times(), self.alphas_cumprod, self.sqrt_one_minus_alphas_cumprod,
-                             self.ddim_sampling_eta, self.clip_denoised)
-            self._schedule_key = key
-        return eng
+        with self._locked_engine(batch) as eng:
+            return eng
 
     def draw_noise(self, target_shape, device):
         """The reference's RNG consumption for one sampler call: randn for y_T (DIFF:275), then one randn_like
@@ -109,18 +123,18 @@ class GaussianDiffusion(nn.Module):
     @torch.no_grad()
     def ddim_sample_loop(self, x_in, target_shape, noise=None):
         """DIFF:263-300.  `noise=(y_T, step_noise)` makes the draws explicit (parity tests)."""
-        eng = self._engine(target_shape[0])
-        y_T, step_noise = noise if noise is not None else self.draw_noise(target_shape, eng.device)
-        x_in = x_in.detach().to(device=eng.device, dtype=torch.float32).contiguous()
-        return eng.ddim_sample(x_in, y_T.contiguous(), step_noise)
+        with self._locked_engine(target_shape[0]) as eng:
+            y_T, step_noise = noise if noise is not None else self.draw_noise(target_shape, eng.device)
+            x_in = x_in.detach().to(device=eng.device, dtype=torch.float32).contiguous()
+            return eng.ddim_sample(x_in, y_T.contiguous(), step_noise)
 
     @torch.no_grad()
     def ddim_sample_loop_ouput_reverse_diffusion(self, x_in, target_shape, noise=None):
         """DIFF:304-347 (sic): also returns the y_t and x_start stacks, each [B,F,J,3,S]."""
-        eng = self._engine(target_shape[0])
-        y_T, step_noise = noise if noise is not None else self.draw_noise(target_shape, eng.device)
-        x_in = x_in.detach().to(device=eng.device, dtype=torch.float32).contiguous()
-        return eng.ddim_sample(x_in, y_T.contiguous(), step_noise, trace=True)
+        with self._locked_engine(target_shape[0]) as eng:
+            y_T, step_noise = noise if noise is not None else self.draw_noise(target_shape, eng.device)
+            x_in = x_in.detach().to(device=eng.device, dtype=torch.float32).contiguous()
+            return eng.ddim_sample(x_in, y_T.contiguous(), step_noise, trace=True)
 
     def forward_estimate_pose(self, x, target_shape, output_reverse_diffusion_3d=False):
         """DIFF:350-357."""

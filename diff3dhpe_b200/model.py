@@ -9,6 +9,9 @@ libdiff3d_b200.so through `Engine`.  Training is outside the scope of this packa
 """
 from __future__ import annotations
 
+import threading
+import weakref
+from contextlib import contextmanager
 from functools import partial
 from typing import Optional
 
@@ -51,7 +54,74 @@ class _BlockParams(nn.Module):
         self.mlp = _MlpParams(dim, int(dim * mlp_ratio))
 
 
-class ConditionalDiffusionMixSTES2SGRANDLinLift(nn.Module):
+class _MasterRef:
+    """Link from a module to its master copy, shared by the master and its nn.DataParallel replicas.
+
+    `nn.parallel.replicate` builds each replica with a shallow copy of the master's `__dict__` on every forward call,
+    so an object stored there is shared by the replicas, while anything a replica writes on itself is lost after the
+    call.  Replicas also hold their parameters and buffers as plain attributes (copies broadcast for this call) and
+    `parameters()` / `state_dict()` of a replica are empty, so whatever must be stable across calls is read from the
+    master.  The link is weak: a replica must not keep the master alive, and the master does not point at itself."""
+
+    def __init__(self, owner: nn.Module):
+        self._owner = weakref.ref(owner)
+
+    def master(self, caller: nn.Module) -> nn.Module:
+        owner = self._owner()
+        return caller if owner is None else owner
+
+
+class _EngineRecord:
+    """One device's handle and what it was last loaded with.  `lock` serialises every use of the handle (a handle is
+    not thread-safe, include/diff3d_b200.h)."""
+
+    def __init__(self):
+        self.lock = threading.RLock()
+        self.engine: Optional[Engine] = None
+        self.engine_key = None
+        self.weights_key = None
+        self.schedule_key = None        # written by GaussianDiffusion (diffusion.py)
+
+
+class _EngineRegistry(_MasterRef):
+    """One `_EngineRecord` per device, shared by a module and its nn.DataParallel replicas: each device's handle is
+    created once and survives calls, whichever replica object runs on that device."""
+
+    def __init__(self, owner: nn.Module):
+        super().__init__(owner)
+        self._lock = threading.Lock()
+        self._records = {}
+
+    def record(self, device: torch.device) -> _EngineRecord:
+        with self._lock:
+            rec = self._records.get(device)
+            if rec is None:
+                rec = self._records[device] = _EngineRecord()
+            return rec
+
+    def peek(self, device: torch.device) -> Optional[_EngineRecord]:
+        with self._lock:
+            return self._records.get(device)
+
+
+class _SharedWithReplicas:
+    """Gives every instance a fresh `_shared` object of type `_shared_type` at construction, deep copy and unpickling:
+    a copy (an EMA model, say) never shares or closes the original's handles, and the handles are never pickled."""
+    _shared_type = _MasterRef
+
+    def __getstate__(self):
+        state = super().__getstate__()
+        state.pop("_shared", None)
+        return state
+
+    def __setstate__(self, state):
+        super().__setstate__(state)
+        self._shared = self._shared_type(self)
+
+
+class ConditionalDiffusionMixSTES2SGRANDLinLift(_SharedWithReplicas, nn.Module):
+    _shared_type = _EngineRegistry
+
     def __init__(self, num_frame=9, num_joints=17, in_chans=2, embed_dim=32, depth=4,
                  num_heads=8, mlp_ratio=2., qkv_bias=True, qk_scale=None,
                  drop_rate=0., attn_drop_rate=0., drop_path_rate=0.2, norm_layer=None, with_time_emb=True, **kwargs):
@@ -85,10 +155,8 @@ class ConditionalDiffusionMixSTES2SGRANDLinLift(nn.Module):
         self.Temporal_norm = norm_layer(embed_dim)
         self.head = nn.Sequential(nn.LayerNorm(embed_dim), nn.Linear(embed_dim, 3))
 
-        # engine state (not part of the state dict)
-        self._engine: Optional[Engine] = None
-        self._engine_key = None
-        self._weights_key = None
+        # engine state (not part of the state dict): one handle per device, shared with nn.DataParallel replicas
+        self._shared = _EngineRegistry(self)
         self._weights_epoch = 0
         self.gemm_mode = _lib.GEMM_DEFAULT
         self.attn_mode = _lib.ATTN_DEFAULT
@@ -97,43 +165,75 @@ class ConditionalDiffusionMixSTES2SGRANDLinLift(nn.Module):
 
     # ------------------------------------------------------------------ engine management
     def _weights_fingerprint(self):
-        return (self._weights_epoch,) + tuple((p.data_ptr(), p._version) for p in self.parameters())
+        """From the master's parameters: a replica's broadcast copies are new tensors on every call."""
+        master = self._shared.master(self)
+        return (master._weights_epoch,) + tuple((p.data_ptr(), p._version) for p in master.parameters())
 
     def invalidate_weights(self):
         """Forces a re-upload (re-packing) of the weights at the next call.  The engine notices parameter updates through
         `(data_ptr, _version)` of every parameter, which covers optimizer steps, `load_state_dict`, `copy_`, `.to()`
         and in-place ops on the parameter itself -- but NOT writes through `.data` (`p.data.copy_(ema)`, EMA / SWA
         weight swaps), which do not bump `_version`: call this after such a write.  (A content checksum would need a
-        device -> host synchronisation on every sampler call, which the hot path must not have.)"""
+        device -> host synchronisation on every sampler call, which the hot path must not have.)  Every device's
+        engine re-uploads at its next call."""
         self._weights_epoch += 1
 
     def _load_from_state_dict(self, *args, **kwargs):
         self._weights_epoch += 1
         return super()._load_from_state_dict(*args, **kwargs)
 
-    def engine(self, batch: int = 1) -> Engine:
-        """Returns the Engine for the device the parameters live on, (re)building it when the device, the
-        kernel modes or the required capacity changed, and re-uploading weights when any parameter changed."""
+    @property
+    def _engine(self) -> Optional[Engine]:
+        """The engine of the device the parameters live on (None before the first call)."""
+        try:
+            rec = self._shared.peek(self._engine_device())
+        except RuntimeError:            # not on a GPU: no engine
+            return None
+        return None if rec is None else rec.engine
+
+    def _engine_device(self) -> torch.device:
+        """The device this module (or nn.DataParallel replica) runs on: that of its parameters."""
         dev = self.fusion_layer.weight.device
         if dev.type != "cuda":
             raise RuntimeError("diff3dhpe_b200 runs on CUDA (sm_100a) only: move the module to a B200 with .cuda(); "
                                "there is no CPU fallback")
-        need = max(batch, self.max_clips_hint)
-        key = (dev, self.gemm_mode, self.attn_mode, self.use_graph)
-        if self._engine is None or self._engine_key != key or self._engine.max_clips < need:
-            if self._engine is not None:
-                self._engine.close()
-            mlp_hidden = int(self.embed_dim * self.mlp_ratio)
-            self._engine = Engine(self.num_frame, self.num_joints, self.embed_dim, self.block_depth, self.num_heads,
-                                  mlp_hidden, self.with_time_emb, need, dev, self.gemm_mode, self.attn_mode,
-                                  self.use_graph)
-            self._engine_key = key
-            self._weights_key = None
-        fp = self._weights_fingerprint()
-        if self._weights_key != fp:
-            self._engine.load_state_dict({k: v for k, v in self.state_dict().items()})
-            self._weights_key = fp
-        return self._engine
+        return dev
+
+    @contextmanager
+    def _engine_record(self, batch: int):
+        """Holds the lock of the record of the device this module (or replica) runs on while the caller uses its
+        engine, after bringing the engine up to date (see `engine`)."""
+        dev = self._engine_device()
+        rec = self._shared.record(dev)
+        with rec.lock:
+            need = max(batch, self.max_clips_hint)
+            key = (self.gemm_mode, self.attn_mode, self.use_graph)
+            if rec.engine is None or rec.engine.h is None or rec.engine_key != key or rec.engine.max_clips < need:
+                if rec.engine is not None:
+                    rec.engine.close()
+                    rec.engine = None
+                mlp_hidden = int(self.embed_dim * self.mlp_ratio)
+                rec.engine = Engine(self.num_frame, self.num_joints, self.embed_dim, self.block_depth, self.num_heads,
+                                    mlp_hidden, self.with_time_emb, need, dev, self.gemm_mode, self.attn_mode,
+                                    self.use_graph)
+                rec.engine_key, rec.weights_key, rec.schedule_key = key, None, None
+            fp = self._weights_fingerprint()
+            if rec.weights_key != fp:
+                # Uploaded from the master's parameters, the tensors the fingerprint was taken from; the engine stages
+                # those of another device through the host.  A replica's copies hold the same values, but reaching them
+                # relies on how torch lays replicas out, and this runs once per change of the weights, not per call.
+                rec.engine.load_state_dict(dict(self._shared.master(self).state_dict()))
+                rec.weights_key = fp
+            yield rec
+
+    def engine(self, batch: int = 1) -> Engine:
+        """Returns the Engine for the device the parameters live on, (re)building it when the kernel modes changed, the
+        required capacity grew or it was closed, and re-uploading weights when any parameter of the master changed.
+        Each device keeps its own engine, shared by the module and its nn.DataParallel replicas, for as long as the
+        module lives (a module moved to another device keeps the first device's engine too).  The returned engine is
+        not locked: use it from one thread at a time."""
+        with self._engine_record(batch) as rec:
+            return rec.engine
 
     # ------------------------------------------------------------------ reference API
     def forward_denoise(self, x, time):
@@ -145,8 +245,8 @@ class ConditionalDiffusionMixSTES2SGRANDLinLift(nn.Module):
         b, f, n, _ = x.shape
         if f != self.num_frame or n != self.num_joints:
             raise ValueError(f"expected [B,{self.num_frame},{self.num_joints},5], got {tuple(x.shape)}")
-        eng = self.engine(b)
-        return eng.forward_denoise(x.detach().to(torch.float32).contiguous(), time)
+        with self._engine_record(b) as rec:
+            return rec.engine.forward_denoise(x.detach().to(torch.float32).contiguous(), time)
 
     def forward(self, x, time):
         return self.forward_denoise(x, time)

@@ -22,6 +22,10 @@
  *   - `stream` is a cudaStream_t passed as void* (NULL = legacy default stream).  All work is enqueued
  *     asynchronously on it unless stated otherwise.
  *   - a handle is bound to one device and is not thread-safe; use one handle per rank.
+ *   - distinct handles may be created, used and destroyed concurrently from different threads, on the same
+ *     device or on different ones (one thread per device is how nn.DataParallel drives the drop-in modules);
+ *     one handle must not be used by two threads at once.  The library's process-wide state is limited to
+ *     values initialised once, thread-safely, and the thread-local message of d3d_last_error(NULL).
  *   - the library owns packed weights, the time-embedding table, the activation workspace and its CUDA
  *     graphs; nothing is allocated on the hot path.
  */
@@ -95,7 +99,7 @@ D3D_API int d3d_abi_version(void);
 /* Replaces the module constructor (MODEL:140-220): allocates workspace for max_clips clips. */
 D3D_API int d3d_create(const d3d_config* cfg, d3d_handle** out);
 D3D_API void d3d_destroy(d3d_handle* h);
-/* Message of the last failing call on this handle (h == NULL: last failing d3d_create). */
+/* Message of the last failing call on this handle (h == NULL: the calling thread's last failing d3d_create). */
 D3D_API const char* d3d_last_error(const d3d_handle* h);
 
 /* Replaces load_state_dict (RUN:226-235): copies, packs and (for GEMM operands) splits the weights.
