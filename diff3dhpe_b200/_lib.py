@@ -53,6 +53,9 @@ PROTOTYPES = {
                                        C.c_void_p]),
     "d3d_pose_metrics_accumulate": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
                                               C.c_void_p]),
+    "d3d_pck_accumulate": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                     C.POINTER(C.c_float), C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.c_void_p]),
     "d3d_launch_count": (C.c_int64, [C.c_void_p]),
     "d3d_workspace_bytes": (C.c_int64, [C.c_void_p]),
     "d3d_profile_begin": (C.c_int, [C.c_void_p]),

@@ -1103,6 +1103,28 @@ int d3d_pose_metrics_accumulate(d3d_handle* h, const float* pred, const float* g
   return 0;
 }
 
+int d3d_pck_accumulate(d3d_handle* h, const float* pred, const float* gt, const int64_t* frame_index,
+                       const int32_t* frame_group, int64_t n_sel, const float* thresholds, int32_t n_thr,
+                       int32_t n_groups, int64_t* counts, double* err_sum, int64_t* frames, void* stream) {
+  if (!h) return -1;
+  if (!pred || !gt || !thresholds || !counts || !err_sum || !frames) return fail(h, -1, "null argument");
+  if (n_sel < 0) return fail(h, -2, "n_sel < 0");
+  if (n_thr < 1 || n_thr > kPckMaxThresholds) return fail(h, -2, "n_thr out of range [1, 64]");
+  if (n_groups < 1 || n_groups > kPckMaxGroups) return fail(h, -2, "n_groups out of range [1, 65536]");
+  PckThresholds thr{};
+  thr.n = n_thr;
+  for (int k = 0; k < n_thr; ++k) {
+    if (!std::isfinite(thresholds[k])) return fail(h, -2, "thresholds must be finite");
+    if (k > 0 && !(thresholds[k] > thresholds[k - 1])) return fail(h, -2, "thresholds must be strictly ascending");
+    thr.t[k] = thresholds[k];
+  }
+  if (n_sel == 0) return 0;
+  DeviceGuard guard(h->cfg.device);
+  KL(launch_pck_hist(pred, gt, frame_index, frame_group, n_sel, h->J, thr, n_groups, counts, err_sum, frames, h->num_sms,
+                     static_cast<cudaStream_t>(stream)));
+  return 0;
+}
+
 int d3d_profile_begin(d3d_handle* h) {
   if (!h) return -1;
   h->prof = true;

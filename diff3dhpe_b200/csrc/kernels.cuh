@@ -155,6 +155,20 @@ cudaError_t launch_mpjpe(const float* pred, const float* gt, const uint8_t* mask
 cudaError_t launch_pose_metrics(const float* pred, const float* gt, const int64_t* sel /*or null*/, int64_t n_sel, int J,
                                 double* acc, double* vel_tmp, cudaStream_t st);
 
+// Grouped per-joint histogram of joint errors (metrics.cu, d3d_pck_accumulate): counts[g][j][k] += listed frames of group
+// g whose joint-j error is < thr.t[k], err_sum[g][j] += those errors, frames[g] += listed frames of group g.
+constexpr int kPckMaxThresholds = 64;
+constexpr int kPckMaxGroups = 65536;
+constexpr int kPckSmemBinBytes = 32 * 1024;   // histograms up to this size are built in shared memory per block
+struct PckThresholds {                        // passed by value: no device copy, graph-capturable
+  float t[kPckMaxThresholds];                 // t[0] < t[1] < ... < t[n-1], finite (checked by the caller)
+  int n;
+};
+cudaError_t launch_pck_hist(const float* pred, const float* gt, const int64_t* sel /*or null*/,
+                            const int32_t* group /*[n_frames] or null*/, int64_t n_sel, int J, const PckThresholds& thr,
+                            int n_groups, int64_t* counts, double* err_sum, int64_t* frames, int num_sms,
+                            cudaStream_t st);
+
 // ------------------------------------------------------------------ windowing (packed sequences <-> F-frame windows)
 cudaError_t launch_window_gather(const float* seq2d, const int64_t* start, const int32_t* perm /*[J] device*/, float* x2d,
                                  float* x2d_flip /*or null*/, int64_t n_win, int F, int J, cudaStream_t st);

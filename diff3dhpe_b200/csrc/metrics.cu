@@ -3,6 +3,7 @@
 //   reference) and mean_velocity_error (LOSS:133-142), accumulated as fp64 sums so that the whole tail of RUN:602-614
 //   stays on the GPU.  LOSS = common/loss.py.  One thread per frame; the 3 x 3 SVD is a cyclic Jacobi
 //   eigen-decomposition of H^T H in fp64.
+// Also the per-joint error histogram behind the MPI-INF-3DHP PCK / AUC table (pck_hist_kernel).
 #include "kernels.cuh"
 
 namespace d3d {
@@ -182,6 +183,86 @@ __global__ void vel_finalize_kernel(double* __restrict__ acc, double* __restrict
   vel_tmp[1] = 0.0;
 }
 
+// MPI-INF-3DHP PCK / AUC (d3d_pck_accumulate): a grouped, per-joint histogram of joint errors.  The protocol (thresholds,
+// evaluated joints, units) is the caller's; the kernel only counts.  One warp per listed frame, lane j = joint j.
+// The error is d = sqrt((dx*dx + dy*dy) + dz*dz), dx = pred - gt, rounded after every operation (no FMA contraction) so
+// that a float32 restatement on the host reproduces it bit for bit.  Its bin b is the number of thresholds d is NOT
+// below (strict <): the joint counts under thresholds b..n-1.  NaN and +inf land in bin n and count under none.
+// kSmem: the block builds [n_groups][J][n] per-bin counts in shared memory and adds their prefix sums to `counts` at
+// exit, one atomic per non-zero (group, joint, threshold).  Otherwise every joint adds 1 to counts[g][j][b..n-1] directly.
+// The error and frame sums of a lane stay in registers while consecutive frames of the warp share a group.
+template <bool kSmem>
+__global__ void __launch_bounds__(512) pck_hist_kernel(const float* __restrict__ pred, const float* __restrict__ gt,
+                                                       const int64_t* __restrict__ sel, const int32_t* __restrict__ group,
+                                                       int64_t n_sel, int J, const __grid_constant__ PckThresholds thr,
+                                                       int n_groups, unsigned long long* __restrict__ counts,
+                                                       double* __restrict__ err_sum,
+                                                       unsigned long long* __restrict__ frames) {
+  extern __shared__ unsigned int bins[];               // kSmem: [n_groups][J][n]
+  __shared__ float s_thr[kPckMaxThresholds];           // padded with +inf for the fixed-depth search
+  const int n = thr.n;
+  const int rows = n_groups * J;
+  if (threadIdx.x < kPckMaxThresholds) s_thr[threadIdx.x] = threadIdx.x < n ? thr.t[threadIdx.x] : __int_as_float(0x7f800000);
+  if (kSmem)
+    for (int i = threadIdx.x; i < rows * n; i += blockDim.x) bins[i] = 0u;
+  __syncthreads();
+
+  const int lane = threadIdx.x & 31;
+  const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
+  int cur = -1;                                        // group whose sums this lane holds
+  double esum = 0.0;
+  unsigned long long nf = 0;
+  auto flush = [&]() {
+    if (cur < 0) return;
+    if (lane < J) atomicAdd(err_sum + static_cast<int64_t>(cur) * J + lane, esum);
+    if (lane == 0) atomicAdd(frames + cur, nf);
+  };
+  for (int64_t i = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; i < n_sel; i += n_warps) {
+    const int64_t f = sel ? sel[i] : i;
+    const int g = group ? group[f] : 0;
+    if (g < 0 || g >= n_groups) continue;              // warp-uniform: the whole frame is skipped
+    if (g != cur) {
+      flush();
+      cur = g;
+      esum = 0.0;
+      nf = 0;
+    }
+    ++nf;
+    if (lane < J) {
+      const float* P = pred + (f * J + lane) * 3;
+      const float* G = gt + (f * J + lane) * 3;
+      const float dx = __fsub_rn(P[0], G[0]), dy = __fsub_rn(P[1], G[1]), dz = __fsub_rn(P[2], G[2]);
+      const float d = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz)));
+      esum += static_cast<double>(d);
+      // b = #{k : !(d < s_thr[k])}: the predicate is true on a prefix of the 64 padded thresholds
+      int b = 0;
+#pragma unroll
+      for (int step = 32; step > 0; step >>= 1)
+        if (!(d < s_thr[b + step - 1])) b += step;
+      if (!(d < s_thr[b])) ++b;                         // b <= 63 here
+      if (b < n) {
+        const int64_t row = static_cast<int64_t>(g) * J + lane;
+        if (kSmem) {
+          atomicAdd(bins + row * n + b, 1u);
+        } else {
+          for (int k = b; k < n; ++k) atomicAdd(counts + row * n + k, 1ull);
+        }
+      }
+    }
+  }
+  flush();
+  if (kSmem) {
+    __syncthreads();
+    for (int r = threadIdx.x; r < rows; r += blockDim.x) {
+      unsigned long long run = 0;
+      for (int k = 0; k < n; ++k) {
+        run += bins[r * n + k];
+        if (run) atomicAdd(counts + static_cast<int64_t>(r) * n + k, run);
+      }
+    }
+  }
+}
+
 }  // namespace
 
 cudaError_t launch_pose_metrics(const float* pred, const float* gt, const int64_t* sel, int64_t n_sel, int J, double* acc,
@@ -192,6 +273,28 @@ cudaError_t launch_pose_metrics(const float* pred, const float* gt, const int64_
   if (g > 148 * 16) g = 148 * 16;
   pose_metrics_kernel<<<static_cast<unsigned>(g), 128, 0, st>>>(pred, gt, sel, n_sel, J, acc, vel_tmp);
   vel_finalize_kernel<<<1, 1, 0, st>>>(acc, vel_tmp, static_cast<double>(n_sel));
+  return cudaGetLastError();
+}
+
+cudaError_t launch_pck_hist(const float* pred, const float* gt, const int64_t* sel, const int32_t* group, int64_t n_sel,
+                            int J, const PckThresholds& thr, int n_groups, int64_t* counts, double* err_sum,
+                            int64_t* frames, int num_sms, cudaStream_t st) {
+  if (n_sel <= 0) return cudaSuccess;
+  if (J < 1 || J > kMaxJ || thr.n < 1 || thr.n > kPckMaxThresholds || n_groups < 1 || n_groups > kPckMaxGroups)
+    return cudaErrorInvalidValue;
+  constexpr int kThreads = 512;
+  // two blocks per SM: the shared-memory path pays one flush of its whole histogram per block
+  int64_t g = (n_sel + kThreads / 32 - 1) / (kThreads / 32);
+  if (g > 2 * num_sms) g = 2 * num_sms;
+  const int64_t bin_bytes = static_cast<int64_t>(n_groups) * J * thr.n * sizeof(unsigned int);
+  auto* c = reinterpret_cast<unsigned long long*>(counts);
+  auto* fr = reinterpret_cast<unsigned long long*>(frames);
+  if (bin_bytes <= kPckSmemBinBytes)
+    pck_hist_kernel<true><<<static_cast<unsigned>(g), kThreads, static_cast<size_t>(bin_bytes), st>>>(
+        pred, gt, sel, group, n_sel, J, thr, n_groups, c, err_sum, fr);
+  else
+    pck_hist_kernel<false><<<static_cast<unsigned>(g), kThreads, 0, st>>>(pred, gt, sel, group, n_sel, J, thr, n_groups,
+                                                                          c, err_sum, fr);
   return cudaGetLastError();
 }
 

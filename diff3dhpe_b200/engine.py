@@ -5,6 +5,7 @@ from __future__ import annotations
 import ctypes as C
 from typing import Dict, Optional, Sequence
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -221,6 +222,66 @@ class Engine:
         a = acc.tolist()
         n, nv = max(a[3], 1.0), max(a[5], 1.0)
         return a[0] / n, a[2] / n, a[1] / n, a[4] / nv
+
+    def pck_accumulate(self, pred: torch.Tensor, gt: torch.Tensor, counts: torch.Tensor, err_sum: torch.Tensor,
+                       frames: torch.Tensor, thresholds: Sequence[float], frame_index: Optional[torch.Tensor] = None,
+                       frame_group: Optional[torch.Tensor] = None):
+        """Grouped per-joint histogram of joint errors (d3d_pck_accumulate, see include/diff3d_b200.h).  For the frames
+        listed in frame_index (int64, None = all rows in order) adds to counts int64 [G, J, n_thr] the joints whose error
+        ||pred - gt|| is below thresholds[k] (strict), to err_sum fp64 [G, J] the sum of the errors and to frames int64
+        [G] the frames counted.  A frame's group is frame_group[row] (int32 [n_frames], None = group 0); frames of a group
+        outside [0, G) are skipped.  thresholds: 1..64 finite, strictly ascending values in the poses' units (rounded to
+        fp32).  Asynchronous on the current stream."""
+        _check_dev(pred, self.device, name="pred")
+        if tuple(pred.shape[-2:]) != (self.J, 3):
+            raise ValueError(f"pred must have shape [..., {self.J}, 3], got {tuple(pred.shape)}")
+        _check_dev(gt, self.device, tuple(pred.shape), name="gt")
+        n_frames = pred.numel() // (self.J * 3)
+        thr = [float(t) for t in thresholds]
+        G = counts.shape[0] if counts.dim() == 3 else 0
+        _check_dev(counts, self.device, (G, self.J, len(thr)), torch.int64, "counts")
+        _check_dev(err_sum, self.device, (G, self.J), torch.float64, "err_sum")
+        _check_dev(frames, self.device, (G,), torch.int64, "frames")
+        n = n_frames
+        if frame_index is not None:
+            _check_dev(frame_index, self.device, dtype=torch.int64, name="frame_index")
+            n = frame_index.numel()
+        if frame_group is not None:
+            _check_dev(frame_group, self.device, (n_frames,), torch.int32, "frame_group")
+        arr = (C.c_float * max(len(thr), 1))(*thr)
+        _lib.check(self.lib.d3d_pck_accumulate(self.h, _ptr(pred), _ptr(gt), _ptr(frame_index), _ptr(frame_group), n,
+                                               arr, len(thr), G, _ptr(counts), _ptr(err_sum), _ptr(frames),
+                                               self._stream()), self.h, "d3d_pck_accumulate")
+        return counts, err_sum, frames
+
+    @staticmethod
+    def pck_table(counts, err_sum, frames, thresholds: Sequence[float], joints: Sequence[int], pck_threshold: float):
+        """Host-side table from pck_accumulate's buffers, over the joints listed in `joints`: for every group and for all
+        groups pooled (counts and frames summed, then divided) a row {'pck': 100 * share of joint errors below
+        pck_threshold, 'auc': mean of that share (in %) over all thresholds, 'mpjpe': mean joint error in the poses'
+        units, 'frames': frames counted}.  pck_threshold must be one of the thresholds (compared in fp32).  A row
+        without frames has NaN metrics.  Returns {'all': row, 'groups': [row of group 0, 1, ...]}."""
+        def host(x, dtype):
+            return np.asarray(x.detach().cpu().numpy() if isinstance(x, torch.Tensor) else x, dtype=dtype)
+
+        c, e, f = host(counts, np.int64), host(err_sum, np.float64), host(frames, np.int64)
+        thr32 = np.asarray(thresholds, dtype=np.float32)
+        if c.ndim != 3 or c.shape[2] != thr32.size or e.shape != c.shape[:2] or f.shape != c.shape[:1]:
+            raise ValueError("counts [G, J, n_thr], err_sum [G, J] and frames [G] do not match the thresholds")
+        hit = np.flatnonzero(thr32 == np.float32(pck_threshold))
+        if hit.size != 1:
+            raise ValueError(f"pck_threshold {pck_threshold} is not one of the thresholds")
+        joints = list(joints)
+        c, e = c[:, joints, :].sum(axis=1), e[:, joints].sum(axis=1)     # [G, n_thr] int64, [G] fp64
+
+        def row(cnt, err, nf):
+            n = int(nf) * len(joints)
+            if n == 0:
+                return {"pck": float("nan"), "auc": float("nan"), "mpjpe": float("nan"), "frames": int(nf)}
+            share = 100.0 * cnt.astype(np.float64) / n
+            return {"pck": float(share[hit[0]]), "auc": float(share.mean()), "mpjpe": float(err / n), "frames": int(nf)}
+
+        return {"all": row(c.sum(axis=0), e.sum(), f.sum()), "groups": [row(c[g], e[g], f[g]) for g in range(c.shape[0])]}
 
     def profile_begin(self):
         _lib.check(self.lib.d3d_profile_begin(self.h), self.h, "d3d_profile_begin")

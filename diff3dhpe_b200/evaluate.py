@@ -14,6 +14,14 @@ import torch
 import torch.distributed as dist
 
 from . import synthetic
+from .engine import Engine
+
+# The MPI-INF-3DHP test protocol, as the dataset's MATLAB evaluation (mpii_compute_3d_pck.m) defines it: PCK at 150 mm
+# and AUC over 0, 5, ..., 150 mm of the 14 joints 0..13 of the MPI 17-joint order (head-top, neck, then right and left
+# shoulder, elbow, wrist, hip, knee, ankle; pelvis 14, spine 15 and head 16 are not evaluated), and its joint groups.
+MPI3DHP_PCK_JOINTS = tuple(range(14))
+MPI3DHP_JOINT_GROUPS = {"Head": (0,), "Neck": (1,), "Shoulder": (2, 5), "Elbow": (3, 6), "Wrist": (4, 7),
+                        "Hip": (8, 11), "Knee": (9, 12), "Ankle": (10, 13)}
 
 
 def shard_range(n_clips: int, rank: int, world: int) -> Tuple[int, int]:
@@ -137,6 +145,58 @@ def evaluate_sequences(sampler, seq2d: torch.Tensor, gt3d: Optional[torch.Tensor
     if gt3d is not None:
         sampler.mpjpe(out, gt3d.to(device, non_blocking=True).contiguous(), acc, None)
     return {"pred": out, "acc": acc, "n_windows": n_win}
+
+
+def mpi3dhp_thresholds(mm_per_unit: float):
+    """The 31 PCK thresholds 0, 5, ..., 150 mm of the MPI-INF-3DHP protocol in the poses' units: mm_per_unit = 1000 for
+    poses in metres, 1 for poses in millimetres.  The last one is the PCK threshold."""
+    if not mm_per_unit > 0:
+        raise ValueError("mm_per_unit must be positive")
+    return [5.0 * k / mm_per_unit for k in range(31)]
+
+
+def mpi3dhp_metrics(engine: Engine, pred: torch.Tensor, gt: torch.Tensor, *, mm_per_unit: float,
+                    frame_group: Optional[torch.Tensor] = None, n_groups: int = 1, group_names: Optional[Sequence] = None,
+                    frame_index: Optional[torch.Tensor] = None) -> Dict:
+    """The MPI-INF-3DHP PCK / AUC / MPJPE table on the device: one `Engine.pck_accumulate` call over pred / gt ([N, 17, 3]
+    in the MPI joint order, e.g. the packed 'pred' of `evaluate_sequences` and its ground truth), then the host-side table.
+    Errors are taken as given (no root alignment).  frame_group: int32 [N] group id per frame (per sequence, e.g.
+    `seq_id.repeat_interleave(F - first_valid)` from `plan_windows`, or per activity); frames outside [0, n_groups) are
+    left out.  frame_index: the frames to evaluate (int64, None = all).
+    Returns {'overall': row, 'groups': {name: row}, 'joint_groups': {'Head': row, ...}}, where a row holds 'pck' and
+    'auc' (%) and 'mpjpe' (mm) over the 14 evaluated joints (of that joint group in 'joint_groups', over all groups of
+    frames) and 'frames'; 'overall' and 'groups' rows also hold 'mpjpe_all_joints' (mm, all 17 joints)."""
+    if engine.J != 17:
+        raise ValueError("the MPI-INF-3DHP protocol needs poses in the 17-joint MPI order")
+    names = list(range(n_groups)) if group_names is None else list(group_names)
+    if len(names) != n_groups:
+        raise ValueError("group_names must have n_groups entries")
+    thr = mpi3dhp_thresholds(mm_per_unit)
+    dev = engine.device
+    counts = torch.zeros((n_groups, engine.J, len(thr)), device=dev, dtype=torch.int64)
+    err_sum = torch.zeros((n_groups, engine.J), device=dev, dtype=torch.float64)
+    frames = torch.zeros(n_groups, device=dev, dtype=torch.int64)
+    if frame_group is not None:
+        frame_group = frame_group.to(device=dev, dtype=torch.int32).contiguous()
+    if frame_index is not None:
+        frame_index = frame_index.to(device=dev, dtype=torch.int64).contiguous()
+    engine.pck_accumulate(pred.contiguous(), gt.to(dev).contiguous(), counts, err_sum, frames, thr, frame_index,
+                          frame_group)
+    counts, err_sum, frames = counts.cpu(), err_sum.cpu(), frames.cpu()
+
+    def table(joints):
+        return Engine.pck_table(counts, err_sum, frames, thr, joints, thr[-1])
+
+    def in_mm(row, every=None):
+        out = dict(row, mpjpe=row["mpjpe"] * mm_per_unit)
+        if every is not None:
+            out["mpjpe_all_joints"] = every["mpjpe"] * mm_per_unit
+        return out
+
+    main, every = table(MPI3DHP_PCK_JOINTS), table(range(engine.J))
+    return {"overall": in_mm(main["all"], every["all"]),
+            "groups": {n: in_mm(r, a) for n, r, a in zip(names, main["groups"], every["groups"])},
+            "joint_groups": {name: in_mm(table(joints)["all"]) for name, joints in MPI3DHP_JOINT_GROUPS.items()}}
 
 
 def gather_results(local_pred: torch.Tensor, acc: torch.Tensor, n_total: int, group=None):

@@ -149,6 +149,29 @@ D3D_API int d3d_tta_merge(d3d_handle* h, const float* y_dev, const float* y_flip
 D3D_API int d3d_pose_metrics_accumulate(d3d_handle* h, const float* pred_dev, const float* gt_dev,
                                 const int64_t* frame_index_dev, int64_t n_sel, double* acc_dev, void* stream);
 
+/* The counts behind the MPI-INF-3DHP PCK / AUC table (the dataset's MATLAB evaluation, mpii_compute_3d_pck.m, which
+ * the reference runs offline on a .mat dump): a grouped, per-joint histogram of joint errors.  For each of the n_sel
+ * frames listed in frame_index_dev (NULL = rows 0..n_sel-1; a row listed twice counts twice) with group
+ * g = frame_group_dev[row] (int32 [n_frames], indexed by row; NULL = every row in group 0), and each joint j, the error
+ *   d = sqrt((dx*dx + dy*dy) + dz*dz),  (dx, dy, dz) = pred - gt,
+ * is computed in fp32 with every operation rounded (no fused multiply-add) and compared in fp32, and these += :
+ *   counts_dev  [n_groups][J][n_thr] int64   joints whose d < thresholds_host[k]   (strict; NaN counts under none)
+ *   err_sum_dev [n_groups][J]        fp64    sum of d                              (NaN if any d is NaN)
+ *   frames_dev  [n_groups]           int64   frames counted
+ * pred_dev / gt_dev: [n_frames, J, 3].  A frame whose group lies outside [0, n_groups) is skipped entirely.  No root
+ * alignment: errors are taken as given, in the poses' units; thresholds are in the same units.
+ * thresholds_host: n_thr (1..64) finite, strictly ascending floats, read during the call and passed to the kernel by
+ * value, so the call allocates nothing, does not synchronise and can be captured into a CUDA graph.  1 <= n_groups <=
+ * 65536.  Invalid arguments return a negative code before anything is enqueued: -1 a null pointer (other than the two
+ * optional ones), -2 n_sel < 0, n_thr or n_groups out of range, or thresholds not finite and strictly ascending.
+ * n_sel == 0 enqueues nothing and succeeds.
+ * Histograms of up to 32 KB (n_groups * J * n_thr * 4 bytes) are built in shared memory per block; larger ones are
+ * counted with global atomics, about n_thr of them per joint. */
+D3D_API int d3d_pck_accumulate(d3d_handle* h, const float* pred_dev, const float* gt_dev, const int64_t* frame_index_dev,
+                               const int32_t* frame_group_dev, int64_t n_sel, const float* thresholds_host, int32_t n_thr,
+                               int32_t n_groups, int64_t* counts_dev, double* err_sum_dev, int64_t* frames_dev,
+                               void* stream);
+
 /* Windowing on the device (common/nosiy_generators.py:27-48, 264-276; "next" row N3 of SURVEY.md 8f).
  * seq2d_dev: packed sequences [n_frames_total, J, 2]; win_start_dev[w] = first packed frame of window w.  Writes
  * x2d_out_dev [n_win, F, J, 2] and, when x2d_flip_out_dev != NULL, the horizontally flipped copy (x negated, joints
