@@ -4,7 +4,8 @@
 Clips are independent, so rank r of R owns a contiguous block of clips (both flip variants of a clip stay on
 the same rank); nothing is communicated inside the sampler.  One exchange step at the end: gather of the merged
 predictions and an all-reduce of the fp64 (sum of joint errors, joint count) pair -- NCCL on GPUs, gloo in the
-CPU tests of this plumbing.
+CPU tests of this plumbing.  Sweeps over raw packed sequences gather with `gather_packed` (frame counts differ per
+rank) and build the Human3.6M per-action table with `h36m_metrics` on the gathered array.
 """
 from __future__ import annotations
 
@@ -62,6 +63,37 @@ def plan_windows(seq_lengths: Sequence[int], F: int):
         base += int(n)
     return (torch.tensor(starts, dtype=torch.int64), torch.tensor(valid, dtype=torch.int32),
             torch.tensor(sid, dtype=torch.int32))
+
+
+def loader_batch_runs(seq_lengths: Sequence[int], seq_group: Sequence[int], F: int, batch_size: int):
+    """The reference's per-action batching (a new DataLoader per action, RUN:730-736) as runs of packed frames.  The
+    windows of `plan_windows` are cut, in generator order, into batches of `batch_size` consecutive windows that restart
+    at every change of group (seq_group: one id per sequence).  The masked frames of such a batch, flattened window-major
+    as evaluate() flattens them (RUN:589-596), are the packed frames [run_start[r], run_start[r + 1]): the windows do
+    not overlap once the back-shifted last window's target_mask is applied, and sequences are packed back to back.
+    Returns (run_start int64 [R + 1], run_group int32 [R]); the runs tile [0, N).  Raises ValueError when the
+    sequences of a group are not consecutive: the reference never batches such sequences together."""
+    if batch_size < 1:
+        raise ValueError("batch_size must be positive")
+    grp = torch.as_tensor(seq_group, dtype=torch.int64).reshape(-1)
+    if grp.numel() != len(seq_lengths):
+        raise ValueError("seq_group must have one entry per sequence")
+    if grp.numel():
+        first = torch.ones(grp.numel(), dtype=torch.bool)
+        first[1:] = grp[1:] != grp[:-1]
+        if torch.unique(grp[first]).numel() != int(first.sum()):
+            raise ValueError("the sequences of a group must be consecutive in the packing")
+    ws, fv, sid = plan_windows(seq_lengths, F)
+    n_win = ws.numel()
+    wg = grp[sid.long()]
+    idx = torch.arange(n_win)
+    new_block = torch.ones(n_win, dtype=torch.bool)
+    new_block[1:] = wg[1:] != wg[:-1]
+    block_start = torch.cummax(torch.where(new_block, idx, torch.zeros_like(idx)), 0).values if n_win else idx
+    head = (idx - block_start) % batch_size == 0                     # first window of every batch
+    n_total = int(sum(int(n) for n in seq_lengths))
+    run_start = torch.cat([ws[head] + fv[head].long(), torch.tensor([n_total], dtype=torch.int64)])
+    return run_start, wg[head].to(torch.int32)
 
 
 class DeviceSampler:
@@ -199,6 +231,55 @@ def mpi3dhp_metrics(engine: Engine, pred: torch.Tensor, gt: torch.Tensor, *, mm_
             "joint_groups": {name: in_mm(table(joints)["all"]) for name, joints in MPI3DHP_JOINT_GROUPS.items()}}
 
 
+def h36m_metrics(engine: Engine, pred: torch.Tensor, gt: torch.Tensor, seq_lengths: Sequence[int],
+                 seq_action: Sequence[int], *, F: int, batch_size: int, mm_per_unit: float,
+                 action_names: Optional[Sequence] = None) -> Dict:
+    """The Human3.6M per-action table (RUN:730-736, 602-614) on the device, from the packed pred / gt [N, J, 3] of
+    `evaluate_sequences` (sequences back to back, N = sum(seq_lengths)).  seq_action: the action id of every sequence,
+    in [0, G), G = len(action_names) (default: max id + 1, names 0..G-1); an action's sequences must be consecutive.
+    Every batch the reference's per-action loader would form (`loader_batch_runs`, `batch_size` windows of F frames) is
+    one `Engine.pose_metrics_accumulate` call on its run of frames into the action's fp64 accumulator, so MPJPE,
+    N-MPJPE, P-MPJPE and the velocity error carry evaluate()'s `N_b` weighting; all calls are enqueued on the current
+    stream and the accumulators come back in one copy.  mm_per_unit: 1000 for poses in metres, 1 for millimetres.
+    Returns {'actions': {name: row}, 'action_mean': row, 'pooled': row}, a row being {'mpjpe', 'p_mpjpe', 'n_mpjpe',
+    'velocity'} in mm and 'frames'.  'action_mean' is the unweighted mean of the rows of the actions that have frames
+    (the reference's mean over its actions), 'pooled' sums the accumulators before dividing.  A row without frames
+    is NaN.  A batch of a single frame adds no velocity term (the reference's numpy mean over no difference is NaN)."""
+    if not mm_per_unit > 0:
+        raise ValueError("mm_per_unit must be positive")
+    act = torch.as_tensor(seq_action, dtype=torch.int64).reshape(-1)
+    G = len(action_names) if action_names is not None else (int(act.max()) + 1 if act.numel() else 0)
+    names = list(range(G)) if action_names is None else list(action_names)
+    if act.numel() and (int(act.min()) < 0 or int(act.max()) >= G):
+        raise ValueError("seq_action must lie in [0, number of actions)")
+    run_start, run_group = loader_batch_runs(seq_lengths, act, F, batch_size)
+    N = int(run_start[-1])
+    if tuple(pred.shape) != (N, engine.J, 3):
+        raise ValueError(f"pred must have shape {(N, engine.J, 3)} (sum of seq_lengths frames), got {tuple(pred.shape)}")
+    dev = engine.device
+    pred, gt = pred.contiguous(), gt.to(dev).contiguous()
+    acc = torch.zeros((G, 6), device=dev, dtype=torch.float64)
+    bounds = run_start.tolist()
+    for r, g in enumerate(run_group.tolist()):
+        a, b = bounds[r], bounds[r + 1]
+        engine.pose_metrics_accumulate(pred[a:b], gt[a:b], acc[g])
+    acc = acc.cpu()
+
+    def row(a):
+        if a[5].item() == 0:
+            vals = (float("nan"),) * 4
+        else:
+            vals = tuple(v * mm_per_unit for v in Engine.pose_metrics(a))
+        return dict(zip(("mpjpe", "p_mpjpe", "n_mpjpe", "velocity"), vals), frames=int(a[5].item()))
+
+    rows = [row(acc[g]) for g in range(G)]
+    have = [r for r in rows if r["frames"]]
+    keys = ("mpjpe", "p_mpjpe", "n_mpjpe", "velocity")
+    mean = {k: (sum(r[k] for r in have) / len(have) if have else float("nan")) for k in keys}
+    return {"actions": dict(zip(names, rows)), "action_mean": dict(mean, frames=sum(r["frames"] for r in have)),
+            "pooled": row(acc.sum(dim=0))}
+
+
 def gather_results(local_pred: torch.Tensor, acc: torch.Tensor, n_total: int, group=None):
     """The single exchange step: all-gather of the (padded) prediction shards + all-reduce(sum) of the fp64
     (error sum, joint count) pair.  Returns (pred [n_total,F,J,3] on every rank, mpjpe float)."""
@@ -220,3 +301,33 @@ def gather_results(local_pred: torch.Tensor, acc: torch.Tensor, n_total: int, gr
         parts.append(bucket[r * per: r * per + c])
     cnt = acc[1].item()
     return torch.cat(parts), (acc[0].item() / cnt if cnt else float("nan"))
+
+
+def _all_gather(bucket: torch.Tensor, local: torch.Tensor, group):
+    world = dist.get_world_size(group)
+    if bucket.is_cuda:
+        dist.all_gather_into_tensor(bucket, local, group=group)
+    else:
+        dist.all_gather(list(bucket.view(world, *local.shape).unbind(0)), local, group=group)
+
+
+def gather_packed(local_pred: torch.Tensor, group=None) -> torch.Tensor:
+    """All-gather of packed predictions [n_r, ...] whose frame count n_r differs per rank (each rank's sequences of
+    `evaluate_sequences`): the counts first, then every shard padded to the largest, gathered and unpadded in rank
+    order.  When rank r owns a contiguous block of whole sequences (`shard_range` over sequences) the result is the
+    global packed array, on every rank.  NCCL on GPUs, gloo for CPU tensors."""
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+        return local_pred
+    world = dist.get_world_size(group)
+    n = torch.tensor([local_pred.shape[0]], device=local_pred.device, dtype=torch.int64)
+    counts = torch.empty(world, device=local_pred.device, dtype=torch.int64)
+    _all_gather(counts, n, group)
+    counts = counts.tolist()
+    per, tail = max(counts), tuple(local_pred.shape[1:])
+    if per == 0:
+        return local_pred
+    pad =torch.zeros((per,) + tail, device=local_pred.device, dtype=local_pred.dtype)
+    pad[: local_pred.shape[0]] = local_pred
+    bucket = torch.empty((world * per,) + tail, device=local_pred.device, dtype=local_pred.dtype)
+    _all_gather(bucket, pad, group)
+    return torch.cat([bucket[r * per: r * per + c] for r, c in enumerate(counts)])
