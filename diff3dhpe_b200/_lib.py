@@ -62,11 +62,6 @@ PROTOTYPES = {
     "d3d_profile_end": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
     "d3d_op_linear": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                 C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
-    "d3d_op_linear_ln": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                   C.c_float, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
-    "d3d_op_linear_dln_linear": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                           C.c_void_p, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                           C.c_int64, C.c_int32, C.c_void_p]),
     "d3d_op_linear_bench": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                       C.POINTER(C.c_float)]),
     "d3d_op_layernorm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.c_int64,

@@ -40,10 +40,6 @@ struct Blk {
   Lin qkv, proj, fc1, fc2;
   float *tw = nullptr, *tb = nullptr;   // per-block time Linear(1024 -> 512), fp32
   bool have_t = false;
-  // deferred norm2 (d3d_handle::defer_ln2): the raw fc1 weight stays on the device so that it can be re-folded with
-  // norm2.weight whenever either is (re)loaded; fc1_s = column sums of the folded weight, fc1_c = folded bias
-  float *fc1_raw = nullptr, *fc1_s = nullptr, *fc1_c = nullptr;
-  bool fold_dirty = false;
 };
 
 struct OperandBuf {   // a GEMM A operand living in the workspace
@@ -75,10 +71,6 @@ struct d3d_handle {
   float* X = nullptr;
   __half* QKV = nullptr;     // packed fp16 q | k | v_hi | v_lo, [tok_cap, 2048]
   OperandBuf A, ATT, H;
-  // Deferred norm2 (FMT_F4C tcgen05 path): the proj epilogue emits x itself as fc1's A operand plus per-row partial sums
-  // (EPI_F32_EMIT), the fc1 epilogue applies the LayerNorm (EPI_GELU_DLN); no ln_split pass (DESIGN.md 4.1)
-  bool defer_ln2 = false;
-  float2* ln_stats = nullptr;   // [8][tok_cap] (sum, sum of squares) per 64 columns
   CUtensorMap m_x;              // fp32 [tok_cap, 512] view of X in {32 x 32} boxes: destination of the EPI_F32_RED epilogue
   bool have_m_x = false;
   AttnTcMaps attn_tc;        // tcgen05 temporal attention: maps bound to QKV -> ATT
@@ -258,62 +250,21 @@ int pick_bn(const d3d_handle* h, int64_t M, int N) {
   return tiles256 >= 2 * h->num_sms ? 256 : 128;
 }
 
-struct LnFuse {           // LayerNorm fused behind an EPI_F32 GEMM (EPI_F32_LN): parameters and destination operand
-  const float* gamma;
-  const float* beta;
-  float eps;
-  OperandBuf* dst;
-};
-
-// proj + norm2 in one kernel: CTA-pair F8C tcgen05 GEMM with the n-inner tile order only
-bool can_fuse_ln(const d3d_handle* h, int mode) {
-  return mode == D3D_GEMM_TC_F8C && h->fmt == FMT_F8C && pick_cg(kC) == 2 && env_int("D3D_GEMM_N_INNER", 1) == 1;
-}
-// OFF by default.  Measured on B200 at cfg3 (profiles/r01s_bench_fuse*.json): correct, but SLOWER -- GEMM class
-// 2727 -> 3069 ms per step for 198 ms of LayerNorm kernels saved (3802 -> 3943 ms per step).  Between its two passes
-// the epilogue holds BOTH accumulators, so its residual loads / operand stores are no longer hidden behind the next
-// tile's mainloop (~15 us per 128 x 256 pass with 8 warps, against 17 us of mainloop per row tile).
-bool fuse_ln_enabled() { return env_int("D3D_GEMM_FUSE_LN", 0) == 1; }
-
-struct DeferLn {          // deferred LayerNorm (EPI_F32_EMIT producer / EPI_GELU_DLN consumer)
-  const OperandBuf* emit; // EPI_F32_EMIT: destination operand of x
-  float2* stats;
-  const float* colsum;    // EPI_GELU_DLN
-  const float* cbias;     // EPI_GELU_DLN: folded bias (replaces the Linear's own)
-  float eps;
-};
-
 // out = epilogue(Aop . W^T + bias)
 int run_gemm(d3d_handle* h, const OperandBuf& a, const Lin& w, int64_t M, int epi, const float* residual,
              float* out_f32, __half* out_hi, __half* out_lo, __half* out_qkv, int mode, cudaStream_t st,
-             const LnFuse* ln = nullptr, uint8_t* out_sf = nullptr, const DeferLn* dl = nullptr,
-             const CUtensorMap* out_map = nullptr) {
+             uint8_t* out_sf = nullptr, const CUtensorMap* out_map = nullptr) {
   GemmParams p{};
   // in-place residual update on the F4C tcgen05 kernel: let the L2 do the add (TMA reduction) instead of pulling the
   // residual rows into the SM (D3D_GEMM_RED=0: the load-add-store epilogue)
-  if (epi == EPI_F32 && !ln && out_map && residual && residual == out_f32 && mode == D3D_GEMM_TC_F4C && pick_cg(w.N) == 2 &&
+  if (epi == EPI_F32 && out_map && residual && residual == out_f32 && mode == D3D_GEMM_TC_F4C && pick_cg(w.N) == 2 &&
       env_int("D3D_GEMM_RED", 1) == 1)
     epi = EPI_F32_RED;
   p.out_sf = out_sf;
-  if (dl) {
-    if (mode != D3D_GEMM_TC_F4C) return fail(h, -3, "the deferred-LayerNorm epilogues need the F4C tcgen05 GEMM");
-    p.ln_stats = dl->stats;
-    p.ln_eps = dl->eps;
-    if (epi == EPI_F32_EMIT) {
-      p.emit_hi = dl->emit->hi; p.emit_c4 = reinterpret_cast<uint8_t*>(dl->emit->lo); p.emit_sf = dl->emit->sf;
-    } else {
-      p.ln_colsum = dl->colsum;
-    }
-  }
-  if (ln) {
-    epi = EPI_F32_LN;
-    p.ln_gamma = ln->gamma; p.ln_beta = ln->beta; p.ln_eps = ln->eps;
-    p.ln_hi = ln->dst->hi; p.ln_second = ln->dst->lo;
-  }
   p.M = static_cast<int>(M);
   p.N = w.N;
   p.K = w.K;
-  p.bias = (dl && epi == EPI_GELU_DLN) ? dl->cbias : w.bias;
+  p.bias = w.bias;
   p.residual = residual;
   p.out_f32 = out_f32;
   p.out_hi = out_hi;
@@ -342,11 +293,10 @@ int run_gemm(d3d_handle* h, const OperandBuf& a, const Lin& w, int64_t M, int ep
     // epilogue warps per CTA: 16 pays where the epilogue, not the mainloop, sets the tile time
     // GELU epilogue: 16 warps.  After the epilogue diet 8 warps (one more ring stage) are 2 % faster on the isolated fc1
     // launch (r02r) but 1 % slower in the step (r02s: GEMM class 2157 vs 2139 ms on one box)
-    const int ew = (epi == EPI_GELU_SPLIT || epi == EPI_GELU_DLN) ? env_int("D3D_GEMM_EW_GELU", 16)
-                 : epi == EPI_QKV16    ? env_int("D3D_GEMM_EW_QKV", 8)
-                 : epi == EPI_F32_EMIT ? env_int("D3D_GEMM_EW_EMIT", 8)
-                 : epi == EPI_F32_RED  ? 8
-                                        : env_int("D3D_GEMM_EW_F32", 8);
+    const int ew = epi == EPI_GELU_SPLIT ? env_int("D3D_GEMM_EW_GELU", 16)
+                 : epi == EPI_QKV16      ? env_int("D3D_GEMM_EW_QKV", 8)
+                 : epi == EPI_F32_RED    ? 8
+                                         : env_int("D3D_GEMM_EW_F32", 8);
     // D3D_GEMM_SMS: run the persistent GEMM on fewer SMs (diagnostic: is the operand feed limited per SM or chip-wide?)
     const int sms = env_int("D3D_GEMM_SMS", h->num_sms);
     KLP(D3D_PROF_GEMM, st, launch_gemm_tc(m, p, epi, passes, pick_bn(h, M, w.N), pick_cg(w.N), pick_cs(M), ew,
@@ -422,8 +372,6 @@ int check_weights(d3d_handle* h) {
     }
   for (auto& n : need)
     if (!h->loaded.count(n)) return fail(h, -30, "weights not loaded: missing tensor '" + n + "'");
-  for (auto& b : h->blk)
-    if (b.fold_dirty) return fail(h, -30, "internal: norm2 / fc1 of a block were not folded");
   return 0;
 }
 
@@ -478,21 +426,11 @@ int run_blocks(d3d_handle* h, const float* x2d, const float* y, const float* x5,
     const bool spatial = (b % 2) == 0;
     if ((r = run_gemm(h, h->A, k.qkv, T, EPI_QKV16, nullptr, nullptr, nullptr, nullptr, h->QKV, gm, st))) return r;
     if ((r = run_attention(h, h->QKV, h->ATT.hi, h->ATT.lo, nullptr, B, spatial, am, st))) return r;
-    if (fuse_ln_enabled() && can_fuse_ln(h, gm)) {        // proj + residual + norm2 (MODEL:127-128) in one kernel
-      const LnFuse ln2{k.n2g, k.n2b, 1e-6f, &h->A};
-      if ((r = run_gemm(h, h->ATT, k.proj, T, EPI_F32, h->X, h->X, nullptr, nullptr, nullptr, gm, st, &ln2))) return r;
-    } else if (h->defer_ln2) {                            // proj + residual emits x as fc1's operand; fc1 applies norm2
-      const DeferLn dl{&h->A, h->ln_stats, k.fc1_s, k.fc1_c, 1e-6f};
-      if ((r = run_gemm(h, h->ATT, k.proj, T, EPI_F32_EMIT, h->X, h->X, nullptr, nullptr, nullptr, gm, st, nullptr, nullptr, &dl))) return r;
-      if ((r = run_gemm(h, h->A, k.fc1, T, EPI_GELU_DLN, nullptr, nullptr, h->H.hi, h->H.lo, nullptr, gm, st, nullptr, h->H.sf, &dl))) return r;
-    } else {
-      if ((r = run_gemm(h, h->ATT, k.proj, T, EPI_F32, h->X, h->X, nullptr, nullptr, nullptr, gm, st, nullptr, nullptr, nullptr,
-                        h->have_m_x ? &h->m_x : nullptr))) return r;
-      if ((r = norm2_launch(h, b, T, st))) return r;
-    }
-    if (!h->defer_ln2 &&
-        (r = run_gemm(h, h->A, k.fc1, T, EPI_GELU_SPLIT, nullptr, nullptr, h->H.hi, h->H.lo, nullptr, gm, st, nullptr, h->H.sf))) return r;
-    if ((r = run_gemm(h, h->H, k.fc2, T, EPI_F32, h->X, h->X, nullptr, nullptr, nullptr, gm, st, nullptr, nullptr, nullptr,
+    if ((r = run_gemm(h, h->ATT, k.proj, T, EPI_F32, h->X, h->X, nullptr, nullptr, nullptr, gm, st, nullptr,
+                      h->have_m_x ? &h->m_x : nullptr))) return r;
+    if ((r = norm2_launch(h, b, T, st))) return r;
+    if ((r = run_gemm(h, h->A, k.fc1, T, EPI_GELU_SPLIT, nullptr, nullptr, h->H.hi, h->H.lo, nullptr, gm, st, h->H.sf))) return r;
+    if ((r = run_gemm(h, h->H, k.fc2, T, EPI_F32, h->X, h->X, nullptr, nullptr, nullptr, gm, st, nullptr,
                       h->have_m_x ? &h->m_x : nullptr))) return r;
     if (b + 1 < n_blocks && (r = postnorm_launch(h, b + 1, tv, tv_stride, T, st))) return r;
   }
@@ -623,10 +561,6 @@ int d3d_create(const d3d_config* cfg, d3d_handle** out) {
   d3d_handle* h = new d3d_handle();
   h->cfg = *cfg;
   h->fmt = mode_fmt(cfg->gemm_mode);
-  // OFF by default (D3D_DEFER_LN2=1 enables it): measured on B200 at cfg3 (profiles/r02j_*): with the residual update of
-  // proj done by the L2 (EPI_F32_RED) the separate norm2 pass is cheaper than the emitting epilogue, which has to pull
-  // the residual rows into the SM -- 3183 ms per step (RED + norm2 kernel) against 3217 ms (EMIT + DLN)
-  h->defer_ln2 = cfg->gemm_mode == D3D_GEMM_TC_F4C && env_int("D3D_DEFER_LN2", 0) == 1 && pick_cg(kC) == 2;
   h->F = cfg->num_frame;
   h->J = cfg->num_joints;
   h->nblk = 2 * cfg->depth;
@@ -653,11 +587,6 @@ int d3d_create(const d3d_config* cfg, d3d_handle** out) {
       for (float** p : {&b.n1g, &b.n1b, &b.n2g, &b.n2b, &b.tb})
         if ((r = dev_alloc(h, p, kC))) return r;
       if ((r = dev_alloc(h, &b.tw, static_cast<int64_t>(kC) * 2 * kC))) return r;
-      if (h->defer_ln2) {
-        if ((r = dev_alloc(h, &b.fc1_raw, static_cast<int64_t>(kHidden) * kC))) return r;
-        if ((r = dev_alloc(h, &b.fc1_s, kHidden))) return r;
-        if ((r = dev_alloc(h, &b.fc1_c, kHidden))) return r;
-      }
     }
     for (float** p : {&h->bf, &h->sn_g, &h->sn_b, &h->tn_g, &h->tn_b, &h->hg, &h->hb})
       if ((r = dev_alloc(h, p, kC))) return r;
@@ -679,7 +608,6 @@ int d3d_create(const d3d_config* cfg, d3d_handle** out) {
     if ((r = alloc_operand(h, &h->A, h->tok_cap, kC))) return r;
     if ((r = alloc_operand(h, &h->ATT, h->tok_cap, kC))) return r;
     if ((r = alloc_operand(h, &h->H, h->tok_cap, kHidden))) return r;
-    if (h->defer_ln2 && (r = dev_alloc(h, &h->ln_stats, 8 * h->tok_cap))) return r;
     if (h->J == 17) {
       if (make_attn_tc_maps_spatial(&h->attn_sp, h->QKV, h->ATT.hi, h->ATT.lo, h->fmt, h->tok_cap, h->F))
         return fail(h, -20, "cuTensorMapEncodeTiled failed for the spatial-attention maps");
@@ -741,8 +669,9 @@ int d3d_load_weights(d3d_handle* h, const d3d_tensor* tensors, int32_t n) {
     CK(cudaMemcpy(dst, t.data, expect * sizeof(float), t.on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice));
     return 0;
   };
-  // split the fp32 weight in `stage` into the operand arrays of l, with the range guard
-  auto split_stage = [&](Lin& l, const std::string& tname) -> int {
+  auto load_lin_w = [&](Lin& l, const d3d_tensor& t) -> int {
+    int r = copy_to(stage, t, static_cast<int64_t>(l.N) * l.K);
+    if (r) return r;
     CK(cudaMemset(h->absmax_dev, 0, 2 * sizeof(float)));
     CK(launch_split(stage, l.hi, l.lo, l.sf, l.N, l.K, h->fmt, 1, 0, h->absmax_dev));
     CK(cudaDeviceSynchronize());
@@ -751,17 +680,12 @@ int d3d_load_weights(d3d_handle* h, const d3d_tensor* tensors, int32_t n) {
     // over finite values, [1] = 1 when a NaN / Inf was seen.
     float am[2] = {0.f, 0.f};
     CK(cudaMemcpy(am, h->absmax_dev, sizeof(am), cudaMemcpyDeviceToHost));
-    if (am[1] != 0.f) return fail(h, -12, std::string("tensor '") + tname + "' holds NaN / Inf");
+    if (am[1] != 0.f) return fail(h, -12, std::string("tensor '") + t.name + "' holds NaN / Inf");
     if (am[0] > kMaxWeightAbs)
-      return fail(h, -12, std::string("tensor '") + tname + "': max |w| = " + std::to_string(am[0]) +
+      return fail(h, -12, std::string("tensor '") + t.name + "': max |w| = " + std::to_string(am[0]) +
                               " exceeds the fp16 operand range (" + std::to_string(kMaxWeightAbs) + ")");
     l.have_w = true;
     return 0;
-  };
-  auto load_lin_w = [&](Lin& l, const d3d_tensor& t) -> int {
-    int r = copy_to(stage, t, static_cast<int64_t>(l.N) * l.K);
-    if (r) return r;
-    return split_stage(l, t.name);
   };
 
   for (int i = 0; i < n; ++i) {
@@ -803,16 +727,14 @@ int d3d_load_weights(d3d_handle* h, const d3d_tensor* tensors, int32_t n) {
       const std::string sub = name.substr(dot + 1);
       if (sub == "norm1.weight") r = copy_to(b.n1g, t, kC);
       else if (sub == "norm1.bias") r = copy_to(b.n1b, t, kC);
-      else if (sub == "norm2.weight") { r = copy_to(b.n2g, t, kC); b.fold_dirty = h->defer_ln2; }
-      else if (sub == "norm2.bias") { r = copy_to(b.n2b, t, kC); b.fold_dirty = h->defer_ln2; }
+      else if (sub == "norm2.weight") r = copy_to(b.n2g, t, kC);
+      else if (sub == "norm2.bias") r = copy_to(b.n2b, t, kC);
       else if (sub == "attn.qkv.weight") r = load_lin_w(b.qkv, t);
       else if (sub == "attn.qkv.bias") r = copy_to(b.qkv.bias, t, 3 * kC);
       else if (sub == "attn.proj.weight") r = load_lin_w(b.proj, t);
       else if (sub == "attn.proj.bias") r = copy_to(b.proj.bias, t, kC);
-      else if (sub == "mlp.fc1.weight") {
-        if (h->defer_ln2) { r = copy_to(b.fc1_raw, t, static_cast<int64_t>(kHidden) * kC); b.fold_dirty = true; }
-        else r = load_lin_w(b.fc1, t);
-      } else if (sub == "mlp.fc1.bias") { r = copy_to(b.fc1.bias, t, kHidden); b.fold_dirty = h->defer_ln2; }
+      else if (sub == "mlp.fc1.weight") r = load_lin_w(b.fc1, t);
+      else if (sub == "mlp.fc1.bias") r = copy_to(b.fc1.bias, t, kHidden);
       else if (sub == "mlp.fc2.weight") r = load_lin_w(b.fc2, t);
       else if (sub == "mlp.fc2.bias") r = copy_to(b.fc2.bias, t, kC);
       else if (sub == "time_mlp.1.weight") r = copy_to(b.tw, t, static_cast<int64_t>(kC) * 2 * kC);
@@ -823,19 +745,6 @@ int d3d_load_weights(d3d_handle* h, const d3d_tensor* tensors, int32_t n) {
     }
     if (r) return r;
     h->loaded[name] = true;
-  }
-  // deferred norm2: (re)fold every block whose norm2 / fc1 tensors changed, once all four are present
-  for (int bi = 0; bi < h->nblk; ++bi) {
-    Blk& b = h->blk[bi];
-    if (!b.fold_dirty) continue;
-    const std::string pre = std::string(bi % 2 == 0 ? "STEblocks." : "TTEblocks.") + std::to_string(bi / 2) + ".";
-    bool all = true;
-    for (const char* s : {"norm2.weight", "norm2.bias", "mlp.fc1.weight", "mlp.fc1.bias"}) all = all && h->loaded.count(pre + s);
-    if (!all) continue;
-    CK(launch_fold_ln_linear(b.fc1_raw, b.n2g, b.n2b, b.fc1.bias, stage, b.fc1_s, b.fc1_c, kHidden, kC, 0));
-    int r = split_stage(b.fc1, pre + "mlp.fc1.weight (folded with norm2.weight)");
-    if (r) return r;
-    b.fold_dirty = false;
   }
   CK(cudaDeviceSynchronize());
   return 0;
@@ -1323,77 +1232,17 @@ int d3d_op_linear(d3d_handle* h, const float* a, const float* w, const float* bi
   KL(launch_split(a, b.a.hi, b.a.lo, b.a.sf, M, K, fmt, 0, st));
   KL(launch_split(w, b.w.hi, b.w.lo, b.w.sf, N, K, fmt, 1, st));
   if (act) {
-    if ((r = run_gemm(h, b.a, b.w, M, EPI_GELU_SPLIT, nullptr, nullptr, b.o_hi, b.o_lo, nullptr, gemm_mode, st, nullptr, b.o_sf))) return r;
+    if ((r = run_gemm(h, b.a, b.w, M, EPI_GELU_SPLIT, nullptr, nullptr, b.o_hi, b.o_lo, nullptr, gemm_mode, st, b.o_sf))) return r;
     KL(launch_merge(b.o_hi, b.o_lo, b.o_sf, out, M, N, fmt, st));
   } else if (residual && gemm_mode == D3D_GEMM_TC_F4C && N % 256 == 0 && env_int("D3D_GEMM_RED", 1) == 1) {
     // as the sampler runs proj / fc2: the residual already sits in `out`, the epilogue reduce-adds into it
     CUtensorMap om;
     if (make_f32_tile_map(&om, out, M, N)) return fail(h, -20, "cuTensorMapEncodeTiled failed");
     CK(cudaMemcpyAsync(out, residual, static_cast<size_t>(M) * N * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    if ((r = run_gemm(h, b.a, b.w, M, EPI_F32, out, out, nullptr, nullptr, nullptr, gemm_mode, st, nullptr, nullptr, nullptr, &om))) return r;
+    if ((r = run_gemm(h, b.a, b.w, M, EPI_F32, out, out, nullptr, nullptr, nullptr, gemm_mode, st, nullptr, &om))) return r;
   } else {
     if ((r = run_gemm(h, b.a, b.w, M, EPI_F32, residual, out, nullptr, nullptr, nullptr, gemm_mode, st))) return r;
   }
-  CK(cudaStreamSynchronize(st));
-  return 0;
-}
-
-int d3d_op_linear_ln(d3d_handle* h, const float* a, const float* w, const float* bias, const float* residual,
-                     const float* gamma, const float* beta, float eps, float* x_out, float* ln_out, int64_t M, int32_t K,
-                     void* stream) {
-  if (!h || !a || !w || !bias || !residual || !gamma || !beta || !x_out || !ln_out) return -1;
-  if (M < 1 || K % 64 != 0 || K < 64) return fail(h, -2, "need M>=1, K%64==0");
-  if (!can_fuse_ln(h, D3D_GEMM_TC_F8C)) return fail(h, -3, "the fused GEMM + LayerNorm epilogue needs the F8C CTA-pair kernel");
-  DeviceGuard guard(h->cfg.device);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  OpLinearBufs b;
-  int r = prep_op_linear(h, b, M, kC, K, 1 /*allocates o_hi / o_lo [M, 512]*/, FMT_F8C);
-  if (r) return r;
-  b.w.bias = const_cast<float*>(bias);
-  KL(launch_split(a, b.a.hi, b.a.lo, nullptr, M, K, FMT_F8C, 0, st));
-  KL(launch_split(w, b.w.hi, b.w.lo, nullptr, kC, K, FMT_F8C, 1, st));
-  OperandBuf dst;
-  dst.hi = b.o_hi;
-  dst.lo = b.o_lo;
-  const LnFuse ln{gamma, beta, eps, &dst};
-  if ((r = run_gemm(h, b.a, b.w, M, EPI_F32, residual, x_out, nullptr, nullptr, nullptr, D3D_GEMM_TC_F8C, st, &ln))) return r;
-  KL(launch_merge(b.o_hi, b.o_lo, nullptr, ln_out, M, kC, FMT_F8C, st));
-  CK(cudaStreamSynchronize(st));
-  return 0;
-}
-
-int d3d_op_linear_dln_linear(d3d_handle* h, const float* a, const float* w, const float* bias, const float* residual,
-                             const float* gamma, const float* beta, float eps, const float* w2, const float* b2,
-                             float* x_out, float* hid_out, int64_t M, int32_t K, void* stream) {
-  if (!h || !a || !w || !bias || !residual || !gamma || !beta || !w2 || !b2 || !x_out || !hid_out) return -1;
-  if (M < 1 || K % 128 != 0 || K < 128) return fail(h, -2, "need M>=1, K%128==0");
-  if (pick_cg(kC) != 2) return fail(h, -3, "the deferred-LayerNorm epilogues need the CTA-pair kernel");
-  DeviceGuard guard(h->cfg.device);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  OpLinearBufs b1, b2b;
-  int r = prep_op_linear(h, b1, M, kC, K, 1 /*o_hi / o_lo [M,512]: the emitted operand*/, FMT_F4C);
-  if (r) return r;
-  if ((r = prep_op_linear(h, b2b, M, kHidden, kC, 1, FMT_F4C))) return r;
-  const int64_t Mp = (M + 511) / 512 * 512;
-  float2* stats = nullptr;
-  float *wfold = nullptr, *colsum = nullptr, *cbias = nullptr;
-  CK(tmp_alloc(b1, &stats, 8 * Mp));
-  CK(tmp_alloc(b1, &wfold, static_cast<int64_t>(kHidden) * kC));
-  CK(tmp_alloc(b1, &colsum, kHidden));
-  CK(tmp_alloc(b1, &cbias, kHidden));
-  b1.w.bias = const_cast<float*>(bias);
-  b2b.w.bias = const_cast<float*>(b2);
-  KL(launch_split(a, b1.a.hi, b1.a.lo, b1.a.sf, M, K, FMT_F4C, 0, st));
-  KL(launch_split(w, b1.w.hi, b1.w.lo, b1.w.sf, kC, K, FMT_F4C, 1, st));
-  KL(launch_fold_ln_linear(w2, gamma, beta, b2, wfold, colsum, cbias, kHidden, kC, st));
-  KL(launch_split(wfold, b2b.w.hi, b2b.w.lo, b2b.w.sf, kHidden, kC, FMT_F4C, 1, st));
-  CK(cudaMemcpyAsync(x_out, residual, static_cast<size_t>(M) * kC * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  // the emitted operand of the first GEMM IS the A operand of the second: give it the second one's tensor maps
-  OperandBuf mid = b2b.a;
-  const DeferLn dl{&mid, stats, colsum, cbias, eps};
-  if ((r = run_gemm(h, b1.a, b1.w, M, EPI_F32_EMIT, x_out, x_out, nullptr, nullptr, nullptr, D3D_GEMM_TC_F4C, st, nullptr, nullptr, &dl))) return r;
-  if ((r = run_gemm(h, mid, b2b.w, M, EPI_GELU_DLN, nullptr, nullptr, b2b.o_hi, b2b.o_lo, nullptr, D3D_GEMM_TC_F4C, st, nullptr, b2b.o_sf, &dl))) return r;
-  KL(launch_merge(b2b.o_hi, b2b.o_lo, b2b.o_sf, hid_out, M, kHidden, FMT_F4C, st));
   CK(cudaStreamSynchronize(st));
   return 0;
 }
@@ -1406,21 +1255,10 @@ int d3d_op_linear_bench(d3d_handle* h, int64_t M, int32_t N, int32_t K, int32_t 
   cudaStream_t st = h->cap_stream;
   OpLinearBufs b;
   const int fmt = mode_fmt(gemm_mode);
-  // act: 0 fp32 out, 1 GELU -> operand, 2 fp32 out + in-place residual, 3 = 2 + emitted operand + row statistics
-  // (EPI_F32_EMIT), 4 GELU with the deferred LayerNorm (EPI_GELU_DLN)
-  if (act < 0 || act > 4) return fail(h, -2, "act out of range");
-  if (act >= 3 && gemm_mode != D3D_GEMM_TC_F4C) return fail(h, -3, "act 3 / 4 need D3D_GEMM_TC_F4C");
+  // act: 0 fp32 out, 1 GELU -> operand, 2 fp32 out + in-place residual
+  if (act < 0 || act > 2) return fail(h, -2, "act out of range");
   int r = prep_op_linear(h, b, M, N, K, act == 2 ? 0 : act, fmt);
   if (r) return r;
-  const int64_t Mp = (M + 511) / 512 * 512;
-  float2* stats = nullptr;
-  float* colsum = nullptr;
-  OperandBuf emit;
-  if (act >= 3) {
-    CK(tmp_alloc(b, &stats, 8 * Mp));
-    CK(tmp_alloc(b, &colsum, N));
-    emit.hi = b.o_hi; emit.lo = b.o_lo; emit.sf = b.o_sf;
-  }
   float *fa = nullptr, *fo = nullptr, *fb = nullptr;
   CK(tmp_alloc(b, &fa, M * K > static_cast<int64_t>(N) * K ? M * K : static_cast<int64_t>(N) * K));
   CK(tmp_alloc(b, &fo, M * N));
@@ -1437,14 +1275,11 @@ int d3d_op_linear_bench(d3d_handle* h, int64_t M, int32_t N, int32_t K, int32_t 
   cudaEvent_t e0, e1;
   CK(cudaEventCreate(&e0));
   CK(cudaEventCreate(&e1));
-  const DeferLn dl{&emit, stats, colsum, fb, 1e-6f};
   CUtensorMap fo_map;
   if (make_f32_tile_map(&fo_map, fo, M, N)) return fail(h, -20, "cuTensorMapEncodeTiled failed");
   auto once = [&]() -> int {
-    if (act == 1) return run_gemm(h, b.a, b.w, M, EPI_GELU_SPLIT, nullptr, nullptr, b.o_hi, b.o_lo, nullptr, gemm_mode, st, nullptr, b.o_sf);
-    if (act == 2) return run_gemm(h, b.a, b.w, M, EPI_F32, fo, fo, nullptr, nullptr, nullptr, gemm_mode, st, nullptr, nullptr, nullptr, &fo_map);
-    if (act == 3) return run_gemm(h, b.a, b.w, M, EPI_F32_EMIT, fo, fo, nullptr, nullptr, nullptr, gemm_mode, st, nullptr, nullptr, &dl);
-    if (act == 4) return run_gemm(h, b.a, b.w, M, EPI_GELU_DLN, nullptr, nullptr, b.o_hi, b.o_lo, nullptr, gemm_mode, st, nullptr, b.o_sf, &dl);
+    if (act == 1) return run_gemm(h, b.a, b.w, M, EPI_GELU_SPLIT, nullptr, nullptr, b.o_hi, b.o_lo, nullptr, gemm_mode, st, b.o_sf);
+    if (act == 2) return run_gemm(h, b.a, b.w, M, EPI_F32, fo, fo, nullptr, nullptr, nullptr, gemm_mode, st, nullptr, &fo_map);
     return run_gemm(h, b.a, b.w, M, EPI_F32, nullptr, fo, nullptr, nullptr, nullptr, gemm_mode, st);
   };
   for (int i = 0; i < 3; ++i)

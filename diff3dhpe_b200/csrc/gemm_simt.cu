@@ -29,7 +29,7 @@ template <int EPI, int FMT>
 __global__ void __launch_bounds__(256)
 gemm_simt_kernel(const __half* __restrict__ a_hi, const __half* __restrict__ a_lo, const uint8_t* __restrict__ a_sf,
                  const __half* __restrict__ b_hi, const __half* __restrict__ b_lo, const uint8_t* __restrict__ b_sf,
-                 const GemmParams p) {
+                 const __grid_constant__ GemmParams p) {
   __shared__ float As[TK][TM + 1];
   __shared__ float Bs[TK][TN + 1];
   __shared__ float A8[FMT != FMT_SPLIT16 ? 2 * TK : 1][TM + 1];  // F8C: [0,TK) e5m2(a 2^-8), [TK,2TK) e5m2(a_lo 2^4); F4C: P, Q

@@ -30,8 +30,7 @@
 //   * epilogues (kernels.cuh GemmEpi): fp32 (+ residual) through a swizzled transpose buffer; the SHIPPED in-place residual
 //     update of proj / fc2 as a TMA reduction (EPI_F32_RED: the L2 adds, X never enters the SM -- the L2 -> SM operand
 //     feed is what bounds all four GEMMs, DESIGN.md 4.1); q | k | v_hi | v_lo fp16 pack; GELU -> block-scaled operand (1-MUFU
-//     GELU, bias from shared memory, per-lane store addressing); the deferred-LayerNorm pair EPI_F32_EMIT / EPI_GELU_DLN
-//     (measured, off by default).
+//     GELU, bias from shared memory, per-lane store addressing).
 //
 // Warp roles (384 threads): 0 = TMA producer, 1 = MMA issuer (leader CTA), 2 = TMEM allocator, 3 = idle,
 // 4..11 = epilogue (EW = 16: 640 threads, epilogue warps 4..19, setmaxnreg 32 / 112).
@@ -78,8 +77,9 @@ struct Cfg {
   static constexpr int kRing = ((PASSES == 2 || PASSES == 4) ? kSmemBudget : 200 * 1024) + 8 * 4096 - kStagingBytes;   // + 8 KB vectors (F4C)
   static constexpr int kStages = (kRing / kStageBytes) > 8 ? 8 : (kRing / kStageBytes);
   static constexpr int kTmemCols = 2 * BN;   // 256 or 512 (power of two)
-  // FMT_F4C operand-producing epilogues (GELU / deferred LayerNorm) read bias (and the folded weight's column sums) from
-  // shared memory, just in time, instead of holding 32 prefetched registers per lane across the accumulator wait
+  // the FMT_F4C GELU epilogue reads bias from shared memory, just in time, instead of holding 32 prefetched registers per
+  // lane across the accumulator wait.  Only the first 4 KB are used; the second half is spare, kept so that the ring
+  // depth and the shared-memory carve-out of every F4C kernel stay as measured
   static constexpr int kVecBytes = PASSES == 4 ? 2 * 1024 * 4 : 0;
   static constexpr int kSmemBytes = kStages * kStageBytes + kStagingBytes + 1024 /*align*/ + 256 /*barriers*/ + kVecBytes;
   static_assert(kStages >= 2, "need at least a double buffer");
@@ -202,9 +202,11 @@ __device__ __forceinline__ float4 lds_f4(uint32_t addr) {
   return v;
 }
 
+#if !D3D_EPI_PACKED
 __device__ __forceinline__ uint32_t pack_h2(__half a, __half b) {
   return static_cast<uint32_t>(__half_as_ushort(a)) | (static_cast<uint32_t>(__half_as_ushort(b)) << 16);
 }
+#endif
 
 // Coalesced stores of one FMT_F4C staging buffer (32 rows x 128 B: granules 0..3 = 32 hi halves, 4 = 32 P nibbles,
 // 5 = 32 Q nibbles; 8 lanes = one row).  Which array a lane writes depends only on its granule, so base pointer and row
@@ -252,53 +254,6 @@ __device__ __forceinline__ void f4c_store_chunk(const F4cStore& st, uint32_t stg
   }
 }
 
-// FMT_F4C image of one 32 x 32 chunk of fp32 values (lane = row, r = the bits of its 32 consecutive columns = exactly one
-// scale block of each part): hi halves into the staging row (granules 0..3) with the block maxima of x and of x - hi, then
-// both e2m1 images (granule 4 = 32 nibbles of P = q4(x), granule 5 = Q = q4(x - hi)), then the coalesced stores.  The two
-// ue8m0 scale bytes join the lane's words (byte (gcol / 32) % 4); the caller writes them once per tile.
-__device__ __forceinline__ void f4c_emit_chunk(const uint32_t (&r)[32], uint32_t stg, int lane, int row_w, int gcol, int M,
-                                               const F4cStore& st, bool stream_out, uint32_t& sfp_w, uint32_t& sfq_w) {
-  float ax = 0.f, al = 0.f;
-#pragma unroll
-  for (int v = 0; v < 4; ++v) {
-    uint32_t hw[4];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      const float x0 = __uint_as_float(r[8 * v + 2 * e + 0]), x1 = __uint_as_float(r[8 * v + 2 * e + 1]);
-      const __half2 h01 = __floats2half2_rn(x0, x1);
-      const float2 hf = __half22float2(h01);
-      hw[e] = *reinterpret_cast<const uint32_t*>(&h01);
-      ax = fmaxf(ax, fmaxf(fabsf(x0), fabsf(x1)));
-      al = fmaxf(al, fmaxf(fabsf(x0 - hf.x), fabsf(x1 - hf.y)));
-    }
-    stg_st(stg, lane, v, make_uint4(hw[0], hw[1], hw[2], hw[3]));
-  }
-  const uint32_t bp = op_ue8m0_of(ax), bq = op_ue8m0_of(al);
-  const ptx::f32x2 ip = ptx::splat2(op_ue8m0_inv(bp)), iq = ptx::splat2(op_ue8m0_inv(bq));
-  uint32_t pw[4], qw[4];
-#pragma unroll
-  for (int w = 0; w < 4; ++w) {
-    uint32_t pa = 0, qa = 0;
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      const float x0 = __uint_as_float(r[8 * w + 2 * e + 0]), x1 = __uint_as_float(r[8 * w + 2 * e + 1]);
-      const float2 hf = __half22float2(__floats2half2_rn(x0, x1));
-      float a0, a1, l0, l1;
-      ptx::unpack2(ptx::mul2(ptx::pack2(x0, x1), ip), a0, a1);
-      ptx::unpack2(ptx::mul2(ptx::sub2(ptx::pack2(x0, x1), ptx::pack2(hf.x, hf.y)), iq), l0, l1);
-      pa |= op_e2m1x2(a0, a1) << (8 * e);
-      qa |= op_e2m1x2(l0, l1) << (8 * e);
-    }
-    pw[w] = pa; qw[w] = qa;
-  }
-  stg_st(stg, lane, 4, make_uint4(pw[0], pw[1], pw[2], pw[3]));
-  stg_st(stg, lane, 5, make_uint4(qw[0], qw[1], qw[2], qw[3]));
-  sfp_w |= bp << (8 * ((gcol >> 5) & 3));
-  sfq_w |= bq << (8 * ((gcol >> 5) & 3));
-  __syncwarp();
-  f4c_store_chunk(st, stg, lane >> 3, lane & 7, row_w, gcol, M, stream_out);
-}
-
 // CS = CTA pairs per cluster (CG == 2 only).  CS == 2: a cluster of 4 CTAs owns two vertically adjacent 256 x 256
 // tiles (same weight rows).  Each CTA loads only HALF of its 128-row weight tile and TMA-multicasts it to the CTA
 // with the same position in the other pair, so the L2 -> SM weight traffic per MAC halves (48 KB instead of 64 KB
@@ -308,23 +263,20 @@ __global__ void __launch_bounds__(128 + 32 * EW, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
                const __grid_constant__ CUtensorMap tm_b_hi, const __grid_constant__ CUtensorMap tm_b_lo,
                const __grid_constant__ CUtensorMap tm_a_sf, const __grid_constant__ CUtensorMap tm_b_sf,
-               const __grid_constant__ CUtensorMap tm_out, const GemmParams p) {
+               const __grid_constant__ CUtensorMap tm_out, const __grid_constant__ GemmParams p) {
   using C = Cfg<CG, BN, PASSES, EW>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* staging = smem + C::kStages * C::kStageBytes;
   Barriers* bars = reinterpret_cast<Barriers*>(staging + C::kStagingBytes);
-  float* sm_bias = reinterpret_cast<float*>(staging + C::kStagingBytes + 256);      // [1024] bias, [1024] column sums
-  float* sm_colsum = sm_bias + 1024;
+  float* sm_bias = reinterpret_cast<float*>(staging + C::kStagingBytes + 256);      // [1024] bias
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   static_assert(CS == 1 || (CG == 2 && PASSES == 2), "pair clusters are implemented for the CTA-pair F8C kernel");
-  static_assert(PASSES != 4 || EPI != EPI_F32_LN, "the fused LayerNorm epilogue keeps x in TMEM: no room for scale factors");
-  static_assert(PASSES == 4 || (EPI != EPI_F32_EMIT && EPI != EPI_GELU_DLN), "deferred LayerNorm: FMT_F4C kernel only");
-  constexpr bool kF32 = EPI == EPI_F32 || EPI == EPI_F32_LN || EPI == EPI_F32_EMIT;          // fp32 output (+ residual)
+  constexpr bool kF32 = EPI == EPI_F32;                                                      // fp32 output (+ residual)
   static_assert(EPI != EPI_F32_RED || PASSES == 4, "the reduction epilogue is built for the FMT_F4C kernel");
-  constexpr bool kGelu4 = (EPI == EPI_GELU_SPLIT || EPI == EPI_GELU_DLN) && PASSES == 4;      // GELU -> FMT_F4C operand
+  constexpr bool kGelu4 = EPI == EPI_GELU_SPLIT && PASSES == 4;                              // GELU -> FMT_F4C operand
   const uint32_t crank = CG == 2 ? ptx::cluster_ctarank() : 0u;     // rank in the cluster (0 .. 2*CS-1)
   const uint32_t rank = crank & 1u;                                 // position in the CTA pair, 0 = leader
   const uint32_t pair = crank >> 1;                                 // pair index inside the cluster (0 .. CS-1)
@@ -382,11 +334,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constan
     if (CG == 2) ptx::tmem_alloc_cg2<C::kTmemCols>(&bars->tmem_base);
     else ptx::tmem_alloc<C::kTmemCols>(&bars->tmem_base);
   }
-  if (kGelu4 || EPI == EPI_F32_EMIT) {           // N <= 1024 (checked by the launcher)
-    for (int i = threadIdx.x; i < p.N; i += blockDim.x) {
-      sm_bias[i] = p.bias[i];
-      if (EPI == EPI_GELU_DLN) sm_colsum[i] = p.ln_colsum[i];
-    }
+  if (kGelu4) {                                  // N <= 1024 (checked by the launcher)
+    for (int i = threadIdx.x; i < p.N; i += blockDim.x) sm_bias[i] = p.bias[i];
   }
   ptx::tc_fence_before();
   if (CG == 2) ptx::cluster_sync(); else __syncthreads();
@@ -631,25 +580,13 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constan
     const int rsub = lane >> 3, gsub = lane & 7;      // coalesced mapping: instruction j covers rows 4j + rsub
     int acc = 0;
     uint32_t acc_phase = 0;
-    // EPI_F32_LN: running (mean, M2) of this lane's row over the 128 columns this warp owns in each accumulator
-    float ln_mean[2] = {0.f, 0.f}, ln_m2[2] = {0.f, 0.f};
-    constexpr bool kSmemVec = kGelu4 || EPI == EPI_F32_EMIT;     // bias / column sums come from shared memory
-    const F4cStore f4st = EPI == EPI_F32_EMIT ? f4c_store_init(p.emit_hi, p.emit_c4, p.N, gsub)
-                                              : f4c_store_init(p.out_hi, reinterpret_cast<uint8_t*>(p.out_lo), p.N, gsub);
+    const F4cStore f4st = f4c_store_init(p.out_hi, reinterpret_cast<uint8_t*>(p.out_lo), p.N, gsub);
     // PASSES == 4 (the shipped kernel): streaming stores are compiled in (D3D_GEMM_STREAM_OUT=0 at BUILD time for the A/B);
     // a run-time choice cost two predicated stores and four R2UR per store instruction (distinct memory descriptors)
 #ifndef D3D_GEMM_STREAM_OUT
 #define D3D_GEMM_STREAM_OUT 1
 #endif
     const bool stream_out = PASSES == 4 ? (D3D_GEMM_STREAM_OUT != 0) : (p.stream_out != 0);
-    // EPI_GELU_DLN: (rstd, -rstd mean) of this lane's row, valid for all n-tiles of the current m-tile; the partial sums
-    // of the NEXT m-tile's row are fetched a few per tile while this m-tile is processed (their latency would otherwise
-    // sit on the epilogue's critical path, which sets the tile time of fc1)
-    ptx::f32x2 dln_a = ptx::splat2(1.0f), dln_b = ptx::splat2(0.0f);
-    int dln_mt = -1;                         // m-tile the pair (dln_a, dln_b) belongs to
-    float dln_s1 = 0.f, dln_s2 = 0.f;        // sums gathered so far for m-tile dln_next_mt
-    int dln_next_mt = -1, dln_parts_done = 0;
-    auto dln_row_of = [&](int mt) { return ((mt * CS + static_cast<int>(pair)) * TM + static_cast<int>(rank) * BM) + q * 32 + lane; };
     for (int q_ = 0, tile; (tile = tile_of(q_)) >= 0; ++q_) {
       const int m0 = ((tile / n_tiles_n) * CS + static_cast<int>(pair)) * TM + static_cast<int>(rank) * BM;
       const int n0 = (tile % n_tiles_n) * BN;
@@ -660,10 +597,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constan
       // (read + write) and, with the F4C mainloop at ~5 us per tile, sets the tile time of proj / fc2: ncu had them at
       // 55-58 % of DRAM with ONE 4 KB chunk per warp in flight (32 KB per SM, below bandwidth x latency ~ 44 B/ns x 0.8 us);
       // two chunks per warp double the bytes in flight (profiles/r02d_full_gemm.md -> r02e).
-      constexpr int kResDepth = (EPI == EPI_F32 && EW == 8) ? D3D_GEMM_RES_DEPTH : 1;      // EMIT / 16 warps: no registers to spare
-      // 16 warps at 104 registers: x (32 registers) stays live through the operand emission, so the next residual chunk is
-      // requested only after it (four warps per scheduler cover the exposed latency)
-      constexpr bool kLateRes = EPI == EPI_F32_EMIT && EW == 16;
+      constexpr int kResDepth = (EPI == EPI_F32 && EW == 8) ? D3D_GEMM_RES_DEPTH : 1;      // 16 warps: no registers to spare
       float4 resv[kResDepth][8];
       auto load_res = [&](int ci) {                     // residual chunk ci, coalesced (row 4j + rsub, granule gsub)
 #pragma unroll
@@ -679,42 +613,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constan
         for (int c = 0; c < kResDepth; ++c) load_res(c);
       }
       uint32_t sfp_w = 0, sfq_w = 0;         // F4C output operand: this row's scale bytes of the tile's k-blocks (P / Q part)
-      ptx::f32x2 ln_s1p = ptx::splat2(0.f), ln_s2p = ptx::splat2(0.f);   // EPI_F32_EMIT: (sum, sum of squares) of this lane's row, 64 columns
-      float2 dln_pf[2] = {make_float2(0.f, 0.f), make_float2(0.f, 0.f)};   // partial sums in flight during this tile
-      int dln_pf_n = 0;
-      if (EPI == EPI_GELU_DLN) {
-        const int parts = p.K >> 6;
-        const int mt = tile / n_tiles_n;
-        if (mt != dln_mt) {
-          // statistics of this m-tile: whatever was not prefetched is loaded now (all of it for the first m-tile)
-          const int rr = dln_row_of(mt);
-          if (dln_next_mt != mt) { dln_s1 = 0.f; dln_s2 = 0.f; dln_parts_done = 0; }
-          if (rr < p.M)           // same order of additions as the prefetched path: results must not depend on which
-            for (int pt = dln_parts_done; pt < parts; pt += 2) {      // tiles of a CTA a row falls into (batch-split invariance)
-              const float2 v0 = p.ln_stats[static_cast<size_t>(pt) * p.M + rr];
-              const float2 v1 = p.ln_stats[static_cast<size_t>(pt + 1) * p.M + rr];
-              dln_s1 += v0.x + v1.x; dln_s2 += v0.y + v1.y;
-            }
-          const float inv_k = 1.0f / static_cast<float>(p.K);
-          const float mean = dln_s1 * inv_k;
-          const float var = fmaxf(fmaf(-mean, mean, dln_s2 * inv_k), 0.0f);
-          const float rstd = 1.0f / sqrtf(var + p.ln_eps);
-          dln_a = ptx::splat2(rstd);
-          dln_b = ptx::splat2(-rstd * mean);
-          dln_mt = mt;
-          dln_s1 = 0.f; dln_s2 = 0.f; dln_parts_done = 0;
-          const int nt = tile_of(q_ + n_tiles_n - tile % n_tiles_n);       // first tile of this unit's next m-tile
-          dln_next_mt = nt >= 0 ? nt / n_tiles_n : -1;
-        }
-        if (dln_next_mt >= 0 && dln_parts_done < parts) {                   // two more parts of the next m-tile's row
-          const int rr = dln_row_of(dln_next_mt);
-          dln_pf_n = 2;                                                     // K % 128 == 0: an even number of parts
-          if (rr < p.M) {
-            dln_pf[0] = p.ln_stats[static_cast<size_t>(dln_parts_done) * p.M + rr];
-            dln_pf[1] = p.ln_stats[static_cast<size_t>(dln_parts_done + 1) * p.M + rr];
-          }
-        }
-      }
       ptx::mbar_wait(&bars->tmem_full[acc], acc_phase);
       ptx::tc_fence_after();
 #pragma unroll
@@ -726,15 +624,15 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constan
 #pragma unroll
           for (int j = 0; j < 8; ++j) stg_st(stg, 4 * j + rsub, gsub, *reinterpret_cast<uint4*>(&resv[ci % kResDepth][j]));
           __syncwarp();
-          if (!kLateRes && ci + kResDepth < kChunks) load_res(ci + kResDepth);
+          if (ci + kResDepth < kChunks) load_res(ci + kResDepth);
         }
         const int gcol = n0 + col0;
         float4 bias4[8];                                 // issued before the TMEM wait so their latency is hidden
-        if (!kSmemVec) {
+        if (!kGelu4) {
 #pragma unroll
           for (int v = 0; v < 8; ++v) bias4[v] = __ldg(reinterpret_cast<const float4*>(p.bias + gcol) + v);
         }
-        const uint32_t sb4 = ptx::smem_u32(sm_bias + gcol), sc4 = ptx::smem_u32(sm_colsum + gcol);   // kSmemVec: read just in time
+        const uint32_t sb4 = ptx::smem_u32(sm_bias + gcol);   // kGelu4: read just in time
         ptx::tmem_ld_wait();
         if (PASSES == 4 && ci == 0 && half == 0) {
           // columns 0..31 of this accumulator are in registers: the NEXT tile's e2m1 stages may put their scale factors there
@@ -760,56 +658,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constan
             ptx::tma_reduce_add_2d(&tm_out, stg, gcol, row_w);
             ptx::bulk_commit();
           }
-        } else if (EPI == EPI_F32_EMIT) {
-          // x = acc + bias + residual on packed pairs; x stays in r for the operand image; (sum, sum of squares) per lane
-#pragma unroll
-          for (int v = 0; v < 8; ++v) {
-            const float4 b = lds_f4(sb4 + 16 * v);
-            const uint4 ru = stg_ld(stg, lane, v);
-            const ptx::f32x2 o01 = ptx::add2(ptx::add2(ptx::pack2(__uint_as_float(r[4 * v + 0]), __uint_as_float(r[4 * v + 1])), ptx::pack2(b.x, b.y)),
-                                             ptx::pack2(__uint_as_float(ru.x), __uint_as_float(ru.y)));
-            const ptx::f32x2 o23 = ptx::add2(ptx::add2(ptx::pack2(__uint_as_float(r[4 * v + 2]), __uint_as_float(r[4 * v + 3])), ptx::pack2(b.z, b.w)),
-                                             ptx::pack2(__uint_as_float(ru.z), __uint_as_float(ru.w)));
-            float o0, o1, o2, o3;
-            ptx::unpack2(o01, o0, o1);
-            ptx::unpack2(o23, o2, o3);
-            r[4 * v + 0] = __float_as_uint(o0); r[4 * v + 1] = __float_as_uint(o1);
-            r[4 * v + 2] = __float_as_uint(o2); r[4 * v + 3] = __float_as_uint(o3);
-            stg_st(stg, lane, v, make_uint4(r[4 * v + 0], r[4 * v + 1], r[4 * v + 2], r[4 * v + 3]));
-            ln_s1p = ptx::add2(ln_s1p, ptx::add2(o01, o23));
-            ln_s2p = ptx::fma2(o01, o01, ptx::fma2(o23, o23, ln_s2p));
-          }
-          __syncwarp();
-          uint4 vals[8];
-#pragma unroll
-          for (int j = 0; j < 8; ++j) vals[j] = stg_ld(stg, 4 * j + rsub, gsub);
-          {
-            float* d = p.out_f32 + static_cast<size_t>(row_w + rsub) * p.N + gcol + gsub * 4;
-            const size_t step = static_cast<size_t>(4) * p.N;
-            if (p.M - row_w >= 32) {
-#pragma unroll
-              for (int j = 0; j < 8; ++j) { ptx::st_global_cs(d, vals[j]); d += step; }
-            } else {
-#pragma unroll
-              for (int j = 0; j < 8; ++j) { if (row_w + 4 * j + rsub < p.M) ptx::st_global_cs(d, vals[j]); d += step; }
-            }
-          }
-          __syncwarp();                        // every lane has read the fp32 rows out of the staging buffer
-          f4c_emit_chunk(r, stg, lane, row_w, gcol, p.M, f4st, stream_out, sfp_w, sfq_w);
-          if (kLateRes && ci + 1 < kChunks) load_res(ci + 1);
-          if (ci & 1) {                        // two chunks = 64 columns = one statistics part
-            const int rr = row_w + lane;
-            float a0, a1, q0, q1;
-            ptx::unpack2(ln_s1p, a0, a1);
-            ptx::unpack2(ln_s2p, q0, q1);
-            if (rr < p.M) p.ln_stats[static_cast<size_t>(gcol >> 6) * p.M + rr] = make_float2(a0 + a1, q0 + q1);
-            ln_s1p = ptx::splat2(0.f); ln_s2p = ptx::splat2(0.f);
-          }
         } else if (kF32) {
-          float csum = 0.f;
 #pragma unroll
           for (int v = 0; v < 8; ++v) {
-            const float4 b = kSmemVec ? lds_f4(sb4 + 16 * v) : bias4[v];
+            const float4 b = bias4[v];
             float4 o;
             o.x = __uint_as_float(r[4 * v + 0]) + b.x;
             o.y = __uint_as_float(r[4 * v + 1]) + b.y;
@@ -820,30 +672,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constan
               o.x += __uint_as_float(ru.x); o.y += __uint_as_float(ru.y); o.z += __uint_as_float(ru.z); o.w += __uint_as_float(ru.w);
             }
             stg_st(stg, lane, v, make_uint4(__float_as_uint(o.x), __float_as_uint(o.y), __float_as_uint(o.z), __float_as_uint(o.w)));
-            if (EPI == EPI_F32_LN) {           // keep x for the statistics and the TMEM write-back
-              r[4 * v + 0] = __float_as_uint(o.x); r[4 * v + 1] = __float_as_uint(o.y);
-              r[4 * v + 2] = __float_as_uint(o.z); r[4 * v + 3] = __float_as_uint(o.w);
-              csum += (o.x + o.y) + (o.z + o.w);
-            }
-          }
-          if (EPI == EPI_F32_LN) {
-            // x goes back into the accumulator columns (pass 2 normalises it without re-reading the residual), and the
-            // chunk's (mean, M2) joins the lane's running pair (Chan et al.: no E[x^2] - mean^2 cancellation)
-            ptx::tmem_st_32x32(tmem_base + acc * BN + col0 + (static_cast<uint32_t>(q * 32) << 16), r);
-            const float cmean = csum * (1.0f / 32.0f);
-            float cm2 = 0.f;
-#pragma unroll
-            for (int e = 0; e < 32; ++e) {
-              const float d = __uint_as_float(r[e]) - cmean;
-              cm2 = fmaf(d, d, cm2);
-            }
-            const float cnt = 32.0f * ci, tot = cnt + 32.0f;
-            const float delta = cmean - ln_mean[acc];
-            if (ci == 0) { ln_mean[acc] = cmean; ln_m2[acc] = cm2; }
-            else {
-              ln_mean[acc] += delta * (32.0f / tot);
-              ln_m2[acc] += cm2 + delta * delta * (cnt * 32.0f / tot);
-            }
           }
           __syncwarp();
           uint4 vals[8];                       // all shared loads first, then all global stores (distinct registers)
@@ -869,16 +697,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constan
             for (int e = 0; e < 4; ++e) {
               const float4 b = lds_f4(sb4 + 16 * (2 * v + (e >> 1)));
               const ptx::f32x2 accp = ptx::pack2(__uint_as_float(r[8 * v + 2 * e + 0]), __uint_as_float(r[8 * v + 2 * e + 1]));
-              ptx::f32x2 bp2 = (e & 1) ? ptx::pack2(b.z, b.w) : ptx::pack2(b.x, b.y);
-              ptx::f32x2 xp;
-              if (EPI == EPI_GELU_DLN) {        // rstd acc + (c_n - rstd mean s_n)
-                const float4 cs = lds_f4(sc4 + 16 * (2 * v + (e >> 1)));
-                bp2 = ptx::fma2(dln_b, (e & 1) ? ptx::pack2(cs.z, cs.w) : ptx::pack2(cs.x, cs.y), bp2);
-                xp = ptx::fma2(dln_a, accp, bp2);
-              } else {
-                xp = ptx::add2(accp, bp2);
-              }
-              xp = gelu_erf2(xp);
+              const ptx::f32x2 bp2 = (e & 1) ? ptx::pack2(b.z, b.w) : ptx::pack2(b.x, b.y);
+              const ptx::f32x2 xp = gelu_erf2(ptx::add2(accp, bp2));
               float x0, x1;
               ptx::unpack2(xp, x0, x1);
               const __half2 h01 = __floats2half2_rn(x0, x1);
@@ -1018,15 +838,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constan
         }
         __syncwarp();          // the buffer is rewritten by the next chunk
       }
-      if (kGelu4 || EPI == EPI_F32_EMIT) {
+      if (kGelu4) {
         // scale bytes of row (row_w + lane): k-blocks colbase/32 .. +kChunks-1 of part P, the same + N/32 of part Q; they
         // are adjacent bytes of one scale-factor atom (operand.cuh), written as one word (4 chunks) or half-word (2)
         const int rr = row_w + lane;
         if (rr < p.M) {
           const int kb0 = colbase >> 5, apt = p.N / 64;
-          uint8_t* sf_out = EPI == EPI_F32_EMIT ? p.emit_sf : p.out_sf;
-          uint8_t* dp = sf_out + op_sf_offset(rr, kb0, apt);
-          uint8_t* dq = sf_out + op_sf_offset(rr, (p.N >> 5) + kb0, apt);
+          uint8_t* dp = p.out_sf + op_sf_offset(rr, kb0, apt);
+          uint8_t* dq = p.out_sf + op_sf_offset(rr, (p.N >> 5) + kb0, apt);
           if (kChunks == 4) {
             *reinterpret_cast<uint32_t*>(dp) = sfp_w;
             *reinterpret_cast<uint32_t*>(dq) = sfq_w;
@@ -1036,97 +855,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constan
           }
         }
       }
-      if (EPI == EPI_F32_LN) {
-        // The two n-tiles of a row tile land in accumulators 0 and 1 back to back (n-inner order, N == 2 BN).  After
-        // pass 1 of the second one the full 512-wide rows are known: exchange the partial statistics with the warp that
-        // owns the other 128 columns of these rows, then pass 2 re-reads x from TMEM, normalises and writes the next
-        // GEMM's A operand.  Accumulator 0 is released only here (x lives in it between the passes).
-        if (acc == 1) {
-          ptx::tmem_st_wait();
-          *reinterpret_cast<float4*>(staging + (warp - 4) * 4096 + lane * 16) = make_float4(ln_mean[0], ln_m2[0], ln_mean[1], ln_m2[1]);
-          ptx::bar_sync(1, EW * 32);
-          const float4 oth = *reinterpret_cast<const float4*>(staging + ((warp - 4) ^ 4) * 4096 + lane * 16);
-          ptx::bar_sync(1, EW * 32);                       // every partner row is read: the buffers may be reused
-          // Chan combination of equal-sized groups: mean = (a + b) / 2, M2 = M2a + M2b + (b - a)^2 n / 2
-          const float d0 = oth.x - ln_mean[0], d1 = oth.z - ln_mean[1];
-          const float mean0 = ln_mean[0] + 0.5f * d0, m20 = ln_m2[0] + oth.y + d0 * d0 * 64.0f;     // 256 columns each
-          const float mean1 = ln_mean[1] + 0.5f * d1, m21 = ln_m2[1] + oth.w + d1 * d1 * 64.0f;
-          const float dd = mean1 - mean0;
-          const float mean = mean0 + 0.5f * dd;
-          const float var = (m20 + m21 + dd * dd * 128.0f) * (1.0f / 512.0f);
-          const float rstd = 1.0f / sqrtf(var + p.ln_eps);      // as ln_rows() of rowwise.cu
-          uint8_t* c8 = reinterpret_cast<uint8_t*>(p.ln_second);
-#pragma unroll
-          for (int a = 0; a < 2; ++a) {
-#pragma unroll
-            for (int ci = 0; ci < kChunks; ++ci) {
-              const int col0 = half * kColsW + ci * 32;
-              const int gcol = a * BN + col0;
-              uint32_t r[32];
-              ptx::tmem_ld_32x32(tmem_base + a * BN + col0 + (static_cast<uint32_t>(q * 32) << 16), r);
-              ptx::tmem_ld_wait();
-              uint32_t a8w[8], l8w[8];
-#pragma unroll
-              for (int v = 0; v < 4; ++v) {
-                const float4 g0 = __ldg(reinterpret_cast<const float4*>(p.ln_gamma + gcol) + 2 * v);
-                const float4 g1 = __ldg(reinterpret_cast<const float4*>(p.ln_gamma + gcol) + 2 * v + 1);
-                const float4 b0 = __ldg(reinterpret_cast<const float4*>(p.ln_beta + gcol) + 2 * v);
-                const float4 b1 = __ldg(reinterpret_cast<const float4*>(p.ln_beta + gcol) + 2 * v + 1);
-                const float gg[8] = {g0.x, g0.y, g0.z, g0.w, g1.x, g1.y, g1.z, g1.w};
-                const float bb[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-                uint32_t hw[4], a16[4], l16[4];
-#pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                  const float x0 = fmaf((__uint_as_float(r[8 * v + 2 * e]) - mean) * rstd, gg[2 * e], bb[2 * e]);
-                  const float x1 = fmaf((__uint_as_float(r[8 * v + 2 * e + 1]) - mean) * rstd, gg[2 * e + 1], bb[2 * e + 1]);
-                  const __half h0 = __float2half_rn(x0), h1 = __float2half_rn(x1);
-                  hw[e] = pack_h2(h0, h1);
-                  a16[e] = op_e5m2x2(x0 * kActHiScale, x1 * kActHiScale);
-                  l16[e] = op_e5m2x2((x0 - __half2float(h0)) * kActLoScale, (x1 - __half2float(h1)) * kActLoScale);
-                }
-                stg_st(stg, lane, v, make_uint4(hw[0], hw[1], hw[2], hw[3]));
-                a8w[2 * v] = a16[0] | (a16[1] << 16); a8w[2 * v + 1] = a16[2] | (a16[3] << 16);
-                l8w[2 * v] = l16[0] | (l16[1] << 16); l8w[2 * v + 1] = l16[2] | (l16[3] << 16);
-              }
-              stg_st(stg, lane, 4, make_uint4(a8w[0], a8w[1], a8w[2], a8w[3]));
-              stg_st(stg, lane, 5, make_uint4(a8w[4], a8w[5], a8w[6], a8w[7]));
-              stg_st(stg, lane, 6, make_uint4(l8w[0], l8w[1], l8w[2], l8w[3]));
-              stg_st(stg, lane, 7, make_uint4(l8w[4], l8w[5], l8w[6], l8w[7]));
-              __syncwarp();
-              uint4 vals[8];
-#pragma unroll
-              for (int j = 0; j < 8; ++j) vals[j] = stg_ld(stg, 4 * j + rsub, gsub);
-#pragma unroll
-              for (int j = 0; j < 8; ++j) {
-                const int rr = row_w + 4 * j + rsub;
-                if (rr >= p.M) continue;
-                void* dst = gsub < 4 ? static_cast<void*>(p.ln_hi + static_cast<size_t>(rr) * p.N + gcol + gsub * 8)
-                                     : static_cast<void*>(c8 + static_cast<size_t>(rr) * (2 * p.N) + (gsub < 6 ? 0 : p.N) +
-                                                          gcol + (gsub & 1) * 16);
-                if (stream_out) ptx::st_global_cs(dst, vals[j]); else *reinterpret_cast<uint4*>(dst) = vals[j];
-              }
-              __syncwarp();
-            }
-            ptx::tc_fence_before();
-            __syncwarp();
-            if (lane == 0) {
-              if (CG == 2) ptx::mbar_arrive_cluster(ptx::mapa(ptx::smem_u32(&bars->tmem_empty[a]), leader));
-              else ptx::mbar_arrive(&bars->tmem_empty[a]);
-            }
-          }
-        }
-      } else {
-        ptx::tc_fence_before();
-        __syncwarp();
-        if (lane == 0) {
-          if (CG == 2) ptx::mbar_arrive_cluster(ptx::mapa(ptx::smem_u32(&bars->tmem_empty[acc]), leader));
-          else ptx::mbar_arrive(&bars->tmem_empty[acc]);
-        }
-      }
-      if (EPI == EPI_GELU_DLN && dln_pf_n > 0) {       // the prefetched partial sums have long arrived
-        dln_s1 += dln_pf[0].x + dln_pf[1].x;
-        dln_s2 += dln_pf[0].y + dln_pf[1].y;
-        dln_parts_done += dln_pf_n;
+      ptx::tc_fence_before();
+      __syncwarp();
+      if (lane == 0) {
+        if (CG == 2) ptx::mbar_arrive_cluster(ptx::mapa(ptx::smem_u32(&bars->tmem_empty[acc]), leader));
+        else ptx::mbar_arrive(&bars->tmem_empty[acc]);
       }
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
     }
@@ -1230,7 +963,6 @@ cudaError_t configure_gemm_tc() {
   if ((e = configure_one<2, 256, 2, EPI_QKV16, 2>()) != cudaSuccess) return e;
   if ((e = configure_one<2, 256, 2, EPI_GELU_SPLIT, 1, 16>()) != cudaSuccess) return e;
   if ((e = configure_one<2, 256, 2, EPI_QKV16, 1, 16>()) != cudaSuccess) return e;
-  if ((e = configure_one<2, 256, 2, EPI_F32_LN>()) != cudaSuccess) return e;
   if ((e = configure_one<2, 256, 2, EPI_F32, 1, 16>()) != cudaSuccess) return e;
   if ((e = configure_one<2, 256, 4, EPI_F32>()) != cudaSuccess) return e;
   if ((e = configure_one<2, 256, 4, EPI_GELU_SPLIT>()) != cudaSuccess) return e;
@@ -1239,10 +971,6 @@ cudaError_t configure_gemm_tc() {
   if ((e = configure_one<2, 256, 4, EPI_GELU_SPLIT, 1, 16>()) != cudaSuccess) return e;
   if ((e = configure_one<2, 256, 4, EPI_QKV16, 1, 16>()) != cudaSuccess) return e;
   if ((e = configure_one<2, 256, 4, EPI_F32_RED>()) != cudaSuccess) return e;
-  if ((e = configure_one<2, 256, 4, EPI_F32_EMIT>()) != cudaSuccess) return e;
-  if ((e = configure_one<2, 256, 4, EPI_F32_EMIT, 1, 16>()) != cudaSuccess) return e;
-  if ((e = configure_one<2, 256, 4, EPI_GELU_DLN>()) != cudaSuccess) return e;
-  if ((e = configure_one<2, 256, 4, EPI_GELU_DLN, 1, 16>()) != cudaSuccess) return e;
   return cudaSuccess;
 }
 
@@ -1251,37 +979,22 @@ cudaError_t launch_gemm_tc(const GemmMaps& maps, const GemmParams& p, int epi, i
   if (p.M <= 0) return cudaSuccess;
   if (passes == 4) {
     // FMT_F4C: CTA-pair 256 x 256 tiles only; K in whole e2m1 stages (256 nibbles = 128 bytes of the K-byte c4 row)
-    if (p.N % 256 != 0 || p.K % 128 != 0 || epi == EPI_F32_LN) return cudaErrorInvalidValue;
+    if (p.N % 256 != 0 || p.K % 128 != 0) return cudaErrorInvalidValue;
     if (epi == EPI_QKV16 && p.N != 3 * kC) return cudaErrorInvalidValue;
-    if ((epi == EPI_GELU_SPLIT || epi == EPI_GELU_DLN) && (!p.out_sf || p.N > 1024)) return cudaErrorInvalidValue;
-    // deferred LayerNorm: statistics parts of 64 columns, eight per 512-wide row
-    if (epi == EPI_F32_EMIT && (p.N != kC || !p.residual || !p.emit_hi || !p.emit_c4 || !p.emit_sf || !p.ln_stats))
-      return cudaErrorInvalidValue;
-    if (epi == EPI_GELU_DLN && (p.K != kC || !p.ln_stats || !p.ln_colsum)) return cudaErrorInvalidValue;
+    if (epi == EPI_GELU_SPLIT && (!p.out_sf || p.N > 1024)) return cudaErrorInvalidValue;
     if (epi == EPI_F32_RED && (!p.out_f32 || epi_warps == 16)) return cudaErrorInvalidValue;
     if (epi_warps == 16) {
       if (epi == EPI_F32) return launch_one<2, 256, 4, EPI_F32, 1, 16>(maps, p, num_sms, st);
       if (epi == EPI_GELU_SPLIT) return launch_one<2, 256, 4, EPI_GELU_SPLIT, 1, 16>(maps, p, num_sms, st);
-      if (epi == EPI_F32_EMIT) return launch_one<2, 256, 4, EPI_F32_EMIT, 1, 16>(maps, p, num_sms, st);
-      if (epi == EPI_GELU_DLN) return launch_one<2, 256, 4, EPI_GELU_DLN, 1, 16>(maps, p, num_sms, st);
       return launch_one<2, 256, 4, EPI_QKV16, 1, 16>(maps, p, num_sms, st);
     }
     if (epi == EPI_F32) return launch_one<2, 256, 4, EPI_F32>(maps, p, num_sms, st);
     if (epi == EPI_F32_RED) return launch_one<2, 256, 4, EPI_F32_RED>(maps, p, num_sms, st);
     if (epi == EPI_GELU_SPLIT) return launch_one<2, 256, 4, EPI_GELU_SPLIT>(maps, p, num_sms, st);
-    if (epi == EPI_F32_EMIT) return launch_one<2, 256, 4, EPI_F32_EMIT>(maps, p, num_sms, st);
-    if (epi == EPI_GELU_DLN) return launch_one<2, 256, 4, EPI_GELU_DLN>(maps, p, num_sms, st);
     return launch_one<2, 256, 4, EPI_QKV16>(maps, p, num_sms, st);
   }
-  if (epi == EPI_F32_EMIT || epi == EPI_GELU_DLN || epi == EPI_F32_RED) return cudaErrorInvalidValue;     // FMT_F4C kernel only
+  if (epi == EPI_F32_RED) return cudaErrorInvalidValue;     // FMT_F4C kernel only
   if (cta_group == 2 || passes == 2) bn = 256;
-  if (epi == EPI_F32_LN) {
-    // needs: both 256-column halves of a row tile on the same CTA pair, back to back, in accumulators 0 and 1
-    if (cta_group != 2 || passes != 2 || p.N != 2 * 256 || !p.n_inner || !p.residual || !p.ln_gamma || !p.ln_beta ||
-        !p.ln_hi || !p.ln_second)
-      return cudaErrorInvalidValue;
-    return launch_one<2, 256, 2, EPI_F32_LN>(maps, p, num_sms, st);
-  }
   if (epi_warps == 16 && cta_group == 2 && passes == 2 && pair_cluster != 2) {
     if (epi == EPI_F32) return launch_one<2, 256, 2, EPI_F32, 1, 16>(maps, p, num_sms, st);
     if (epi == EPI_GELU_SPLIT) return launch_one<2, 256, 2, EPI_GELU_SPLIT, 1, 16>(maps, p, num_sms, st);

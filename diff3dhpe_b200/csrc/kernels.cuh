@@ -17,26 +17,19 @@ constexpr int kHidden = 1024;  // mlp hidden
 // EPI_GELU_SPLIT out_hi/out_lo[M,N] = split_fp16(gelu_erf(acc + bias))            (fc1 -> A operand of fc2)
 // EPI_QKV16      N == 1536: out_qkv[M, 2048] fp16 rows = q(512) | k(512) | v_hi(512) | v_lo(512)
 //                (q, k rounded to fp16; v kept as a hi/lo pair so that the GRAND "- V" term stays exact)
-// EPI_F32_LN     EPI_F32 with a residual, N == 512, PLUS the following LayerNorm fused (proj + norm2, MODEL:127-128):
-//                out_f32 = x = acc + bias + residual;  ln_hi/ln_second[M,512] = operand(LN(x; ln_gamma, ln_beta, ln_eps)).
-//                CTA-pair F8C tcgen05 kernel only (both 256-column halves of a row tile finish back to back on the
-//                same CTA pair with the n-inner tile order, so the full rows sit in the two TMEM accumulators).
-// EPI_F32_EMIT   EPI_F32 with a residual, N == 512, FMT_F4C CTA-pair kernel: out_f32 = x = acc + bias + residual AND
-//                the SAME x leaves as a block-scaled GEMM operand (emit_hi / emit_c4 / emit_sf, K_out = N) together with
-//                per-row partial statistics ln_stats[part][M] = (sum, sum of squares) over columns 64 part .. 64 part + 63.
-//                This is proj + the DEFERRED norm2 (MODEL:127-128): the LayerNorm itself is applied by the consumer,
-// EPI_GELU_DLN   EPI_GELU_SPLIT whose A operand is that un-normalised x and whose weights were folded at load time
-//                (W' = gamma (.) W):  LN(x) . W^T + b = rstd_r (acc - mean_r s_n) + c_n  with  s_n = sum_k W'[n,k]
-//                (ln_colsum), c_n = b_n + sum_k W[n,k] beta_k (passed as `bias`), (mean_r, rstd_r) from ln_stats.
 // EPI_F32_RED    out_f32[M,N] += acc + bias: the in-place residual update of proj / fc2 (MODEL:127-128) as a TMA REDUCTION
 //                (cp.reduce.async.bulk.tensor .add.f32): the L2 adds the staged fp32 chunk to X, so the residual rows
 //                never travel L2 -> SM -- the link that bounds all four GEMMs.  Needs the `out` tensor map of GemmMaps
 //                ({32 floats x 32 rows} boxes over out_f32); same single fp32 rounding as (acc + bias) + x.
-enum GemmEpi { EPI_F32 = 0, EPI_GELU_SPLIT = 1, EPI_QKV16 = 2, EPI_F32_LN = 3, EPI_F32_EMIT = 4, EPI_GELU_DLN = 5,
-               EPI_F32_RED = 6 };
+// The values are part of the kernel symbols (gemm_tc_kernel<..., EPI, ...>) that the captures under profiles/ name, so
+// EPI_F32_RED keeps 6.
+enum GemmEpi { EPI_F32 = 0, EPI_GELU_SPLIT = 1, EPI_QKV16 = 2, EPI_F32_RED = 6 };
 
 constexpr int kQkvRow = 4 * kC;   // halves per token row of the packed q|k|v_hi|v_lo tensor
 
+// The GEMM kernels take it as a __grid_constant__ parameter: fields are read from parameter space where they are used.
+// Passed as a plain by-value struct of at most 128 bytes, it is loaded into registers at kernel entry instead (ptxas on
+// this struct: up to 22 more registers per thread, and spills in the fp32 epilogue kernels).
 struct GemmParams {
   int M, N, K;
   const float* bias;      // [N] (never null)
@@ -50,18 +43,8 @@ struct GemmParams {
   // activation (A) and weight (B) operand loads (0 normal, 1 evict_last, 2 evict_first) and streaming (evict-first)
   // output stores / residual loads
   int hint_a, hint_b, stream_out;
-  const float* ln_gamma;  // EPI_F32_LN
-  const float* ln_beta;
-  float ln_eps;
-  __half* ln_hi;          // A operand of the next GEMM (FMT_F8C: hi fp16 [M,512] + c8 bytes [M,1024])
-  __half* ln_second;
   int n_inner;            // tile order of the persistent tcgen05 kernel: 1 = all n-tiles of an m-tile on the same CTA pair
   int prefetch_a;         // FMT_F4C, n-inner: L2-prefetch the A rows of the unit's next m-tile while the current one runs
-  __half* emit_hi;        // EPI_F32_EMIT: x as a FMT_F4C operand [M,N] (hi fp16, c4 bytes, scale-factor atoms)
-  uint8_t* emit_c4;
-  uint8_t* emit_sf;
-  float2* ln_stats;       // EPI_F32_EMIT (written) / EPI_GELU_DLN (read): [8][M] (sum, sum of squares) per 64 columns
-  const float* ln_colsum; // EPI_GELU_DLN: s_n = sum_k W'[n,k]  [N]
 };
 
 // A: [M,K] fp16 (hi, lo), W: [N,K] fp16 (hi, lo); K-major.  Tensor maps use a {64, 128} box, SWIZZLE_128B.
@@ -110,11 +93,6 @@ cudaError_t launch_split(const float* in, __half* hi, __half* second, uint8_t* s
                          int is_weight, cudaStream_t st, float* absmax = nullptr);
 cudaError_t launch_merge(const __half* hi, const __half* second, const uint8_t* sf, float* out, int64_t rows, int K,
                          int fmt, cudaStream_t st);
-
-// Deferred LayerNorm (EPI_GELU_DLN): w_out = w (.) gamma (fp32, to be split), colsum[n] = sum_k w_out[n,k],
-// cbias[n] = bias[n] + sum_k w[n,k] beta[k]   (fold.cu; fp64 sums)
-cudaError_t launch_fold_ln_linear(const float* w, const float* gamma, const float* beta, const float* bias, float* w_out,
-                                  float* colsum, float* cbias, int N, int K, cudaStream_t st);
 
 // FMT_F4C scale factors of `rows` rows in atom layout -> row-major [rows][K / 16] bytes (test read-back)
 cudaError_t launch_sf_rows(const uint8_t* sf, uint8_t* out, int64_t rows, int K, cudaStream_t st);

@@ -309,26 +309,6 @@ class Engine:
                                           act, gemm_mode, self._stream()), self.h, "d3d_op_linear")
         return out
 
-    def op_linear_ln(self, a, w, bias, residual, gamma, beta, eps):
-        """Fused GEMM + residual + LayerNorm kernel: returns (x = a w^T + bias + residual, LayerNorm(x))."""
-        M, K = a.shape
-        x = torch.empty((M, self.C), device=self.device, dtype=torch.float32)
-        ln = torch.empty_like(x)
-        _lib.check(self.lib.d3d_op_linear_ln(self.h, _ptr(a), _ptr(w), _ptr(bias), _ptr(residual), _ptr(gamma),
-                                             _ptr(beta), float(eps), _ptr(x), _ptr(ln), M, K, self._stream()), self.h,
-                   "d3d_op_linear_ln")
-        return x, ln
-
-    def op_linear_dln_linear(self, a, w, bias, residual, gamma, beta, eps, w2, b2):
-        """Deferred-norm2 pair of the F4C path: returns (x = a w^T + bias + residual, gelu(LayerNorm(x) w2^T + b2))."""
-        M, K = a.shape
-        x = torch.empty((M, self.C), device=self.device, dtype=torch.float32)
-        hid = torch.empty((M, w2.shape[0]), device=self.device, dtype=torch.float32)
-        _lib.check(self.lib.d3d_op_linear_dln_linear(self.h, _ptr(a), _ptr(w), _ptr(bias), _ptr(residual), _ptr(gamma),
-                                                     _ptr(beta), float(eps), _ptr(w2), _ptr(b2), _ptr(x), _ptr(hid), M, K,
-                                                     self._stream()), self.h, "d3d_op_linear_dln_linear")
-        return x, hid
-
     def op_linear_bench(self, M, N, K, act=0, gemm_mode=_lib.GEMM_TC_SPLIT3, iters=10) -> float:
         ms = C.c_float()
         _lib.check(self.lib.d3d_op_linear_bench(self.h, M, N, K, act, gemm_mode, iters, C.byref(ms)), self.h,

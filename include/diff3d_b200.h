@@ -224,9 +224,7 @@ D3D_API int d3d_op_linear(d3d_handle* h, const float* a_dev, const float* w_dev,
                   const float* residual_dev, float* out_dev, int64_t M, int32_t N, int32_t K, int32_t act,
                   int32_t gemm_mode, void* stream);
 /* Times `iters` back-to-back launches of the GEMM kernel alone (operands pre-split), returns ms/launch.
- * act: 0 fp32 output, 1 GELU -> operand, 2 fp32 output + in-place residual (proj / fc2 as they run in the step),
- * 3 = 2 + the emitted operand and row statistics of the deferred norm2 (N == 512), 4 = GELU with the deferred
- * LayerNorm applied in the epilogue (K == 512); 3 and 4 need D3D_GEMM_TC_F4C. */
+ * act: 0 fp32 output, 1 GELU -> operand, 2 fp32 output + in-place residual (proj / fc2 as they run in the step). */
 D3D_API int d3d_op_linear_bench(d3d_handle* h, int64_t M, int32_t N, int32_t K, int32_t act, int32_t gemm_mode,
                         int32_t iters, float* ms_per_launch);
 
@@ -249,23 +247,6 @@ D3D_API int d3d_op_time_table(d3d_handle* h, const float* t_host, int32_t R, flo
  * residual stream [B*F*J, C] as it stands BEFORE the next post-norm into x_out_dev. */
 D3D_API int d3d_debug_forward_blocks(d3d_handle* h, const float* x5_dev, const int64_t* t_dev, int32_t B,
                              int32_t n_blocks, float* x_out_dev, void* stream);
-
-/* The fused "proj + residual + norm2" kernel (MODEL:127-128) on explicit operands: x_out = a . w^T + bias + residual
- * ([M,512], K = columns of a), ln_out = LayerNorm(x_out; gamma, beta, eps) read back from the operand format it is
- * written in (fp16 hi + e5m2 lo).  Needs gemm_mode D3D_GEMM_TC_F8C. */
-D3D_API int d3d_op_linear_ln(d3d_handle* h, const float* a_dev, const float* w_dev, const float* bias_dev,
-                     const float* residual_dev, const float* gamma_dev, const float* beta_dev, float eps,
-                     float* x_out_dev, float* ln_out_dev, int64_t M, int32_t K, void* stream);
-
-/* The deferred-norm2 pair of the F4C tcgen05 path (MODEL:127-128, 51-52) on explicit operands:
- *   x_out [M,512]    = a . w^T + bias + residual                       (proj: EPI_F32_EMIT, also emits x as an operand)
- *   hid_out [M,1024] = gelu(LayerNorm(x_out; gamma, beta, eps) . w2^T + b2)   (fc1: EPI_GELU_DLN on that operand, with
- *                      w2 folded with gamma at "load time" and the row statistics applied in the epilogue),
- * hid_out read back from the block-scaled operand format it is written in.  K = columns of a, K % 128 == 0. */
-D3D_API int d3d_op_linear_dln_linear(d3d_handle* h, const float* a_dev, const float* w_dev, const float* bias_dev,
-                             const float* residual_dev, const float* gamma_dev, const float* beta_dev, float eps,
-                             const float* w2_dev, const float* b2_dev, float* x_out_dev, float* hid_out_dev, int64_t M,
-                             int32_t K, void* stream);
 
 /* Runs one attention core like d3d_op_attention but returns the result in the raw GEMM A-operand format the proj
  * GEMM consumes: hi_out_dev [T, C] fp16 and second_out_dev [T, 2*C] bytes (operand format of the handle's gemm_mode:

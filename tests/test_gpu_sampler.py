@@ -77,15 +77,14 @@ def test_sampler_golden(golden, name, use_graph, gemm_mode):
     assert _mpjpe_delta(pred, ref, gt) < MPJPE_BAR / margin
 
 
-@pytest.mark.parametrize("env", [{"D3D_DEFER_LN2": "1"}, {"D3D_GEMM_RED": "0"}, {"D3D_DEFER_LN2": "1", "D3D_GEMM_RED": "0"},
-                                 {"D3D_LN_ROWS": "1"}, {"D3D_ATTN_WG2": "1"}, {"D3D_ATTN_SLOTS": "3"}, {"D3D_ATTN_SLOTS": "2"}])
+@pytest.mark.parametrize("env", [{"D3D_GEMM_RED": "0"}, {"D3D_LN_ROWS": "1"}, {"D3D_ATTN_WG2": "1"}, {"D3D_ATTN_SLOTS": "3"},
+                                 {"D3D_ATTN_SLOTS": "2"}])
 @pytest.mark.parametrize("name", ["sampler_f27_b2_s3_clip", "sampler_f243_b1_s9_clip", "sampler_f27_b2_s9_notime"])
 def test_sampler_golden_alternative_epilogues(golden, monkeypatch, name, env):
-    """The two measured-and-kept alternatives of the F4C path, through the whole sampler against the reference goldens:
-    D3D_DEFER_LN2=1 (proj emits x as fc1's operand + row sums, fc1 applies norm2 in its epilogue; read at d3d_create, the
-    weights are folded at load time) and D3D_GEMM_RED=0 (residual update by load-add-store instead of the TMA reduction;
-    read when the launch sequence is built).  RED on / off must not change a single bit, and neither must the one-row-per-
-    warp LayerNorm kernels (D3D_LN_ROWS=1; shipped: two rows per warp sharing every parameter load).  D3D_ATTN_WG2=1 is the
+    """Measured-and-kept alternatives of the F4C path, through the whole sampler against the reference goldens:
+    D3D_GEMM_RED=0 (residual update by load-add-store instead of the TMA reduction; read when the launch sequence is
+    built).  RED on / off must not change a single bit, and neither must the one-row-per-warp LayerNorm kernels
+    (D3D_LN_ROWS=1; shipped: two rows per warp sharing every parameter load).  D3D_ATTN_WG2=1 is the
     two-warpgroups-per-slot temporal attention kernel (same arithmetic per element, different summation split of the row;
     measured slower, ships off)."""
     for k, v in env.items():
@@ -99,7 +98,7 @@ def test_sampler_golden_alternative_epilogues(golden, monkeypatch, name, env):
     ref = torch.from_numpy(g["pred"])
     assert (pred - ref).abs().max().item() < MAXABS_BAR / MARGIN_F4C
     assert _mpjpe_delta(pred, ref, gt) < MPJPE_BAR / MARGIN_F4C
-    if "D3D_DEFER_LN2" not in env and "D3D_ATTN_WG2" not in env and "D3D_ATTN_SLOTS" not in env:
+    if "D3D_ATTN_WG2" not in env and "D3D_ATTN_SLOTS" not in env:
         for k in env:
             monkeypatch.delenv(k)
         diff2 = _diffusion(F, S, 0.0, bool(g["clip"]), bool(g["with_time_emb"]), gemm_mode=_lib.GEMM_TC_F4C, max_clips=B)
