@@ -6,14 +6,15 @@
 // One CTA per (sequence, head).  Token of position n in sequence s:  (s / inner) * outer + (s % inner) + n * tok_stride
 //   spatial : inner = 1, outer = J, tok_stride = 1, N = J      (s = b*F + f)
 //   temporal: inner = J, outer = F*J, tok_stride = J, N = F    (s = b*J + j)   -- no transposes (MODEL:119-121,130-133)
-// Also: pack_qkv16_kernel, fp32 [T,1536] -> the packed fp16 layout (op-level test entry point only; in the
-// sampler the qkv GEMM epilogue writes the packed layout directly).
+// Also: pack_qkv16_kernel, fp32 [T, 3 C] -> the packed fp16 layout (op-level test entry point only; in the
+// sampler the qkv GEMM epilogue writes the packed layout directly).  The validation kernel is built for C = 512 only.
 #include "kernels.cuh"
 #include "operand.cuh"
 
 namespace d3d {
 namespace {
 
+constexpr int kC = Width<512>::kC, kHd = Width<512>::kHd, kQkvRow = Width<512>::kQkvRow;
 constexpr float kScale = 0.125f;   // head_dim ** -0.5, MODEL:65
 constexpr int KPAD = kHd + 1;
 
@@ -110,16 +111,18 @@ attn_generic_kernel(const __half* __restrict__ qkv, __half* __restrict__ o_hi, _
   }
 }
 
+template <int C>
 __global__ void pack_qkv16_kernel(const float* __restrict__ in, __half* __restrict__ out, int64_t T) {
-  const int64_t n = T * (3 * kC);
+  constexpr int kRow = Width<C>::kQkvRow;
+  const int64_t n = T * (3 * C);
   for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
        i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-    const int64_t t = i / (3 * kC);
-    const int c = static_cast<int>(i - t * (3 * kC));
+    const int64_t t = i / (3 * C);
+    const int c = static_cast<int>(i - t * (3 * C));
     const float v = in[i];
     const __half h = __float2half_rn(v);
-    out[t * kQkvRow + c] = h;
-    if (c >= 2 * kC) out[t * kQkvRow + c + kC] = __float2half_rn(v - __half2float(h));
+    out[t * kRow + c] = h;
+    if (c >= 2 * C) out[t * kRow + c + C] = __float2half_rn(v - __half2float(h));
   }
 }
 
@@ -145,11 +148,13 @@ cudaError_t launch_attn_temporal_simt(const __half* qkv, __half* o_hi, __half* o
   return launch_attn_generic_simt(qkv, o_hi, o_lo, o_f32, fmt, B * J, F, static_cast<int64_t>(F) * J, J, J, st);
 }
 
-cudaError_t launch_pack_qkv16(const float* qkv_f32, __half* out, int64_t T, cudaStream_t st) {
+cudaError_t launch_pack_qkv16(int C, const float* qkv_f32, __half* out, int64_t T, cudaStream_t st) {
   if (T <= 0) return cudaSuccess;
-  int64_t g = (T * 3 * kC + 255) / 256;
+  if (!width_supported(C)) return cudaErrorInvalidValue;
+  int64_t g = (T * 3 * C + 255) / 256;
   if (g > 148 * 32) g = 148 * 32;
-  pack_qkv16_kernel<<<static_cast<unsigned>(g), 256, 0, st>>>(qkv_f32, out, T);
+  if (C == 256) pack_qkv16_kernel<256><<<static_cast<unsigned>(g), 256, 0, st>>>(qkv_f32, out, T);
+  else pack_qkv16_kernel<512><<<static_cast<unsigned>(g), 256, 0, st>>>(qkv_f32, out, T);
   return cudaGetLastError();
 }
 

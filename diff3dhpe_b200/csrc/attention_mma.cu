@@ -24,6 +24,9 @@
 namespace d3d {
 namespace {
 
+// mma.sync kernels (validation / bring-up modes): built for C = 512 only
+constexpr int kC = Width<512>::kC, kHd = Width<512>::kHd, kQkvRow = Width<512>::kQkvRow;
+
 constexpr int KS = 72;            // smem row stride in halves (144 B: ldmatrix rows hit distinct banks)
 constexpr float kScaleLog2e = 0.125f * 1.4426950408889634f;   // head_dim ** -0.5 (MODEL:65) in the exp2 domain
 

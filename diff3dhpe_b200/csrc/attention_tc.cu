@@ -26,6 +26,11 @@
 //
 // Warp roles (384 threads): 0..3 softmax + epilogue of slot 0 (TMEM lane quadrant = warp & 3), 4..7 of slot 1,
 // 8 = TMA producer, 9 = MMA issuer and TMEM allocator, 10..11 idle (they complete the control warpgroup).
+//
+// Width: the kernel is a template of the head dimension HD = C / 8.  HD = 64 (C = 512): Q / K / V rows are 128 B, SWIZZLE_128B
+// boxes, QK^T is 4 k-steps of 16, P.V has N = 64 and the proj operand row of a head is two scale blocks per part.  HD = 32
+// (C = 256, FMT_F4C only): 64-byte rows in SWIZZLE_64B boxes with matching UMMA descriptors, 2 k-steps, N = 32, one scale
+// block per part.  The softmax scale HD^-0.5 (32^-0.5 is not a power of two) stays applied to the fp32 scores.
 #include <cstdlib>
 #include "kernels.cuh"
 #include "operand.cuh"
@@ -46,10 +51,19 @@ constexpr int kTcThreads = 384;           // 3 warpgroups: softmax slot 0, softm
 constexpr int kCtrlRegs = 40, kSoftmaxRegs = 216;
 static_assert(2 * 128 * (kSoftmaxRegs - 168) <= 128 * (168 - kCtrlRegs), "setmaxnreg pool overdrawn");
 constexpr int kSpatialRows = 7 * 17;      // spatial mode: tokens (7 frames) per unit
-constexpr int kTile = 128 * 128;          // bytes of one {64 halves x 128 rows} box
+constexpr int kTile = 128 * 128;          // bytes of one {64 halves x 128 rows} box (HD = 64; the two-warpgroup kernel)
 constexpr int kSlotCols = 256;            // TMEM columns of one slot: S up to 256 fp32; P aliases [0,128), O [128,192)
 constexpr int kOCol = 128;
-constexpr float kScaleLog2e = 0.125f * 1.4426950408889634f;   // head_dim ** -0.5 (MODEL:65) in the exp2 domain
+// head_dim ** -0.5 (MODEL:65) in the exp2 domain
+template <int HD>
+constexpr float scale_log2e() {
+  static_assert(HD == 64 || HD == 32, "head_dim 64 (C = 512) or 32 (C = 256)");
+  return HD == 64 ? 0.125f * 1.4426950408889634f : 0.17677669529663687 * 1.4426950408889634;
+}
+constexpr float kScaleLog2e = scale_log2e<64>();
+// bytes of one {HD halves x 128 rows} box
+template <int HD>
+constexpr int tile_bytes() { return 128 * HD * 2; }
 
 // NSLOT = 128-query tiles in flight per CTA (each with its own 4 softmax warps and 256 TMEM columns).  Shipped: 2.  (A first version with one slot and two CTAs per SM measured 430 ms
 // per cfg3 step against 398 ms, profiles/r01m_bench_slots*.json.)
@@ -103,6 +117,29 @@ __device__ __forceinline__ uint64_t make_desc_mn_sw128(uint32_t smem_addr) {
   d |= static_cast<uint64_t>(2) << 61;
   return d;
 }
+// The same for HD = 32: 8 keys x 64 B per SWIZZLE_64B atom (layout type 4), next 8 keys SBO = 512 B further; N = 32 halves
+// is one atom wide.
+__device__ __forceinline__ uint64_t make_desc_mn_sw64(uint32_t smem_addr) {
+  uint64_t d = 0;
+  d |= static_cast<uint64_t>((smem_addr & 0x3ffffu) >> 4);
+  d |= static_cast<uint64_t>(1) << 16;
+  d |= static_cast<uint64_t>(512 >> 4) << 32;
+  d |= static_cast<uint64_t>(1) << 46;
+  d |= static_cast<uint64_t>(4) << 61;
+  return d;
+}
+template <int HD>
+__device__ __forceinline__ uint64_t make_desc_mn(uint32_t smem_addr) {
+  return HD == 64 ? make_desc_mn_sw128(smem_addr) : make_desc_mn_sw64(smem_addr);
+}
+// K-major Q / K operand of QK^T: {HD halves x 128 rows} box in the SWIZZLE_128B (HD = 64) or SWIZZLE_64B (HD = 32) layout
+template <int HD>
+__device__ __forceinline__ uint64_t make_desc_k(uint32_t smem_addr) {
+  return HD == 64 ? ptx::make_desc_k_sw128(smem_addr) : ptx::make_desc_k_sw64(smem_addr);
+}
+// byte offset of 16-byte granule g of row r inside a swizzled {HD halves x 128 rows} box: XOR with bits 7.. of r * 2 HD
+template <int HD>
+__device__ __forceinline__ int swz_xor(int r) { return HD == 64 ? (r & 7) << 4 : ((r >> 1) & 3) << 4; }
 
 
 __device__ __forceinline__ float row_sum(const ptx::f32x2 (&ls)[2]) {
@@ -118,8 +155,9 @@ __device__ __forceinline__ float row_sum(const ptx::f32x2 (&ls)[2]) {
 // TMEM reads are issued one batch (two 32-column chunks) ahead of the batch being processed.  NCH > 0: the number of
 // chunks is a compile-time constant and F > 32 (NCH - 1), so every offset is an immediate and only the last chunk is
 // masked; NCH == 0: runtime chunk count (<= 8).
-template <int NCH>
+template <int HD, int NCH>
 __device__ __forceinline__ float softmax_row(uint32_t taddr, int F, int n_chunks_rt) {
+  constexpr float kScaleLog2e = scale_log2e<HD>();
   constexpr int kMax = NCH > 0 ? NCH : 8;
   const int n = NCH > 0 ? NCH : n_chunks_rt;
   uint32_t a0[32], a1[32], b0[32], b1[32];
@@ -207,11 +245,12 @@ __device__ __forceinline__ float softmax_row(uint32_t taddr, int F, int n_chunks
 // (the masked form over all 96 loaded columns cost ~7 instructions per column, 665 per row; this one ~70 per frame, and
 // a warp runs at most three of them divergently).  Writes the packed fp16 P pairs of its window into pk (zero elsewhere)
 // and returns the row sum.
-template <int CS, int FR>
+template <int HD, int CS, int FR>
 __device__ __forceinline__ float spatial_window(const uint32_t (&a)[32], const uint32_t (&b)[32], const uint32_t (&c)[32],
                                                 uint32_t (&pk0)[16], uint32_t (&pk1)[16], uint32_t (&pk2)[16]) {
   constexpr int L = 17 * FR - 32 * CS;          // first window column among the 96 loaded ones
   static_assert(L >= 0 && L + 17 <= 96, "frame window outside the loaded chunks");
+  constexpr float kScaleLog2e = scale_log2e<HD>();
   float sv[18];
 #pragma unroll
   for (int k = 0; k < 17; ++k) {
@@ -246,6 +285,7 @@ __device__ __forceinline__ float spatial_window(const uint32_t (&a)[32], const u
   return s0 + s1;
 }
 
+template <int HD>
 __device__ __forceinline__ float softmax_row_spatial(uint32_t taddr, int row_l, int wq) {
   const int cs = wq >> 1;
   uint32_t a[32], b[32], c[32];
@@ -260,17 +300,17 @@ __device__ __forceinline__ float softmax_row_spatial(uint32_t taddr, int row_l, 
   float sum;
   if (cs == 0) {
     switch (fr) {
-      case 0: sum = spatial_window<0, 0>(a, b, c, pk0, pk1, pk2); break;
-      case 1: sum = spatial_window<0, 1>(a, b, c, pk0, pk1, pk2); break;
-      case 2: sum = spatial_window<0, 2>(a, b, c, pk0, pk1, pk2); break;
-      default: sum = spatial_window<0, 3>(a, b, c, pk0, pk1, pk2); break;
+      case 0: sum = spatial_window<HD, 0, 0>(a, b, c, pk0, pk1, pk2); break;
+      case 1: sum = spatial_window<HD, 0, 1>(a, b, c, pk0, pk1, pk2); break;
+      case 2: sum = spatial_window<HD, 0, 2>(a, b, c, pk0, pk1, pk2); break;
+      default: sum = spatial_window<HD, 0, 3>(a, b, c, pk0, pk1, pk2); break;
     }
   } else {
     switch (fr) {
-      case 3: sum = spatial_window<1, 3>(a, b, c, pk0, pk1, pk2); break;
-      case 4: sum = spatial_window<1, 4>(a, b, c, pk0, pk1, pk2); break;
-      case 5: sum = spatial_window<1, 5>(a, b, c, pk0, pk1, pk2); break;
-      default: sum = spatial_window<1, 6>(a, b, c, pk0, pk1, pk2); break;
+      case 3: sum = spatial_window<HD, 1, 3>(a, b, c, pk0, pk1, pk2); break;
+      case 4: sum = spatial_window<HD, 1, 4>(a, b, c, pk0, pk1, pk2); break;
+      case 5: sum = spatial_window<HD, 1, 5>(a, b, c, pk0, pk1, pk2); break;
+      default: sum = spatial_window<HD, 1, 6>(a, b, c, pk0, pk1, pk2); break;
     }
   }
   __syncwarp();                                   // tcgen05.st is .sync.aligned: the frames of the warp reconverge here
@@ -286,7 +326,9 @@ __device__ __forceinline__ float softmax_row_spatial(uint32_t taddr, int row_l, 
 // joints -- share one 128-row tile, row r = f G + jj (the {64 channels, G joints, 128 / G frames} TMA box lands exactly so).
 // Query row r attends the keys of its own joint only: columns c with c % G == r % G and c / G < F.  One pass over the
 // 128 columns for the max, one for exp2 / sum; P is zero elsewhere, so the P.V chain is the same as in the other modes.
+template <int HD>
 __device__ __forceinline__ float softmax_row_packed(uint32_t taddr, int F, int G, int row_l) {
+  constexpr float kScaleLog2e = scale_log2e<HD>();
   const int jj = row_l & (G - 1);
   const uint32_t vm = (G == 4 ? 0x11111111u : 0x55555555u) << jj;      // own-joint columns of any aligned 32-column chunk
   const int nk = F * G;                                                // columns >= nk are frames >= F (zero-filled rows)
@@ -335,13 +377,17 @@ __device__ __forceinline__ float softmax_row_packed(uint32_t taddr, int F, int G
 // views encoded with rank 4 (coordinates (channel, token, 0, 0)); n_mt == 1, NKp == 128; the store maps have 119-row
 // boxes, the *_tail maps (F % 7) * 17-row boxes.  J carries the groups per clip.
 // PACKED: G = `pk_g` joints per tile (softmax_row_packed); J then counts the joint GROUPS per clip and `j_tok` the joints.
-template <int FMT, int NSLOT, int NCH, bool SPATIAL, bool PACKED = false>
+template <int HD, int FMT, int NSLOT, int NCH, bool SPATIAL, bool PACKED = false>
 __global__ void __launch_bounds__((4 * NSLOT + 4) * 32, 1)
 attn_temporal_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_constant__ CUtensorMap tm_hi,
                         const __grid_constant__ CUtensorMap tm_second, const __grid_constant__ CUtensorMap tm_hi_tail,
                         const __grid_constant__ CUtensorMap tm_second_tail, uint8_t* __restrict__ sf_out, int F, int J,
                         int n_units, int n_mt, int NKp, int n_stage, int pk_g = 1, int j_tok = 0) {
   static_assert(!PACKED || (!SPATIAL && NCH == 0), "the packed mode is a temporal mode with a runtime chunk count");
+  static_assert(HD == 64 || (HD == 32 && FMT == FMT_F4C && NSLOT == 2), "head_dim 32 (C = 256): the shipped FMT_F4C kernel");
+  constexpr int kTile = tile_bytes<HD>();                      // one {HD halves x 128 rows} box
+  constexpr int kCw = kHeads * HD;                             // embed_dim
+  constexpr int kHd = HD;
   // NSLOT == 3 (single-tile modes, S only 128 columns wide, FMT_F4C): three 128-column slots, three softmax warpgroups
   // (512 threads, 128 registers at launch, control 40 / softmax 152), P aliases [0, 64), O [64, 128), 8 KB of staging per slot
   static_assert(NSLOT == 2 || (NSLOT == 3 && FMT == FMT_F4C && (SPATIAL || PACKED)), "three slots: single-tile F4C modes only");
@@ -354,7 +400,7 @@ attn_temporal_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const int stage_bytes = 3 * n_mt * kTile;          // Q tiles | K tiles | V tiles of one unit
-  uint8_t* StgAll = smem + n_stage * stage_bytes;    // 16 KB per slot: second-part staging of one 128-row output tile
+  uint8_t* StgAll = smem + n_stage * stage_bytes;    // kStgSlot per slot: second-part staging of one 128-row output tile
   TcBars<NSLOT>* bars = reinterpret_cast<TcBars<NSLOT>*>(StgAll + NSLOT * kStgSlot);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -405,9 +451,9 @@ attn_temporal_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
         ptx::mbar_wait(&bars->stage_free[stage], (k & 1) ^ 1);
         ptx::mbar_arrive_expect_tx(&bars->full[stage], 3 * n_mt * kTile);
         for (int t = 0; t < n_mt; ++t) {
-          ptx::tma_load_4d(Ks + t * kTile, &tm_qkv, &bars->full[stage], kC + h * kHd, j, t * 128, b);
+          ptx::tma_load_4d(Ks + t * kTile, &tm_qkv, &bars->full[stage], kCw + h * kHd, j, t * 128, b);
           ptx::tma_load_4d(Qs + t * kTile, &tm_qkv, &bars->full[stage], h * kHd, j, t * 128, b);
-          ptx::tma_load_4d(Vs + t * kTile, &tm_qkv, &bars->full[stage], 2 * kC + h * kHd, j, t * 128, b);
+          ptx::tma_load_4d(Vs + t * kTile, &tm_qkv, &bars->full[stage], 2 * kCw + h * kHd, j, t * 128, b);
         }
       }
     }
@@ -419,14 +465,14 @@ attn_temporal_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
       const uint32_t idesc_pv = ptx::make_idesc_f16(128, kHd, 0) | (1u << 16);      // B (= V) is MN-major
       const uint32_t s0 = ptx::smem_u32(smem);
       const int n_ks = NKp >> 4;
-      auto issue_pv = [&](int w) {           // O[128, 64] = P[128, NKp] (TMEM) . V[NKp, 64], 16 keys per MMA
+      auto issue_pv = [&](int w) {           // O[128, HD] = P[128, NKp] (TMEM) . V[NKp, HD], 16 keys per MMA
         const int slot = w % NSLOT, i = w / NSLOT, stage = (w / n_mt) % n_stage;
         const uint32_t sV = s0 + stage * stage_bytes + 2 * n_mt * kTile;
         const uint32_t tcol = tmem_base + slot * kSC;
         ptx::mbar_wait(&bars->p_full[slot], i & 1);
         ptx::tc_fence_after();
         for (int ks = 0; ks < n_ks; ++ks)
-          ptx::mma_f16_ts(tcol + kOC, tcol + ks * 8, make_desc_mn_sw128(sV + ks * 2048), idesc_pv, ks != 0 ? 1u : 0u);
+          ptx::mma_f16_ts(tcol + kOC, tcol + ks * 8, make_desc_mn<HD>(sV + ks * 32 * HD), idesc_pv, ks != 0 ? 1u : 0u);
         ptx::mma_commit(&bars->o_full[slot]);
       };
       for (int w = 0; w < W; ++w) {
@@ -440,9 +486,9 @@ attn_temporal_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
         ptx::mbar_wait(&bars->tmem_free[slot], (i & 1) ^ 1);
         ptx::tc_fence_after();
 #pragma unroll
-        for (int k = 0; k < 4; ++k)            // S[128, NKp] = Q_m[128, 64] . K[NKp, 64]^T, 16 channels per MMA
-          ptx::mma_f16_ss(tmem_base + slot * kSC, ptx::make_desc_k_sw128(sQ + m * kTile + k * 32),
-                          ptx::make_desc_k_sw128(sK + k * 32), idesc_qk, k != 0 ? 1u : 0u);
+        for (int k = 0; k < HD / 16; ++k)      // S[128, NKp] = Q_m[128, HD] . K[NKp, HD]^T, 16 channels per MMA
+          ptx::mma_f16_ss(tmem_base + slot * kSC, make_desc_k<HD>(sQ + m * kTile + k * 32),
+                          make_desc_k<HD>(sK + k * 32), idesc_qk, k != 0 ? 1u : 0u);
         ptx::mma_commit(&bars->s_full[slot]);
         // the P.V of the item NSLOT-1 back: with two slots, S of this item is already being computed while the other
         // slot's softmax finishes
@@ -474,11 +520,11 @@ attn_temporal_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
         const CUtensorMap* ms = tail ? &tm_second_tail : &tm_second;
         ptx::tma_store_4d(mh, Qs + m * kTile, h * kHd, j, m * 128, b);
         if (FMT == FMT_F4C) {
-          ptx::tma_store_4d(ms, Stg, h * 32, j, m * 128, b);
-          ptx::tma_store_4d(ms, Stg + 4096, (kC >> 1) + h * 32, j, m * 128, b);
+          ptx::tma_store_4d(ms, Stg, h * (HD / 2), j, m * 128, b);
+          ptx::tma_store_4d(ms, Stg + 64 * HD, (kCw >> 1) + h * (HD / 2), j, m * 128, b);
         } else {
           ptx::tma_store_4d(ms, Stg, h * kHd, j, m * 128, b);
-          if (FMT != FMT_SPLIT16) ptx::tma_store_4d(ms, Stg + 8192, kC + h * kHd, j, m * 128, b);
+          if (FMT != FMT_SPLIT16) ptx::tma_store_4d(ms, Stg + 8192, kCw + h * kHd, j, m * 128, b);
         }
         ptx::bulk_commit();
         ptx::bulk_wait_read_all();           // Stg / Q_m have been read: the tile has left shared memory
@@ -496,7 +542,7 @@ attn_temporal_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
     const int n_chunks = (NKp + 31) >> 5;
     if (!SPATIAL && NCH > 0 && (n_chunks != NCH || F <= 32 * (NCH - 1))) __trap();    // launcher / instantiation mismatch
     if ((SPATIAL || PACKED) && (n_mt != 1 || NKp != 128)) __trap();
-    const int sw = (row_l & 7) << 4;                                      // swizzle XOR of this row (bytes)
+    const int sw = swz_xor<HD>(row_l);                                   // swizzle XOR of this row (bytes)
     const bool issuer = row_l == 0;                                       // issues the slot's TMA stores
     uint8_t* Stg = StgAll + slot * kStgSlot;
     for (int w = slot; w < W; w += NSLOT) {
@@ -515,11 +561,11 @@ attn_temporal_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
       ptx::tc_fence_after();
       if (issuer) {      // Q_m is dead once S is complete: it receives the v_lo rows of the tile (exact "- V" term)
         ptx::mbar_arrive_expect_tx(&bars->vlo_full[slot], kTile);
-        ptx::tma_load_4d(Qs + m * kTile, &tm_qkv, &bars->vlo_full[slot], 3 * kC + h * kHd, j, m * 128, b);
+        ptx::tma_load_4d(Qs + m * kTile, &tm_qkv, &bars->vlo_full[slot], 3 * kCw + h * kHd, j, m * 128, b);
       }
-      const float inv = SPATIAL ? softmax_row_spatial(taddr, row_l, warp & 3)
-                      : PACKED  ? softmax_row_packed(taddr, F, pk_g, row_l)
-                                : softmax_row<NCH>(taddr, F, n_chunks);
+      const float inv = SPATIAL ? softmax_row_spatial<HD>(taddr, row_l, warp & 3)
+                      : PACKED  ? softmax_row_packed<HD>(taddr, F, pk_g, row_l)
+                                : softmax_row<HD, NCH>(taddr, F, n_chunks);
       ptx::tc_fence_before();
       ptx::mbar_arrive(&bars->p_full[slot]);
 
@@ -527,18 +573,18 @@ attn_temporal_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
       // landed in the dead Q tile long ago; ncu had 15 % of the softmax warps' samples idle on o_full and another 10 % on
       // the shared-memory loads below when they sat inside the epilogue loop, profiles/r01p_full_attn_tc.md)
       ptx::mbar_wait(&bars->vlo_full[slot], i & 1);
-      uint8_t* hi_row = Qs + m * kTile + row_l * 128;        // v_lo row in, hi row out (same thread, same 16 bytes)
-      const uint8_t* v_row = Vs + static_cast<size_t>(r) * 128;
-      ptx::f32x2 nv[32];
+      uint8_t* hi_row = Qs + m * kTile + row_l * (2 * HD);   // v_lo row in, hi row out (same thread, same 16 bytes)
+      const uint8_t* v_row = Vs + static_cast<size_t>(r) * (2 * HD);
+      ptx::f32x2 nv[HD / 2];
       {
-        uint4 vh[8], vl[8];
+        uint4 vh[HD / 8], vl[HD / 8];
 #pragma unroll
-        for (int g = 0; g < 8; ++g) {
+        for (int g = 0; g < HD / 8; ++g) {
           vh[g] = *reinterpret_cast<const uint4*>(v_row + ((g << 4) ^ sw));
           vl[g] = *reinterpret_cast<const uint4*>(hi_row + ((g << 4) ^ sw));
         }
 #pragma unroll
-        for (int g = 0; g < 8; ++g) {
+        for (int g = 0; g < HD / 8; ++g) {
           const uint32_t vhw[4] = {vh[g].x, vh[g].y, vh[g].z, vh[g].w};
           const uint32_t vlw[4] = {vl[g].x, vl[g].y, vl[g].z, vl[g].w};
 #pragma unroll
@@ -557,7 +603,7 @@ attn_temporal_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
       ptx::tc_fence_after();
       uint32_t o0[32], o1[32];
       ptx::tmem_ld_32x32(taddr + kOC, o0);
-      ptx::tmem_ld_32x32(taddr + kOC + 32, o1);
+      if (HD == 64) ptx::tmem_ld_32x32(taddr + kOC + 32, o1);
       ptx::tmem_ld_wait();
       ptx::tc_fence_before();
       ptx::mbar_arrive(&bars->tmem_free[slot]);
@@ -570,12 +616,12 @@ attn_temporal_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
       }
       const ptx::f32x2 inv2 = ptx::splat2(inv);
       if (FMT == FMT_F4C) {
-        // block-scaled operand (operand.cuh): the row's 64 channels are two 32-element scale blocks of each part.
+        // block-scaled operand (operand.cuh): the row's HD channels are HD / 32 scale blocks of 32 elements of each part.
         // Pass 1: x = O inv - (v_hi + v_lo) back into the O registers, hi halves into the (dead) Q row, block maxima of
         // x and of x - hi.  Pass 2: P = q4(x), Q = q4(x - hi) as [128 rows][32 B] tiles for the two TMA stores.
         float ax[2] = {0.f, 0.f}, al[2] = {0.f, 0.f};
 #pragma unroll
-        for (int g = 0; g < 8; ++g) {
+        for (int g = 0; g < HD / 8; ++g) {
           uint32_t hw[4];
 #pragma unroll
           for (int e = 0; e < 4; ++e) {
@@ -596,7 +642,7 @@ attn_temporal_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
         const uint32_t bp0 = op_ue8m0_of(ax[0]), bp1 = op_ue8m0_of(ax[1]), bq0 = op_ue8m0_of(al[0]), bq1 = op_ue8m0_of(al[1]);
         uint32_t pw[8], qw[8];
 #pragma unroll
-        for (int g = 0; g < 8; ++g) {
+        for (int g = 0; g < HD / 8; ++g) {
           const ptx::f32x2 ip = ptx::splat2(op_ue8m0_inv(g < 4 ? bp0 : bp1)), iq = ptx::splat2(op_ue8m0_inv(g < 4 ? bq0 : bq1));
           uint32_t pa = 0, qa = 0;
 #pragma unroll
@@ -612,27 +658,33 @@ attn_temporal_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
           }
           pw[g] = pa; qw[g] = qa;
         }
-        {                                                              // [128 rows][32 B] P tile, then the Q tile
-          uint4* stp = reinterpret_cast<uint4*>(Stg + row_l * 32);
+        {                                                              // [128 rows][HD / 2 B] P tile, then the Q tile
+          uint4* stp = reinterpret_cast<uint4*>(Stg + row_l * (HD / 2));
           stp[0] = make_uint4(pw[0], pw[1], pw[2], pw[3]);
-          stp[1] = make_uint4(pw[4], pw[5], pw[6], pw[7]);
-          stp[256] = make_uint4(qw[0], qw[1], qw[2], qw[3]);
-          stp[257] = make_uint4(qw[4], qw[5], qw[6], qw[7]);
+          if (HD == 64) stp[1] = make_uint4(pw[4], pw[5], pw[6], pw[7]);
+          stp[4 * HD] = make_uint4(qw[0], qw[1], qw[2], qw[3]);
+          if (HD == 64) stp[4 * HD + 1] = make_uint4(qw[4], qw[5], qw[6], qw[7]);
         }
-        // the row's four scale bytes: k-blocks (2h, 2h+1) of part P and (16 + 2h, 16 + 2h + 1) of part Q are adjacent
-        // bytes of a scale-factor atom.  Rows the TMA stores clip (>= F, or past the unit) must not be written here.
+        // the row's scale bytes: k-blocks (HD / 32) h .. of part P and C / 32 + (HD / 32) h .. of part Q are adjacent
+        // bytes of a scale-factor atom (HD = 64: two per part, HD = 32: one).  Rows the TMA stores clip (>= F, or past the
+        // unit) must not be written here.
         const int pf = PACKED ? row_l / pk_g : 0, pj = PACKED ? j + (row_l & (pk_g - 1)) : 0;   // packed: frame, joint of the row
         const int64_t tok = SPATIAL  ? static_cast<int64_t>(j) + row_l
                             : PACKED ? (static_cast<int64_t>(b) * F + pf) * j_tok + pj
                                      : (static_cast<int64_t>(b) * F + r) * J + j;
         const bool live = SPATIAL ? row_l < (tail ? (F % 7) * 17 : kSpatialRows) : PACKED ? (pf < F && pj < j_tok) : r < F;
         if (live) {
-          *reinterpret_cast<uint16_t*>(sf_out + op_sf_offset(tok, 2 * h, kC / 64)) = static_cast<uint16_t>(bp0 | (bp1 << 8));
-          *reinterpret_cast<uint16_t*>(sf_out + op_sf_offset(tok, 16 + 2 * h, kC / 64)) = static_cast<uint16_t>(bq0 | (bq1 << 8));
+          if (HD == 64) {
+            *reinterpret_cast<uint16_t*>(sf_out + op_sf_offset(tok, 2 * h, kCw / 64)) = static_cast<uint16_t>(bp0 | (bp1 << 8));
+            *reinterpret_cast<uint16_t*>(sf_out + op_sf_offset(tok, 16 + 2 * h, kCw / 64)) = static_cast<uint16_t>(bq0 | (bq1 << 8));
+          } else {
+            sf_out[op_sf_offset(tok, h, kCw / 64)] = static_cast<uint8_t>(bp0);
+            sf_out[op_sf_offset(tok, kCw / 32 + h, kCw / 64)] = static_cast<uint8_t>(bq0);
+          }
         }
       } else {
 #pragma unroll
-      for (int g = 0; g < 8; ++g) {
+      for (int g = 0; g < HD / 8; ++g) {
         // packed pairs: x = O inv - (v_hi + v_lo), lo = x - fp16(x) and the two e5m2 scalings as FFMA2 / FADD2 / FMUL2
         uint32_t hw[4], lw[4], a8[4], l8[4];
 #pragma unroll
@@ -674,12 +726,12 @@ attn_temporal_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
         const CUtensorMap* mh = tail ? &tm_hi_tail : &tm_hi;
         const CUtensorMap* ms = tail ? &tm_second_tail : &tm_second;
         ptx::tma_store_4d(mh, Qs + m * kTile, h * kHd, j, m * 128, b);
-        if (FMT == FMT_F4C) {                // c4 row: 256 B of P nibbles | 256 B of Q nibbles; 32 B per head and part
-          ptx::tma_store_4d(ms, Stg, h * 32, j, m * 128, b);
-          ptx::tma_store_4d(ms, Stg + 4096, (kC >> 1) + h * 32, j, m * 128, b);
+        if (FMT == FMT_F4C) {                // c4 row: C / 2 B of P nibbles | C / 2 B of Q nibbles; HD / 2 B per head and part
+          ptx::tma_store_4d(ms, Stg, h * (HD / 2), j, m * 128, b);
+          ptx::tma_store_4d(ms, Stg + 64 * HD, (kCw >> 1) + h * (HD / 2), j, m * 128, b);
         } else {
           ptx::tma_store_4d(ms, Stg, h * kHd, j, m * 128, b);
-          if (FMT != FMT_SPLIT16) ptx::tma_store_4d(ms, Stg + 8192, kC + h * kHd, j, m * 128, b);
+          if (FMT != FMT_SPLIT16) ptx::tma_store_4d(ms, Stg + 8192, kCw + h * kHd, j, m * 128, b);
         }
         ptx::bulk_commit();
         ptx::bulk_wait_read_all();           // Stg / Q_m have been read: the tile has left shared memory
@@ -736,6 +788,7 @@ attn_temporal_tc2_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __gri
                          const __grid_constant__ CUtensorMap tm_second, uint8_t* __restrict__ sf_out, int F, int J,
                          int n_units, int n_mt, int NKp, int n_stage) {
   constexpr int NSLOT = 2;
+  constexpr int kC = Width<512>::kC, kHd = Width<512>::kHd;     // built for C = 512 only
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const int stage_bytes = 3 * n_mt * kTile;
@@ -1096,10 +1149,10 @@ int encode_tokens_2d(CUtensorMap* out, void* base, CUtensorMapDataType dt, int e
 }
 
 inline int tc_stages(int n_mt) { return n_mt == 1 ? 4 : 2; }
-template <int NSLOT>
+template <int HD, int NSLOT>
 int tc_smem_bytes(int n_mt) {
-  return tc_stages(n_mt) * 3 * n_mt * kTile + NSLOT * (NSLOT == 2 ? kTile : 8192) + static_cast<int>(sizeof(TcBars<NSLOT>)) +
-         1024 /*alignment slack*/;
+  return tc_stages(n_mt) * 3 * n_mt * tile_bytes<HD>() + NSLOT * (NSLOT == 2 ? tile_bytes<HD>() : 8192) +
+         static_cast<int>(sizeof(TcBars<NSLOT>)) + 1024 /*alignment slack*/;
 }
 
 }  // namespace
@@ -1111,88 +1164,138 @@ inline bool three_slots() {
 }
 inline int packed_group(int F) { return F <= 32 ? 4 : (F <= 64 ? 2 : 1); }     // joints per 128-row tile
 
-int make_attn_tc_maps(AttnTcMaps* maps, const __half* qkv, __half* o_hi, __half* o_second, int fmt, int F, int J,
+// Q / K / V and hi boxes of a head: {HD halves} rows, 128 B (SWIZZLE_128B) at C = 512, 64 B (SWIZZLE_64B) at C = 256;
+// the c4 boxes of the F4C second array: HD / 2 bytes of one part, no swizzle
+int make_attn_tc_maps(int C, AttnTcMaps* maps, const __half* qkv, __half* o_hi, __half* o_second, int fmt, int F, int J,
                       int64_t max_clips) {
-  const int G = packed_group(F);
-  if (encode_tokens_4d(&maps->qkv, const_cast<__half*>(qkv), CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, kQkvRow, J, F, max_clips,
-                       CU_TENSOR_MAP_SWIZZLE_128B, 64, G))
+  if (!width_supported(C) || (C != 512 && fmt != FMT_F4C)) return -2;
+  const int G = packed_group(F), hd = C / kHeads;
+  const CUtensorMapSwizzle swz = C == 512 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
+  if (encode_tokens_4d(&maps->qkv, const_cast<__half*>(qkv), CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, 4 * C, J, F, max_clips,
+                       swz, hd, G))
     return -1;
-  if (encode_tokens_4d(&maps->o_hi, o_hi, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, kC, J, F, max_clips,
-                       CU_TENSOR_MAP_SWIZZLE_128B, 64, G))
+  if (encode_tokens_4d(&maps->o_hi, o_hi, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, C, J, F, max_clips, swz, hd, G))
     return -1;
   if (fmt == FMT_F8C)
-    return encode_tokens_4d(&maps->o_second, o_second, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, 2 * kC, J, F, max_clips,
+    return encode_tokens_4d(&maps->o_second, o_second, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, 2 * C, J, F, max_clips,
                             CU_TENSOR_MAP_SWIZZLE_NONE, 64, G);
-  if (fmt == FMT_F4C)       // c4 rows of K = 512 bytes; {32 B x 128 rows} boxes (one head of one part)
-    return encode_tokens_4d(&maps->o_second, o_second, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, kC, J, F, max_clips,
-                            CU_TENSOR_MAP_SWIZZLE_NONE, 32, G);
-  return encode_tokens_4d(&maps->o_second, o_second, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, kC, J, F, max_clips,
+  if (fmt == FMT_F4C)       // c4 rows of K = C bytes; {HD / 2 B x 128 rows} boxes (one head of one part)
+    return encode_tokens_4d(&maps->o_second, o_second, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, C, J, F, max_clips,
+                            CU_TENSOR_MAP_SWIZZLE_NONE, hd / 2, G);
+  return encode_tokens_4d(&maps->o_second, o_second, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, C, J, F, max_clips,
                           CU_TENSOR_MAP_SWIZZLE_128B, 64, G);
 }
 
-int make_attn_tc_maps_spatial(AttnTcMaps* maps, const __half* qkv, __half* o_hi, __half* o_second, int fmt,
+int make_attn_tc_maps_spatial(int C, AttnTcMaps* maps, const __half* qkv, __half* o_hi, __half* o_second, int fmt,
                               int64_t tokens, int F) {
+  if (!width_supported(C) || (C != 512 && fmt != FMT_F4C)) return -2;
+  const int hd = C / kHeads;
+  const CUtensorMapSwizzle swz = C == 512 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
   const int tail_rows = (F % 7) ? (F % 7) * 17 : kSpatialRows;
-  if (encode_tokens_2d(&maps->o_hi_tail, o_hi, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, kC, tokens, tail_rows,
-                       CU_TENSOR_MAP_SWIZZLE_128B))
+  if (encode_tokens_2d(&maps->o_hi_tail, o_hi, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, C, tokens, tail_rows, swz, hd))
     return -1;
-  if (fmt == FMT_F8C   ? encode_tokens_2d(&maps->o_second_tail, o_second, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, 2 * kC, tokens,
+  if (fmt == FMT_F8C   ? encode_tokens_2d(&maps->o_second_tail, o_second, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, 2 * C, tokens,
                                           tail_rows, CU_TENSOR_MAP_SWIZZLE_NONE)
-      : fmt == FMT_F4C ? encode_tokens_2d(&maps->o_second_tail, o_second, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, kC, tokens,
-                                          tail_rows, CU_TENSOR_MAP_SWIZZLE_NONE, 32)
-                       : encode_tokens_2d(&maps->o_second_tail, o_second, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, kC, tokens,
+      : fmt == FMT_F4C ? encode_tokens_2d(&maps->o_second_tail, o_second, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, C, tokens,
+                                          tail_rows, CU_TENSOR_MAP_SWIZZLE_NONE, hd / 2)
+                       : encode_tokens_2d(&maps->o_second_tail, o_second, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, C, tokens,
                                           tail_rows, CU_TENSOR_MAP_SWIZZLE_128B))
     return -1;
   // loads: 128-row boxes (rows beyond the 119 of a unit are read but masked); stores: 119-row boxes
-  if (encode_tokens_2d(&maps->qkv, const_cast<__half*>(qkv), CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, kQkvRow, tokens, 128,
-                       CU_TENSOR_MAP_SWIZZLE_128B))
+  if (encode_tokens_2d(&maps->qkv, const_cast<__half*>(qkv), CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, 4 * C, tokens, 128, swz, hd))
     return -1;
-  if (encode_tokens_2d(&maps->o_hi, o_hi, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, kC, tokens, kSpatialRows,
-                       CU_TENSOR_MAP_SWIZZLE_128B))
+  if (encode_tokens_2d(&maps->o_hi, o_hi, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, C, tokens, kSpatialRows, swz, hd))
     return -1;
   if (fmt == FMT_F8C)
-    return encode_tokens_2d(&maps->o_second, o_second, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, 2 * kC, tokens, kSpatialRows,
+    return encode_tokens_2d(&maps->o_second, o_second, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, 2 * C, tokens, kSpatialRows,
                             CU_TENSOR_MAP_SWIZZLE_NONE);
   if (fmt == FMT_F4C)
-    return encode_tokens_2d(&maps->o_second, o_second, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, kC, tokens, kSpatialRows,
-                            CU_TENSOR_MAP_SWIZZLE_NONE, 32);
-  return encode_tokens_2d(&maps->o_second, o_second, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, kC, tokens, kSpatialRows,
+    return encode_tokens_2d(&maps->o_second, o_second, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, C, tokens, kSpatialRows,
+                            CU_TENSOR_MAP_SWIZZLE_NONE, hd / 2);
+  return encode_tokens_2d(&maps->o_second, o_second, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, C, tokens, kSpatialRows,
                           CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
 cudaError_t configure_attention_tc() {
   cudaError_t e;
-#define D3D_CFG_TC(FMT_, NCH_, SP_)                                                                                       \
-  if ((e = cudaFuncSetAttribute(attn_temporal_tc_kernel<FMT_, 2, NCH_, SP_>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                tc_smem_bytes<2>(2))) != cudaSuccess)                                                    \
+#define D3D_CFG_TC(FMT_, NCH_, SP_)                                                                                           \
+  if ((e = cudaFuncSetAttribute(attn_temporal_tc_kernel<64, FMT_, 2, NCH_, SP_>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                                tc_smem_bytes<64, 2>(2))) != cudaSuccess)                                                    \
     return e;
   D3D_CFG_TC(FMT_SPLIT16, 0, false) D3D_CFG_TC(FMT_F8C, 0, false) D3D_CFG_TC(FMT_SPLIT16, 3, false)
   D3D_CFG_TC(FMT_F8C, 3, false) D3D_CFG_TC(FMT_SPLIT16, 8, false) D3D_CFG_TC(FMT_F8C, 8, false)
   D3D_CFG_TC(FMT_SPLIT16, 0, true) D3D_CFG_TC(FMT_F8C, 0, true)
   D3D_CFG_TC(FMT_F4C, 0, false) D3D_CFG_TC(FMT_F4C, 3, false) D3D_CFG_TC(FMT_F4C, 8, false) D3D_CFG_TC(FMT_F4C, 0, true)
 #undef D3D_CFG_TC
-  if ((e = cudaFuncSetAttribute(attn_temporal_tc_kernel<FMT_F4C, 3, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                tc_smem_bytes<3>(1))) != cudaSuccess)
+  if ((e = cudaFuncSetAttribute(attn_temporal_tc_kernel<64, FMT_F4C, 3, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                tc_smem_bytes<64, 3>(1))) != cudaSuccess)
     return e;
-  if ((e = cudaFuncSetAttribute(attn_temporal_tc_kernel<FMT_F4C, 3, 0, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                tc_smem_bytes<3>(1))) != cudaSuccess)
+  if ((e = cudaFuncSetAttribute(attn_temporal_tc_kernel<64, FMT_F4C, 3, 0, false, true>,
+                                cudaFuncAttributeMaxDynamicSharedMemorySize, tc_smem_bytes<64, 3>(1))) != cudaSuccess)
     return e;
   for (auto kern : {attn_temporal_tc2_kernel<8>, attn_temporal_tc2_kernel<3>, attn_temporal_tc2_kernel<0>})
-    if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, tc_smem_bytes<2>(2))) != cudaSuccess) return e;
-#define D3D_CFG_PK(FMT_)                                                                                                     \
-  if ((e = cudaFuncSetAttribute(attn_temporal_tc_kernel<FMT_, 2, 0, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                tc_smem_bytes<2>(1))) != cudaSuccess)                                                        \
+    if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, tc_smem_bytes<64, 2>(2))) != cudaSuccess) return e;
+#define D3D_CFG_PK(FMT_)                                                                                                         \
+  if ((e = cudaFuncSetAttribute(attn_temporal_tc_kernel<64, FMT_, 2, 0, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                                tc_smem_bytes<64, 2>(1))) != cudaSuccess)                                                        \
     return e;
   D3D_CFG_PK(FMT_SPLIT16) D3D_CFG_PK(FMT_F8C) D3D_CFG_PK(FMT_F4C)
 #undef D3D_CFG_PK
+  // C = 256 (head_dim 32): the FMT_F4C kernel in its temporal, packed and spatial modes
+  for (auto kern : {attn_temporal_tc_kernel<32, FMT_F4C, 2, 0, false>, attn_temporal_tc_kernel<32, FMT_F4C, 2, 3, false>,
+                    attn_temporal_tc_kernel<32, FMT_F4C, 2, 8, false>})
+    if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, tc_smem_bytes<32, 2>(2))) != cudaSuccess) return e;
+  for (auto kern : {attn_temporal_tc_kernel<32, FMT_F4C, 2, 0, true>, attn_temporal_tc_kernel<32, FMT_F4C, 2, 0, false, true>})
+    if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, tc_smem_bytes<32, 2>(1))) != cudaSuccess) return e;
   return cudaSuccess;
 }
 
-cudaError_t launch_attn_temporal_tc(const AttnTcMaps& maps, const __half* qkv, uint8_t* o_sf, int fmt, int B, int F, int J,
-                                    int num_sms, cudaStream_t st, int wg2) {
+namespace {
+// C = 256: every mode on the head_dim-32 FMT_F4C kernel (two slots; the three-slot and two-warpgroup variants are C = 512 only)
+cudaError_t launch_attn_tc_hd32(const AttnTcMaps& maps, uint8_t* o_sf, int fmt, int B, int F, int J, bool spatial,
+                                int num_sms, cudaStream_t st) {
+  if (fmt != FMT_F4C || !o_sf) return cudaErrorInvalidValue;
+  if (spatial) {
+    const int G = (F + 6) / 7;
+    const int64_t units64 = static_cast<int64_t>(B) * G * kHeads;
+    if (units64 > 0x7fffffff) return cudaErrorInvalidValue;
+    const int n_units = static_cast<int>(units64);
+    const int grid = n_units < num_sms ? n_units : num_sms;
+    attn_temporal_tc_kernel<32, FMT_F4C, 2, 0, true><<<grid, kTcThreads, tc_smem_bytes<32, 2>(1), st>>>(
+        maps.qkv, maps.o_hi, maps.o_second, maps.o_hi_tail, maps.o_second_tail, o_sf, F, G, n_units, 1, 128, tc_stages(1));
+    return cudaGetLastError();
+  }
+  if (F <= 64) {
+    const int G = packed_group(F), JG = (J + G - 1) / G;
+    const int64_t units64 = static_cast<int64_t>(B) * JG * kHeads;
+    if (units64 > 0x7fffffff) return cudaErrorInvalidValue;
+    const int n_units = static_cast<int>(units64);
+    const int grid = n_units < num_sms ? n_units : num_sms;
+    attn_temporal_tc_kernel<32, FMT_F4C, 2, 0, false, true><<<grid, kTcThreads, tc_smem_bytes<32, 2>(1), st>>>(
+        maps.qkv, maps.o_hi, maps.o_second, maps.o_hi, maps.o_second, o_sf, F, JG, n_units, 1, 128, tc_stages(1), G, J);
+    return cudaGetLastError();
+  }
+  const int n_mt = (F + 127) / 128;
+  const int NKp = (F + 15) / 16 * 16;
+  const int n_units = B * J * kHeads;
+  const int n_chunks = (NKp + 31) / 32;
+  const int nch = (n_chunks == 8 && F > 224) ? 8 : ((n_chunks == 3 && F > 64) ? 3 : 0);
+  const int grid = n_units < num_sms ? n_units : num_sms;
+  auto kern = nch == 8 ? attn_temporal_tc_kernel<32, FMT_F4C, 2, 8, false>
+            : nch == 3 ? attn_temporal_tc_kernel<32, FMT_F4C, 2, 3, false> : attn_temporal_tc_kernel<32, FMT_F4C, 2, 0, false>;
+  kern<<<grid, kTcThreads, tc_smem_bytes<32, 2>(n_mt), st>>>(maps.qkv, maps.o_hi, maps.o_second, maps.o_hi, maps.o_second, o_sf,
+                                                             F, J, n_units, n_mt, NKp, tc_stages(n_mt), 1, 0);
+  return cudaGetLastError();
+}
+}  // namespace
+
+cudaError_t launch_attn_temporal_tc(int C, const AttnTcMaps& maps, const __half* qkv, uint8_t* o_sf, int fmt, int B, int F,
+                                    int J, int num_sms, cudaStream_t st, int wg2) {
   if (B <= 0) return cudaSuccess;
   if (F < 1 || F > 256) return cudaErrorInvalidValue;
   if (fmt == FMT_F4C && !o_sf) return cudaErrorInvalidValue;
+  if (C == 256) return wg2 ? cudaErrorInvalidValue : launch_attn_tc_hd32(maps, o_sf, fmt, B, F, J, false, num_sms, st);
+  if (C != 512) return cudaErrorInvalidValue;
   if (F <= 64) {
     // packed mode: G joints of one (clip, head) per 128-row tile; the maps were built with {.., G, 128 / G, 1} boxes
     const int G = packed_group(F), JG = (J + G - 1) / G;
@@ -1200,12 +1303,12 @@ cudaError_t launch_attn_temporal_tc(const AttnTcMaps& maps, const __half* qkv, u
     if (units64 > 0x7fffffff) return cudaErrorInvalidValue;
     const int n_units = static_cast<int>(units64);
     const int grid = n_units < num_sms ? n_units : num_sms;
-    const int smem = tc_smem_bytes<2>(1);
+    const int smem = tc_smem_bytes<64, 2>(1);
 #define D3D_LAUNCH_PK(FMT_)                                                                   \
-  attn_temporal_tc_kernel<FMT_, 2, 0, false, true><<<grid, kTcThreads, smem, st>>>(           \
+  attn_temporal_tc_kernel<64, FMT_, 2, 0, false, true><<<grid, kTcThreads, smem, st>>>(       \
       maps.qkv, maps.o_hi, maps.o_second, maps.o_hi, maps.o_second, o_sf, F, JG, n_units, 1, 128, tc_stages(1), G, J)
     if (fmt == FMT_F4C && three_slots())
-      attn_temporal_tc_kernel<FMT_F4C, 3, 0, false, true><<<grid, 512, tc_smem_bytes<3>(1), st>>>(
+      attn_temporal_tc_kernel<64, FMT_F4C, 3, 0, false, true><<<grid, 512, tc_smem_bytes<64, 3>(1), st>>>(
           maps.qkv, maps.o_hi, maps.o_second, maps.o_hi, maps.o_second, o_sf, F, JG, n_units, 1, 128, tc_stages(1), G, J);
     else if (fmt == FMT_F4C) D3D_LAUNCH_PK(FMT_F4C);
     else if (fmt == FMT_F8C) D3D_LAUNCH_PK(FMT_F8C);
@@ -1219,9 +1322,9 @@ cudaError_t launch_attn_temporal_tc(const AttnTcMaps& maps, const __half* qkv, u
   const int n_chunks = (NKp + 31) / 32;
   const int nch = (n_chunks == 8 && F > 224) ? 8 : ((n_chunks == 3 && F > 64) ? 3 : 0);   // F = 243 / 81 specialisations
   const int grid = n_units < num_sms ? n_units : num_sms;
-  const int smem = tc_smem_bytes<2>(n_mt);
+  const int smem = tc_smem_bytes<64, 2>(n_mt);
 #define D3D_LAUNCH_TC(FMT_, NCH_)                                                                               \
-  attn_temporal_tc_kernel<FMT_, 2, NCH_, false><<<grid, kTcThreads, smem, st>>>(                      \
+  attn_temporal_tc_kernel<64, FMT_, 2, NCH_, false><<<grid, kTcThreads, smem, st>>>(                            \
       maps.qkv, maps.o_hi, maps.o_second, maps.o_hi, maps.o_second, o_sf, F, J, n_units, n_mt, NKp, tc_stages(n_mt))
   if (fmt == FMT_F4C && wg2) {
     // two softmax warpgroups per slot (D3D_ATTN_WG2=0: the one-warpgroup kernel)
@@ -1244,28 +1347,30 @@ cudaError_t launch_attn_temporal_tc(const AttnTcMaps& maps, const __half* qkv, u
 }
 
 // Spatial mode (J == 17): units of (clip, 7-frame group, head)
-cudaError_t launch_attn_spatial_tc(const AttnTcMaps& maps, uint8_t* o_sf, int fmt, int B, int F, int num_sms,
+cudaError_t launch_attn_spatial_tc(int C, const AttnTcMaps& maps, uint8_t* o_sf, int fmt, int B, int F, int num_sms,
                                    cudaStream_t st) {
   if (B <= 0) return cudaSuccess;
+  if (C == 256) return launch_attn_tc_hd32(maps, o_sf, fmt, B, F, 17, true, num_sms, st);
+  if (C != 512) return cudaErrorInvalidValue;
   const int G = (F + 6) / 7;
   const int64_t units64 = static_cast<int64_t>(B) * G * kHeads;
   if (units64 > 0x7fffffff) return cudaErrorInvalidValue;
   const int n_units = static_cast<int>(units64);
   const int grid = n_units < num_sms ? n_units : num_sms;
-  const int smem = tc_smem_bytes<2>(1);
+  const int smem = tc_smem_bytes<64, 2>(1);
   if (fmt == FMT_F4C && three_slots()) {
     if (!o_sf) return cudaErrorInvalidValue;
-    attn_temporal_tc_kernel<FMT_F4C, 3, 0, true><<<grid, 512, tc_smem_bytes<3>(1), st>>>(
+    attn_temporal_tc_kernel<64, FMT_F4C, 3, 0, true><<<grid, 512, tc_smem_bytes<64, 3>(1), st>>>(
         maps.qkv, maps.o_hi, maps.o_second, maps.o_hi_tail, maps.o_second_tail, o_sf, F, G, n_units, 1, 128, tc_stages(1));
   } else if (fmt == FMT_F4C) {
     if (!o_sf) return cudaErrorInvalidValue;
-    attn_temporal_tc_kernel<FMT_F4C, 2, 0, true><<<grid, kTcThreads, smem, st>>>(
+    attn_temporal_tc_kernel<64, FMT_F4C, 2, 0, true><<<grid, kTcThreads, smem, st>>>(
         maps.qkv, maps.o_hi, maps.o_second, maps.o_hi_tail, maps.o_second_tail, o_sf, F, G, n_units, 1, 128, tc_stages(1));
   } else if (fmt == FMT_F8C) {
-    attn_temporal_tc_kernel<FMT_F8C, 2, 0, true><<<grid, kTcThreads, smem, st>>>(
+    attn_temporal_tc_kernel<64, FMT_F8C, 2, 0, true><<<grid, kTcThreads, smem, st>>>(
         maps.qkv, maps.o_hi, maps.o_second, maps.o_hi_tail, maps.o_second_tail, o_sf, F, G, n_units, 1, 128, tc_stages(1));
   } else {
-    attn_temporal_tc_kernel<FMT_SPLIT16, 2, 0, true><<<grid, kTcThreads, smem, st>>>(
+    attn_temporal_tc_kernel<64, FMT_SPLIT16, 2, 0, true><<<grid, kTcThreads, smem, st>>>(
         maps.qkv, maps.o_hi, maps.o_second, maps.o_hi_tail, maps.o_second_tail, o_sf, F, G, n_units, 1, 128, tc_stages(1));
   }
   return cudaGetLastError();

@@ -38,7 +38,7 @@ struct Lin {
 struct Blk {
   float *n1g = nullptr, *n1b = nullptr, *n2g = nullptr, *n2b = nullptr;
   Lin qkv, proj, fc1, fc2;
-  float *tw = nullptr, *tb = nullptr;   // per-block time Linear(1024 -> 512), fp32
+  float *tw = nullptr, *tb = nullptr;   // per-block time Linear(2 C -> C), fp32
   bool have_t = false;
 };
 
@@ -54,6 +54,7 @@ struct OperandBuf {   // a GEMM A operand living in the workspace
 struct d3d_handle {
   d3d_config cfg{};
   int F = 0, J = 0, nblk = 0, num_sms = 148;
+  int C = 512, hidden = 1024;   // embed_dim (selects the kernel instantiations) and mlp hidden width 2 C
   int fmt = FMT_SPLIT16;   // GEMM operand format of the workspace and the packed weights (operand.cuh)
   int64_t tok_cap = 0;   // workspace rows (multiple of 128)
   std::string err;
@@ -69,9 +70,9 @@ struct d3d_handle {
 
   // workspace
   float* X = nullptr;
-  __half* QKV = nullptr;     // packed fp16 q | k | v_hi | v_lo, [tok_cap, 2048]
+  __half* QKV = nullptr;     // packed fp16 q | k | v_hi | v_lo, [tok_cap, 4 C]
   OperandBuf A, ATT, H;
-  CUtensorMap m_x;              // fp32 [tok_cap, 512] view of X in {32 x 32} boxes: destination of the EPI_F32_RED epilogue
+  CUtensorMap m_x;              // fp32 [tok_cap, C] view of X in {32 x 32} boxes: destination of the EPI_F32_RED epilogue
   bool have_m_x = false;
   AttnTcMaps attn_tc;        // tcgen05 temporal attention: maps bound to QKV -> ATT
   bool have_attn_tc = false;
@@ -81,9 +82,9 @@ struct d3d_handle {
   int64_t in_noise_cap = 0;
   float *t_f32 = nullptr, *e0 = nullptr, *h1 = nullptr, *h2 = nullptr;   // time-MLP scratch, max(max_clips, S) rows
   int t_rows_cap = 0;
-  float* tv_steps = nullptr;     // [S, nblk, 512] table for the DDIM loop
+  float* tv_steps = nullptr;     // [S, nblk, C] table for the DDIM loop
   int tv_cap = 0;
-  float* tv_general = nullptr;   // [max_clips, nblk, 512] for per-sample t
+  float* tv_general = nullptr;   // [max_clips, nblk, C] for per-sample t
   int32_t* perm_dev = nullptr;
   int32_t perm_host[64];
   bool perm_valid = false;
@@ -310,6 +311,19 @@ bool attn_tc_has_f4c() { return D3D_ATTN_TC_F4C != 0; }
 int run_attention(d3d_handle* h, const __half* qkv, __half* o_hi, __half* o_lo, float* o_f32, int B, bool spatial,
                   int mode, cudaStream_t st) {
   const int64_t T_all = static_cast<int64_t>(B) * h->F * h->J;
+  if (h->C != 512) {
+    // C = 256: the tcgen05 kernel in every mode, whatever the A/B switches say (the other kernels are built for 512)
+    if (mode != D3D_ATTN_DEFAULT) return fail(h, -3, "embed_dim 256 runs attn_mode D3D_ATTN_DEFAULT only");
+    if (qkv != h->QKV || (!o_f32 && (o_hi != h->ATT.hi || o_lo != h->ATT.lo)))
+      return fail(h, -2, "attention output must be the ATT operand");
+    if (spatial)
+      KLP(D3D_PROF_ATTN_SPATIAL, st, launch_attn_spatial_tc(h->C, h->attn_sp, h->ATT.sf, h->fmt, B, h->F, h->num_sms, st));
+    else
+      KLP(D3D_PROF_ATTN_TEMPORAL, st,
+          launch_attn_temporal_tc(h->C, h->attn_tc, qkv, h->ATT.sf, h->fmt, B, h->F, h->J, h->num_sms, st, 0));
+    if (o_f32) KL(launch_merge(h->ATT.hi, h->ATT.lo, h->ATT.sf, o_f32, T_all, h->C, h->fmt, st));
+    return 0;
+  }
   const bool tc_path = mode == D3D_ATTN_DEFAULT && qkv == h->QKV &&
                        (spatial ? (h->have_attn_sp && h->J == 17 && env_int("D3D_ATTN_TC_SPATIAL", 1))
                                 : (h->have_attn_tc && env_int("D3D_ATTN_TC", 1)));
@@ -321,7 +335,7 @@ int run_attention(d3d_handle* h, const __half* qkv, __half* o_hi, __half* o_lo, 
     int r = run_attention(h, qkv, nullptr, nullptr, scratch, B, spatial, mode == D3D_ATTN_DEFAULT ? D3D_ATTN_MMA_SYNC : mode, st);
     if (r) return r;
     KLP(spatial ? D3D_PROF_ATTN_SPATIAL : D3D_PROF_ATTN_TEMPORAL, st,
-        launch_split(scratch, h->ATT.hi, h->ATT.lo, h->ATT.sf, T_all, kC, FMT_F4C, 0, st));
+        launch_split(scratch, h->ATT.hi, h->ATT.lo, h->ATT.sf, T_all, h->C, FMT_F4C, 0, st));
     return 0;
   }
   if (spatial) {
@@ -330,8 +344,8 @@ int run_attention(d3d_handle* h, const __half* qkv, __half* o_hi, __half* o_lo, 
     } else if (tc_path && (h->fmt != FMT_F4C || attn_tc_has_f4c())) {
       if (!o_f32 && (o_hi != h->ATT.hi || o_lo != h->ATT.lo)) return fail(h, -2, "attention output must be the ATT operand");
       const int64_t T = static_cast<int64_t>(B) * h->F * h->J;
-      KLP(D3D_PROF_ATTN_SPATIAL, st, launch_attn_spatial_tc(h->attn_sp, h->ATT.sf, h->fmt, B, h->F, h->num_sms, st));
-      if (o_f32) KL(launch_merge(h->ATT.hi, h->ATT.lo, h->ATT.sf, o_f32, T, kC, h->fmt, st));
+      KLP(D3D_PROF_ATTN_SPATIAL, st, launch_attn_spatial_tc(h->C, h->attn_sp, h->ATT.sf, h->fmt, B, h->F, h->num_sms, st));
+      if (o_f32) KL(launch_merge(h->ATT.hi, h->ATT.lo, h->ATT.sf, o_f32, T, h->C, h->fmt, st));
     } else {
       KLP(D3D_PROF_ATTN_SPATIAL, st, launch_attn_spatial(qkv, o_hi, o_lo, o_f32, h->fmt, static_cast<int64_t>(B) * h->F, h->J, st));
     }
@@ -342,9 +356,9 @@ int run_attention(d3d_handle* h, const __half* qkv, __half* o_hi, __half* o_lo, 
       // the tcgen05 kernel's tensor maps are bound to QKV -> ATT; an fp32 result (op-level entry point) is merged
       // from the operand pair afterwards
       if (!o_f32 && (o_hi != h->ATT.hi || o_lo != h->ATT.lo)) return fail(h, -2, "attention output must be the ATT operand");
-      KLP(D3D_PROF_ATTN_TEMPORAL, st, launch_attn_temporal_tc(h->attn_tc, qkv, h->ATT.sf, h->fmt, B, h->F, h->J, h->num_sms, st,
+      KLP(D3D_PROF_ATTN_TEMPORAL, st, launch_attn_temporal_tc(h->C, h->attn_tc, qkv, h->ATT.sf, h->fmt, B, h->F, h->J, h->num_sms, st,
                                                               env_int("D3D_ATTN_WG2", 0)));
-      if (o_f32) KL(launch_merge(h->ATT.hi, h->ATT.lo, h->ATT.sf, o_f32, static_cast<int64_t>(B) * h->F * h->J, kC, h->fmt, st));
+      if (o_f32) KL(launch_merge(h->ATT.hi, h->ATT.lo, h->ATT.sf, o_f32, static_cast<int64_t>(B) * h->F * h->J, h->C, h->fmt, st));
     } else {
       KLP(D3D_PROF_ATTN_TEMPORAL, st, launch_attn_temporal_mma(qkv, o_hi, o_lo, o_f32, h->fmt, B, h->F, h->J, st));
     }
@@ -375,24 +389,24 @@ int check_weights(d3d_handle* h) {
   return 0;
 }
 
-// [R] fp32 timesteps (device) -> table [R, nblk, 512]
+// [R] fp32 timesteps (device) -> table [R, nblk, C]
 int compute_time_table(d3d_handle* h, const float* t_dev, int R, float* table, cudaStream_t st) {
-  KL(launch_sincos(t_dev, R, h->e0, st));
-  KL(launch_small_linear(h->e0, R, kC, h->tm1w, h->tm1b, 2 * kC, 0, h->h1, 2 * kC, st));
-  KL(launch_small_linear(h->h1, R, 2 * kC, h->tm3w, h->tm3b, 2 * kC, 1, h->h2, 2 * kC, st));
+  KL(launch_sincos(h->C, t_dev, R, h->e0, st));
+  KL(launch_small_linear(h->e0, R, h->C, h->tm1w, h->tm1b, 2 * h->C, 0, h->h1, 2 * h->C, st));
+  KL(launch_small_linear(h->h1, R, 2 * h->C, h->tm3w, h->tm3b, 2 * h->C, 1, h->h2, 2 * h->C, st));
   for (int b = 0; b < h->nblk; ++b)
-    KL(launch_small_linear(h->h2, R, 2 * kC, h->blk[b].tw, h->blk[b].tb, kC, 2, table + b * kC,
-                           static_cast<int64_t>(h->nblk) * kC, st));
+    KL(launch_small_linear(h->h2, R, 2 * h->C, h->blk[b].tw, h->blk[b].tb, h->C, 2, table + b * h->C,
+                           static_cast<int64_t>(h->nblk) * h->C, st));
   return 0;
 }
 
 // The row-wise launches of a denoiser call with the parameters they read (shared by run_blocks and d3d_debug_rowwise).
-// tv: time table of the call ([rows][nblk][512], block 0 first) or null; tv_stride: its row stride (0 = one row for
+// tv: time table of the call ([rows][nblk][C], block 0 first) or null; tv_stride: its row stride (0 = one row for
 // every clip).
 // lift: X = fusion_layer(input) + Spatial_pos_embed + time vector of block 0;  A = norm1 of block 0 (X)
 int lift_launch(d3d_handle* h, const float* x2d, const float* y, const float* x5, const float* tv, int64_t tv_stride,
                 int64_t T, cudaStream_t st) {
-  KLP(D3D_PROF_LIFT, st, launch_lift_ln(x2d, y, x5, h->wf_t, h->bf, h->spos, tv, tv_stride,
+  KLP(D3D_PROF_LIFT, st, launch_lift_ln(h->C, x2d, y, x5, h->wf_t, h->bf, h->spos, tv, tv_stride,
                                         LnParams{h->blk[0].n1g, h->blk[0].n1b}, h->X, h->A.hi, h->A.lo, h->A.sf, h->fmt, T, h->J,
                                         h->F * h->J, st));
   return 0;
@@ -403,13 +417,13 @@ int postnorm_launch(d3d_handle* h, int b, const float* tv, int64_t tv_stride, in
   const LnParams post = ((b - 1) % 2 == 0) ? LnParams{h->sn_g, h->sn_b} : LnParams{h->tn_g, h->tn_b};
   const Blk& nx = h->blk[b];
   KLP(D3D_PROF_LN, st,
-      launch_postnorm_add_ln(h->X, post, (b == 1) ? h->tpos : nullptr, tv ? tv + b * kC : nullptr, tv_stride,
+      launch_postnorm_add_ln(h->C, h->X, post, (b == 1) ? h->tpos : nullptr, tv ? tv + b * h->C : nullptr, tv_stride,
                              LnParams{nx.n1g, nx.n1b}, h->A.hi, h->A.lo, h->A.sf, h->fmt, T, h->J, h->F, st));
   return 0;
 }
 // A = norm2 of block b (X)
 int norm2_launch(d3d_handle* h, int b, int64_t T, cudaStream_t st) {
-  KLP(D3D_PROF_LN, st, launch_ln_split(h->X, LnParams{h->blk[b].n2g, h->blk[b].n2b}, 1e-6f, h->A.hi, h->A.lo, h->A.sf, h->fmt,
+  KLP(D3D_PROF_LN, st, launch_ln_split(h->C, h->X, LnParams{h->blk[b].n2g, h->blk[b].n2b}, 1e-6f, h->A.hi, h->A.lo, h->A.sf, h->fmt,
                                        T, st));
   return 0;
 }
@@ -440,7 +454,7 @@ int run_blocks(d3d_handle* h, const float* x2d, const float* y, const float* x5,
 int run_head(d3d_handle* h, const DdimStep& s, float* y, const float* noise, float* out3, float* trace_y,
              float* trace_x0, int trace_idx, int B, cudaStream_t st) {
   const int64_t T = static_cast<int64_t>(B) * h->F * h->J;
-  KLP(D3D_PROF_HEAD, st, launch_head_ddim(h->X, LnParams{h->tn_g, h->tn_b}, LnParams{h->hg, h->hb}, h->wh, h->bh, s,
+  KLP(D3D_PROF_HEAD, st, launch_head_ddim(h->C, h->X, LnParams{h->tn_g, h->tn_b}, LnParams{h->hg, h->hb}, h->wh, h->bh, s,
                                           y, noise, out3, trace_y, trace_x0, h->S, trace_idx, T, st));
   return 0;
 }
@@ -470,13 +484,13 @@ int prep_batch(d3d_handle* h, int B, cudaStream_t st) {
   const int64_t T = static_cast<int64_t>(B) * h->F * h->J;
   if (T < h->qkv_rows_dirty) {
     const int64_t rows = std::min<int64_t>(128, h->tok_cap - T);
-    if (rows > 0) CK(cudaMemsetAsync(h->QKV + T * kQkvRow, 0, static_cast<size_t>(rows) * kQkvRow * sizeof(__half), st));
+    if (rows > 0) CK(cudaMemsetAsync(h->QKV + T * (4 * h->C), 0, static_cast<size_t>(rows) * (4 * h->C) * sizeof(__half), st));
   }
   if (T > h->qkv_rows_dirty) h->qkv_rows_dirty = T;
   return 0;
 }
 
-// per-sample timesteps (int64, device) -> general time table [B, nblk, 512]; everything stays on the stream
+// per-sample timesteps (int64, device) -> general time table [B, nblk, C]; everything stays on the stream
 int general_time_table(d3d_handle* h, const int64_t* t_dev, int B, cudaStream_t st) {
   KL(launch_t_to_f32(t_dev, B, h->t_f32, st));
   return compute_time_table(h, h->t_f32, B, h->tv_general, st);
@@ -485,7 +499,7 @@ int general_time_table(d3d_handle* h, const int64_t* t_dev, int B, cudaStream_t 
 int run_sampler(d3d_handle* h, int B, float* trace_y, float* trace_x0, cudaStream_t st) {
   const int64_t n3 = static_cast<int64_t>(B) * h->F * h->J * 3;
   for (int s = 0; s < h->S; ++s) {
-    const float* tv = h->cfg.with_time_emb ? h->tv_steps + static_cast<int64_t>(s) * h->nblk * kC : nullptr;
+    const float* tv = h->cfg.with_time_emb ? h->tv_steps + static_cast<int64_t>(s) * h->nblk * h->C : nullptr;
     int r = run_blocks(h, h->in_x2d, h->y, nullptr, tv, 0, B, h->nblk, st);
     if (r) return r;
     const float* nz = (h->need_noise && !h->steps[s].last) ? h->in_noise + static_cast<int64_t>(s) * n3 : nullptr;
@@ -535,8 +549,19 @@ int64_t d3d_workspace_bytes(const d3d_handle* h) { return h ? h->alloc_bytes : 0
 int d3d_create(const d3d_config* cfg, d3d_handle** out) {
   if (!cfg || !out) { g_create_error = "null argument"; return -1; }
   *out = nullptr;
-  if (cfg->embed_dim != kC || cfg->num_heads != kHeads || cfg->mlp_hidden != kHidden) {
-    g_create_error = "unsupported shape: kernels are specialised for embed_dim 512, 8 heads, mlp hidden 1024";
+  if (!width_supported(cfg->embed_dim) || cfg->num_heads != kHeads || cfg->mlp_hidden != 2 * cfg->embed_dim) {
+    g_create_error = "unsupported shape: the kernels are instantiated for embed_dim 256 or 512, 8 heads, mlp hidden "
+                     "2 * embed_dim";
+    return -3;
+  }
+  if (cfg->embed_dim != 512 && (cfg->gemm_mode != D3D_GEMM_TC_F4C || cfg->attn_mode != D3D_ATTN_DEFAULT)) {
+    g_create_error = "unsupported mode: embed_dim 256 runs gemm_mode D3D_GEMM_TC_F4C with attn_mode D3D_ATTN_DEFAULT only "
+                     "(the validation and legacy kernels are built for embed_dim 512)";
+    return -3;
+  }
+  if (cfg->embed_dim != 512 && cfg->num_joints != 17) {
+    g_create_error = "unsupported shape: embed_dim 256 needs num_joints 17 (the spatial attention of other joint counts "
+                     "runs on validation kernels built for embed_dim 512)";
     return -3;
   }
   if (cfg->num_frame < 1 || cfg->num_frame > 256 || cfg->num_joints < 1 || cfg->num_joints > 32 || cfg->depth < 1 ||
@@ -560,6 +585,8 @@ int d3d_create(const d3d_config* cfg, d3d_handle** out) {
   DeviceGuard guard(cfg->device);
   d3d_handle* h = new d3d_handle();
   h->cfg = *cfg;
+  h->C = cfg->embed_dim;
+  h->hidden = cfg->mlp_hidden;
   h->fmt = mode_fmt(cfg->gemm_mode);
   h->F = cfg->num_frame;
   h->J = cfg->num_joints;
@@ -580,41 +607,41 @@ int d3d_create(const d3d_config* cfg, d3d_handle** out) {
     CK(configure_attention_mma());
     CK(configure_attention_tc());
     for (auto& b : h->blk) {
-      if ((r = alloc_lin(h, &b.qkv, 3 * kC, kC))) return r;
-      if ((r = alloc_lin(h, &b.proj, kC, kC))) return r;
-      if ((r = alloc_lin(h, &b.fc1, kHidden, kC))) return r;
-      if ((r = alloc_lin(h, &b.fc2, kC, kHidden))) return r;
+      if ((r = alloc_lin(h, &b.qkv, 3 * h->C, h->C))) return r;
+      if ((r = alloc_lin(h, &b.proj, h->C, h->C))) return r;
+      if ((r = alloc_lin(h, &b.fc1, h->hidden, h->C))) return r;
+      if ((r = alloc_lin(h, &b.fc2, h->C, h->hidden))) return r;
       for (float** p : {&b.n1g, &b.n1b, &b.n2g, &b.n2b, &b.tb})
-        if ((r = dev_alloc(h, p, kC))) return r;
-      if ((r = dev_alloc(h, &b.tw, static_cast<int64_t>(kC) * 2 * kC))) return r;
+        if ((r = dev_alloc(h, p, h->C))) return r;
+      if ((r = dev_alloc(h, &b.tw, static_cast<int64_t>(h->C) * 2 * h->C))) return r;
     }
     for (float** p : {&h->bf, &h->sn_g, &h->sn_b, &h->tn_g, &h->tn_b, &h->hg, &h->hb})
-      if ((r = dev_alloc(h, p, kC))) return r;
-    if ((r = dev_alloc(h, &h->wf_t, 5 * kC))) return r;
-    if ((r = dev_alloc(h, &h->spos, static_cast<int64_t>(h->J) * kC))) return r;
-    if ((r = dev_alloc(h, &h->tpos, static_cast<int64_t>(h->F) * kC))) return r;
-    if ((r = dev_alloc(h, &h->wh, 3 * kC))) return r;
+      if ((r = dev_alloc(h, p, h->C))) return r;
+    if ((r = dev_alloc(h, &h->wf_t, 5 * h->C))) return r;
+    if ((r = dev_alloc(h, &h->spos, static_cast<int64_t>(h->J) * h->C))) return r;
+    if ((r = dev_alloc(h, &h->tpos, static_cast<int64_t>(h->F) * h->C))) return r;
+    if ((r = dev_alloc(h, &h->wh, 3 * h->C))) return r;
     if ((r = dev_alloc(h, &h->bh, 4))) return r;
-    if ((r = dev_alloc(h, &h->tm1w, static_cast<int64_t>(2 * kC) * kC))) return r;
-    if ((r = dev_alloc(h, &h->tm1b, 2 * kC))) return r;
-    if ((r = dev_alloc(h, &h->tm3w, static_cast<int64_t>(2 * kC) * 2 * kC))) return r;
-    if ((r = dev_alloc(h, &h->tm3b, 2 * kC))) return r;
+    if ((r = dev_alloc(h, &h->tm1w, static_cast<int64_t>(2 * h->C) * h->C))) return r;
+    if ((r = dev_alloc(h, &h->tm1b, 2 * h->C))) return r;
+    if ((r = dev_alloc(h, &h->tm3w, static_cast<int64_t>(2 * h->C) * 2 * h->C))) return r;
+    if ((r = dev_alloc(h, &h->tm3b, 2 * h->C))) return r;
     if ((r = dev_alloc(h, &h->perm_dev, 64))) return r;
 
-    if ((r = dev_alloc(h, &h->X, h->tok_cap * kC))) return r;
-    if (make_f32_tile_map(&h->m_x, h->X, h->tok_cap, kC)) return fail(h, -20, "cuTensorMapEncodeTiled failed for X");
+    if ((r = dev_alloc(h, &h->X, h->tok_cap * h->C))) return r;
+    if (make_f32_tile_map(&h->m_x, h->X, h->tok_cap, h->C)) return fail(h, -20, "cuTensorMapEncodeTiled failed for X");
     h->have_m_x = true;
-    if ((r = dev_alloc(h, &h->QKV, h->tok_cap * kQkvRow))) return r;
-    if ((r = alloc_operand(h, &h->A, h->tok_cap, kC))) return r;
-    if ((r = alloc_operand(h, &h->ATT, h->tok_cap, kC))) return r;
-    if ((r = alloc_operand(h, &h->H, h->tok_cap, kHidden))) return r;
+    if ((r = dev_alloc(h, &h->QKV, h->tok_cap * (4 * h->C)))) return r;
+    if ((r = alloc_operand(h, &h->A, h->tok_cap, h->C))) return r;
+    if ((r = alloc_operand(h, &h->ATT, h->tok_cap, h->C))) return r;
+    if ((r = alloc_operand(h, &h->H, h->tok_cap, h->hidden))) return r;
     if (h->J == 17) {
-      if (make_attn_tc_maps_spatial(&h->attn_sp, h->QKV, h->ATT.hi, h->ATT.lo, h->fmt, h->tok_cap, h->F))
+      if (make_attn_tc_maps_spatial(h->C, &h->attn_sp, h->QKV, h->ATT.hi, h->ATT.lo, h->fmt, h->tok_cap, h->F))
         return fail(h, -20, "cuTensorMapEncodeTiled failed for the spatial-attention maps");
       h->have_attn_sp = true;
     }
     {   // every F <= 256 runs on the tcgen05 kernel (F <= 64: 2 or 4 joints packed per 128-row tile)
-      if (make_attn_tc_maps(&h->attn_tc, h->QKV, h->ATT.hi, h->ATT.lo, h->fmt, h->F, h->J, cfg->max_clips))
+      if (make_attn_tc_maps(h->C, &h->attn_tc, h->QKV, h->ATT.hi, h->ATT.lo, h->fmt, h->F, h->J, cfg->max_clips))
         return fail(h, -20, "cuTensorMapEncodeTiled failed for the temporal-attention maps");
       h->have_attn_tc = true;
     }
@@ -622,10 +649,10 @@ int d3d_create(const d3d_config* cfg, d3d_handle** out) {
     if ((r = dev_alloc(h, &h->y, T * 3))) return r;
     h->t_rows_cap = cfg->max_clips > 1024 ? cfg->max_clips : 1024;
     if ((r = dev_alloc(h, &h->t_f32, h->t_rows_cap))) return r;
-    if ((r = dev_alloc(h, &h->e0, static_cast<int64_t>(h->t_rows_cap) * kC))) return r;
-    if ((r = dev_alloc(h, &h->h1, static_cast<int64_t>(h->t_rows_cap) * 2 * kC))) return r;
-    if ((r = dev_alloc(h, &h->h2, static_cast<int64_t>(h->t_rows_cap) * 2 * kC))) return r;
-    if ((r = dev_alloc(h, &h->tv_general, static_cast<int64_t>(cfg->max_clips) * h->nblk * kC))) return r;
+    if ((r = dev_alloc(h, &h->e0, static_cast<int64_t>(h->t_rows_cap) * h->C))) return r;
+    if ((r = dev_alloc(h, &h->h1, static_cast<int64_t>(h->t_rows_cap) * 2 * h->C))) return r;
+    if ((r = dev_alloc(h, &h->h2, static_cast<int64_t>(h->t_rows_cap) * 2 * h->C))) return r;
+    if ((r = dev_alloc(h, &h->tv_general, static_cast<int64_t>(cfg->max_clips) * h->nblk * h->C))) return r;
     CK(cudaDeviceSynchronize());
     return 0;
   };
@@ -658,7 +685,7 @@ int d3d_load_weights(d3d_handle* h, const d3d_tensor* tensors, int32_t n) {
   drop_graphs(h);
   h->table_valid = false;
   float* stage = nullptr;   // device staging for tensors that need a transform
-  const int64_t stage_cap = static_cast<int64_t>(3 * kC) * kHidden;
+  const int64_t stage_cap = static_cast<int64_t>(3 * h->C) * h->hidden;
   CK(cudaMalloc(&stage, stage_cap * sizeof(float)));
   struct Free { float* p; ~Free() { cudaFree(p); } } free_stage{stage};
 
@@ -695,28 +722,28 @@ int d3d_load_weights(d3d_handle* h, const d3d_tensor* tensors, int32_t n) {
     if (name.rfind("module.", 0) == 0) name = name.substr(7);
     if (name.rfind("model.", 0) == 0) name = name.substr(6);
     int r = 0;
-    if (name == "fusion_layer.weight") {           // [512,5] -> transposed [5][512]
-      std::vector<float> w(5 * kC), wt(5 * kC);
-      if (t.numel != 5 * kC) return fail(h, -10, "fusion_layer.weight must be [512,5]");
-      CK(cudaMemcpy(w.data(), t.data, sizeof(float) * 5 * kC, t.on_device ? cudaMemcpyDeviceToHost : cudaMemcpyHostToHost));
-      for (int c = 0; c < kC; ++c)
-        for (int k = 0; k < 5; ++k) wt[k * kC + c] = w[c * 5 + k];
-      CK(cudaMemcpy(h->wf_t, wt.data(), sizeof(float) * 5 * kC, cudaMemcpyHostToDevice));
-    } else if (name == "fusion_layer.bias") r = copy_to(h->bf, t, kC);
-    else if (name == "Spatial_pos_embed") r = copy_to(h->spos, t, static_cast<int64_t>(h->J) * kC);
-    else if (name == "Temporal_pos_embed") r = copy_to(h->tpos, t, static_cast<int64_t>(h->F) * kC);
-    else if (name == "Spatial_norm.weight") r = copy_to(h->sn_g, t, kC);
-    else if (name == "Spatial_norm.bias") r = copy_to(h->sn_b, t, kC);
-    else if (name == "Temporal_norm.weight") r = copy_to(h->tn_g, t, kC);
-    else if (name == "Temporal_norm.bias") r = copy_to(h->tn_b, t, kC);
-    else if (name == "head.0.weight") r = copy_to(h->hg, t, kC);
-    else if (name == "head.0.bias") r = copy_to(h->hb, t, kC);
-    else if (name == "head.1.weight") r = copy_to(h->wh, t, 3 * kC);
+    if (name == "fusion_layer.weight") {           // [C,5] -> transposed [5][C]
+      std::vector<float> w(5 * h->C), wt(5 * h->C);
+      if (t.numel != 5 * h->C) return fail(h, -10, "fusion_layer.weight must be [" + std::to_string(h->C) + ",5]");
+      CK(cudaMemcpy(w.data(), t.data, sizeof(float) * 5 * h->C, t.on_device ? cudaMemcpyDeviceToHost : cudaMemcpyHostToHost));
+      for (int c = 0; c < h->C; ++c)
+        for (int k = 0; k < 5; ++k) wt[k * h->C + c] = w[c * 5 + k];
+      CK(cudaMemcpy(h->wf_t, wt.data(), sizeof(float) * 5 * h->C, cudaMemcpyHostToDevice));
+    } else if (name == "fusion_layer.bias") r = copy_to(h->bf, t, h->C);
+    else if (name == "Spatial_pos_embed") r = copy_to(h->spos, t, static_cast<int64_t>(h->J) * h->C);
+    else if (name == "Temporal_pos_embed") r = copy_to(h->tpos, t, static_cast<int64_t>(h->F) * h->C);
+    else if (name == "Spatial_norm.weight") r = copy_to(h->sn_g, t, h->C);
+    else if (name == "Spatial_norm.bias") r = copy_to(h->sn_b, t, h->C);
+    else if (name == "Temporal_norm.weight") r = copy_to(h->tn_g, t, h->C);
+    else if (name == "Temporal_norm.bias") r = copy_to(h->tn_b, t, h->C);
+    else if (name == "head.0.weight") r = copy_to(h->hg, t, h->C);
+    else if (name == "head.0.bias") r = copy_to(h->hb, t, h->C);
+    else if (name == "head.1.weight") r = copy_to(h->wh, t, 3 * h->C);
     else if (name == "head.1.bias") r = copy_to(h->bh, t, 3);
-    else if (name == "time_mlp.1.weight") r = copy_to(h->tm1w, t, static_cast<int64_t>(2 * kC) * kC);
-    else if (name == "time_mlp.1.bias") r = copy_to(h->tm1b, t, 2 * kC);
-    else if (name == "time_mlp.3.weight") r = copy_to(h->tm3w, t, static_cast<int64_t>(2 * kC) * 2 * kC);
-    else if (name == "time_mlp.3.bias") r = copy_to(h->tm3b, t, 2 * kC);
+    else if (name == "time_mlp.1.weight") r = copy_to(h->tm1w, t, static_cast<int64_t>(2 * h->C) * h->C);
+    else if (name == "time_mlp.1.bias") r = copy_to(h->tm1b, t, 2 * h->C);
+    else if (name == "time_mlp.3.weight") r = copy_to(h->tm3w, t, static_cast<int64_t>(2 * h->C) * 2 * h->C);
+    else if (name == "time_mlp.3.bias") r = copy_to(h->tm3b, t, 2 * h->C);
     else if (name.rfind("STEblocks.", 0) == 0 || name.rfind("TTEblocks.", 0) == 0) {
       const bool spatial = name[0] == 'S';
       const size_t dot = name.find('.', 10);
@@ -725,20 +752,20 @@ int d3d_load_weights(d3d_handle* h, const d3d_tensor* tensors, int32_t n) {
       if (idx < 0 || idx >= h->cfg.depth) return fail(h, -11, "block index out of range in '" + name + "'");
       Blk& b = h->blk[2 * idx + (spatial ? 0 : 1)];
       const std::string sub = name.substr(dot + 1);
-      if (sub == "norm1.weight") r = copy_to(b.n1g, t, kC);
-      else if (sub == "norm1.bias") r = copy_to(b.n1b, t, kC);
-      else if (sub == "norm2.weight") r = copy_to(b.n2g, t, kC);
-      else if (sub == "norm2.bias") r = copy_to(b.n2b, t, kC);
+      if (sub == "norm1.weight") r = copy_to(b.n1g, t, h->C);
+      else if (sub == "norm1.bias") r = copy_to(b.n1b, t, h->C);
+      else if (sub == "norm2.weight") r = copy_to(b.n2g, t, h->C);
+      else if (sub == "norm2.bias") r = copy_to(b.n2b, t, h->C);
       else if (sub == "attn.qkv.weight") r = load_lin_w(b.qkv, t);
-      else if (sub == "attn.qkv.bias") r = copy_to(b.qkv.bias, t, 3 * kC);
+      else if (sub == "attn.qkv.bias") r = copy_to(b.qkv.bias, t, 3 * h->C);
       else if (sub == "attn.proj.weight") r = load_lin_w(b.proj, t);
-      else if (sub == "attn.proj.bias") r = copy_to(b.proj.bias, t, kC);
+      else if (sub == "attn.proj.bias") r = copy_to(b.proj.bias, t, h->C);
       else if (sub == "mlp.fc1.weight") r = load_lin_w(b.fc1, t);
-      else if (sub == "mlp.fc1.bias") r = copy_to(b.fc1.bias, t, kHidden);
+      else if (sub == "mlp.fc1.bias") r = copy_to(b.fc1.bias, t, h->hidden);
       else if (sub == "mlp.fc2.weight") r = load_lin_w(b.fc2, t);
-      else if (sub == "mlp.fc2.bias") r = copy_to(b.fc2.bias, t, kC);
-      else if (sub == "time_mlp.1.weight") r = copy_to(b.tw, t, static_cast<int64_t>(kC) * 2 * kC);
-      else if (sub == "time_mlp.1.bias") r = copy_to(b.tb, t, kC);
+      else if (sub == "mlp.fc2.bias") r = copy_to(b.fc2.bias, t, h->C);
+      else if (sub == "time_mlp.1.weight") r = copy_to(b.tw, t, static_cast<int64_t>(h->C) * 2 * h->C);
+      else if (sub == "time_mlp.1.bias") r = copy_to(b.tb, t, h->C);
       else return fail(h, -11, "unknown tensor '" + name + "'");
     } else {
       return fail(h, -11, "unknown tensor '" + name + "'");
@@ -792,7 +819,7 @@ int d3d_set_schedule(d3d_handle* h, int32_t S, const int32_t* times, const float
   }
   if (S > h->tv_cap) {
     CK(cudaDeviceSynchronize());     // the old table may still be read by in-flight work
-    int r = dev_alloc(h, &h->tv_steps, static_cast<int64_t>(S) * h->nblk * kC);
+    int r = dev_alloc(h, &h->tv_steps, static_cast<int64_t>(S) * h->nblk * h->C);
     if (r) return r;
     h->tv_cap = S;
   }
@@ -817,7 +844,7 @@ int d3d_forward_denoise(d3d_handle* h, const float* x5, const int64_t* t_dev, fl
     if ((r = general_time_table(h, t_dev, B, st))) return r;
     tv = h->tv_general;
   }
-  if ((r = run_blocks(h, nullptr, nullptr, x5, tv, static_cast<int64_t>(h->nblk) * kC, B, h->nblk, st))) return r;
+  if ((r = run_blocks(h, nullptr, nullptr, x5, tv, static_cast<int64_t>(h->nblk) * h->C, B, h->nblk, st))) return r;
   DdimStep s{};
   return run_head(h, s, nullptr, nullptr, out3, nullptr, nullptr, 0, B, st);
 }
@@ -836,9 +863,9 @@ int d3d_debug_forward_blocks(d3d_handle* h, const float* x5, const int64_t* t_de
     if ((r = general_time_table(h, t_dev, B, st))) return r;
     tv = h->tv_general;
   }
-  if ((r = run_blocks(h, nullptr, nullptr, x5, tv, static_cast<int64_t>(h->nblk) * kC, B, n_blocks, st))) return r;
+  if ((r = run_blocks(h, nullptr, nullptr, x5, tv, static_cast<int64_t>(h->nblk) * h->C, B, n_blocks, st))) return r;
   const int64_t T = static_cast<int64_t>(B) * h->F * h->J;
-  CK(cudaMemcpyAsync(x_out, h->X, sizeof(float) * T * kC, cudaMemcpyDeviceToDevice, st));
+  CK(cudaMemcpyAsync(x_out, h->X, sizeof(float) * T * h->C, cudaMemcpyDeviceToDevice, st));
   return 0;
 }
 
@@ -1064,7 +1091,7 @@ int d3d_op_layernorm(d3d_handle* h, const float* x, const float* gamma, const fl
                      int64_t rows, void* stream) {
   if (!h || !x || !gamma || !beta || !out) return -1;
   DeviceGuard guard(h->cfg.device);
-  KL(launch_ln_f32(x, LnParams{gamma, beta}, eps, out, rows, static_cast<cudaStream_t>(stream)));
+  KL(launch_ln_f32(h->C, x, LnParams{gamma, beta}, eps, out, rows, static_cast<cudaStream_t>(stream)));
   return 0;
 }
 
@@ -1076,20 +1103,20 @@ int d3d_op_attention(d3d_handle* h, const float* qkv, float* out, int32_t B, int
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // the hot path receives q | k | v_hi | v_lo fp16 rows from the qkv GEMM epilogue; here they are packed from fp32
   { int r0 = prep_batch(h, B, st); if (r0) return r0; }
-  KL(launch_pack_qkv16(qkv, h->QKV, static_cast<int64_t>(B) * h->F * h->J, st));
+  KL(launch_pack_qkv16(h->C, qkv, h->QKV, static_cast<int64_t>(B) * h->F * h->J, st));
   return run_attention(h, h->QKV, nullptr, nullptr, out, B, spatial != 0, attn_mode, st);
 }
 
-// rows [0, T) of a [tok_cap, 512] workspace operand -> raw arrays (layout: include/diff3d_b200.h,
+// rows [0, T) of a [tok_cap, C] workspace operand -> raw arrays (layout: include/diff3d_b200.h,
 // d3d_debug_attention_operand)
 static int copy_operand_out(d3d_handle* h, const OperandBuf& o, int64_t T, void* hi_out, void* second_out, cudaStream_t st) {
-  CK(cudaMemcpyAsync(hi_out, o.hi, static_cast<size_t>(T) * kC * 2, cudaMemcpyDeviceToDevice, st));
+  CK(cudaMemcpyAsync(hi_out, o.hi, static_cast<size_t>(T) * h->C * 2, cudaMemcpyDeviceToDevice, st));
   if (h->fmt == FMT_F4C) {
-    // second_out: [T][512] c4 bytes (256 B of P nibbles | 256 B of Q nibbles), then [T][32] scale bytes, row-major
-    CK(cudaMemcpyAsync(second_out, o.lo, static_cast<size_t>(T) * kC, cudaMemcpyDeviceToDevice, st));
-    KL(launch_sf_rows(o.sf, static_cast<uint8_t*>(second_out) + static_cast<size_t>(T) * kC, T, kC, st));
+    // second_out: [T][C] c4 bytes (C / 2 B of P nibbles | C / 2 B of Q nibbles), then [T][C / 16] scale bytes, row-major
+    CK(cudaMemcpyAsync(second_out, o.lo, static_cast<size_t>(T) * h->C, cudaMemcpyDeviceToDevice, st));
+    KL(launch_sf_rows(o.sf, static_cast<uint8_t*>(second_out) + static_cast<size_t>(T) * h->C, T, h->C, st));
   } else {
-    CK(cudaMemcpyAsync(second_out, o.lo, static_cast<size_t>(T) * kC * 2, cudaMemcpyDeviceToDevice, st));
+    CK(cudaMemcpyAsync(second_out, o.lo, static_cast<size_t>(T) * h->C * 2, cudaMemcpyDeviceToDevice, st));
   }
   return 0;
 }
@@ -1102,7 +1129,7 @@ int d3d_debug_attention_operand(d3d_handle* h, const float* qkv, void* hi_out, v
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int64_t T = static_cast<int64_t>(B) * h->F * h->J;
   { int r0 = prep_batch(h, B, st); if (r0) return r0; }
-  KL(launch_pack_qkv16(qkv, h->QKV, T, st));
+  KL(launch_pack_qkv16(h->C, qkv, h->QKV, T, st));
   int r = run_attention(h, h->QKV, h->ATT.hi, h->ATT.lo, nullptr, B, spatial != 0, attn_mode, st);
   if (r) return r;
   return copy_operand_out(h, h->ATT, T, hi_out, second_out, st);
@@ -1122,21 +1149,21 @@ int d3d_debug_rowwise(d3d_handle* h, int32_t op, int32_t block, const float* in,
   DeviceGuard guard(h->cfg.device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int64_t T = static_cast<int64_t>(B) * h->F * h->J;
-  const size_t x_bytes = static_cast<size_t>(T) * kC * sizeof(float);
+  const size_t x_bytes = static_cast<size_t>(T) * h->C * sizeof(float);
   const float* tv = nullptr;
   int64_t tv_stride = 0;
   if (timed && h->cfg.with_time_emb) {
     if ((r = general_time_table(h, t_dev, B, st))) return r;
     tv = h->tv_general;
-    tv_stride = shared_t ? 0 : static_cast<int64_t>(h->nblk) * kC;
+    tv_stride = shared_t ? 0 : static_cast<int64_t>(h->nblk) * h->C;
   }
   if (operand) {
     // rows the launch does not write come back as NaN halves / 0xff bytes; the scale atoms (which interleave the
     // padding rows of the last tile) get byte 1, a scale of 2^-126 that no LayerNorm block produces
-    CK(cudaMemsetAsync(h->A.hi, 0xff, static_cast<size_t>(T) * kC * 2, st));
-    CK(cudaMemsetAsync(h->A.lo, 0xff, static_cast<size_t>(T) * (h->fmt == FMT_F4C ? kC : 2 * kC), st));
+    CK(cudaMemsetAsync(h->A.hi, 0xff, static_cast<size_t>(T) * h->C * 2, st));
+    CK(cudaMemsetAsync(h->A.lo, 0xff, static_cast<size_t>(T) * (h->fmt == FMT_F4C ? h->C : 2 * h->C), st));
     if (h->fmt == FMT_F4C)
-      CK(cudaMemsetAsync(h->A.sf, 1, static_cast<size_t>((T + 127) / 128) * 128 * (kC / 16), st));
+      CK(cudaMemsetAsync(h->A.sf, 1, static_cast<size_t>((T + 127) / 128) * 128 * (h->C / 16), st));
   }
   if (op == D3D_ROWWISE_LIFT) {
     CK(cudaMemsetAsync(h->X, 0xff, x_bytes, st));

@@ -7,6 +7,9 @@
 namespace d3d {
 namespace {
 
+// CUDA-core validation GEMM: its packed q|k|v epilogue is built for C = 512 only
+constexpr int kC = Width<512>::kC, kQkvRow = Width<512>::kQkvRow;
+
 constexpr int TM = 64, TN = 64, TK = 16;
 
 __device__ __forceinline__ float gelu_erf(float v) { return 0.5f * v * (1.0f + erff(v * 0.70710678118654752440f)); }

@@ -803,8 +803,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constan
           size_t ld;
           if (EPI == EPI_GELU_SPLIT) {
             hi_base = p.out_hi + gcol; lo_base = p.out_lo + gcol; ld = static_cast<size_t>(p.N);
-          } else {                   // EPI_QKV16: q | k -> fp16; v -> hi at the same column, lo 512 columns further
-            hi_base = p.out_qkv + gcol; lo_base = gcol >= 2 * kC ? p.out_qkv + gcol + kC : nullptr; ld = kQkvRow;
+          } else {                   // EPI_QKV16(_256): q | k -> fp16; v -> hi at the same column, lo C columns further
+            constexpr int kQc = qkv_epi_width(EPI);
+            hi_base = p.out_qkv + gcol; lo_base = gcol >= 2 * kQc ? p.out_qkv + gcol + kQc : nullptr; ld = Width<kQc>::kQkvRow;
           }
           if (EPI == EPI_GELU_SPLIT && PASSES == 2) {
             // c8 row of the fc2 operand: N bytes e5m2(x 2^-8) then N bytes e5m2(lo 2^4); 32 columns = 2 granules each
@@ -970,6 +971,8 @@ cudaError_t configure_gemm_tc() {
   if ((e = configure_one<2, 256, 4, EPI_F32, 1, 16>()) != cudaSuccess) return e;
   if ((e = configure_one<2, 256, 4, EPI_GELU_SPLIT, 1, 16>()) != cudaSuccess) return e;
   if ((e = configure_one<2, 256, 4, EPI_QKV16, 1, 16>()) != cudaSuccess) return e;
+  if ((e = configure_one<2, 256, 4, EPI_QKV16_256>()) != cudaSuccess) return e;
+  if ((e = configure_one<2, 256, 4, EPI_QKV16_256, 1, 16>()) != cudaSuccess) return e;
   if ((e = configure_one<2, 256, 4, EPI_F32_RED>()) != cudaSuccess) return e;
   return cudaSuccess;
 }
@@ -980,17 +983,21 @@ cudaError_t launch_gemm_tc(const GemmMaps& maps, const GemmParams& p, int epi, i
   if (passes == 4) {
     // FMT_F4C: CTA-pair 256 x 256 tiles only; K in whole e2m1 stages (256 nibbles = 128 bytes of the K-byte c4 row)
     if (p.N % 256 != 0 || p.K % 128 != 0) return cudaErrorInvalidValue;
-    if (epi == EPI_QKV16 && p.N != 3 * kC) return cudaErrorInvalidValue;
+    // the packed q|k|v epilogue of either width: N = 3 C
+    if (epi == EPI_QKV16 && p.N == 3 * 256) epi = EPI_QKV16_256;
+    else if (epi == EPI_QKV16 && p.N != 3 * 512) return cudaErrorInvalidValue;
     if (epi == EPI_GELU_SPLIT && (!p.out_sf || p.N > 1024)) return cudaErrorInvalidValue;
     if (epi == EPI_F32_RED && (!p.out_f32 || epi_warps == 16)) return cudaErrorInvalidValue;
     if (epi_warps == 16) {
       if (epi == EPI_F32) return launch_one<2, 256, 4, EPI_F32, 1, 16>(maps, p, num_sms, st);
       if (epi == EPI_GELU_SPLIT) return launch_one<2, 256, 4, EPI_GELU_SPLIT, 1, 16>(maps, p, num_sms, st);
+      if (epi == EPI_QKV16_256) return launch_one<2, 256, 4, EPI_QKV16_256, 1, 16>(maps, p, num_sms, st);
       return launch_one<2, 256, 4, EPI_QKV16, 1, 16>(maps, p, num_sms, st);
     }
     if (epi == EPI_F32) return launch_one<2, 256, 4, EPI_F32>(maps, p, num_sms, st);
     if (epi == EPI_F32_RED) return launch_one<2, 256, 4, EPI_F32_RED>(maps, p, num_sms, st);
     if (epi == EPI_GELU_SPLIT) return launch_one<2, 256, 4, EPI_GELU_SPLIT>(maps, p, num_sms, st);
+    if (epi == EPI_QKV16_256) return launch_one<2, 256, 4, EPI_QKV16_256>(maps, p, num_sms, st);
     return launch_one<2, 256, 4, EPI_QKV16>(maps, p, num_sms, st);
   }
   if (epi == EPI_F32_RED) return cudaErrorInvalidValue;     // FMT_F4C kernel only
@@ -1001,7 +1008,7 @@ cudaError_t launch_gemm_tc(const GemmMaps& maps, const GemmParams& p, int epi, i
     if (epi == EPI_QKV16) return launch_one<2, 256, 2, EPI_QKV16, 1, 16>(maps, p, num_sms, st);
   }
   if (p.K % BK != 0 || p.N % bn != 0 || (bn != 128 && bn != 256)) return cudaErrorInvalidValue;
-  if (epi == EPI_QKV16 && p.N != 3 * kC) return cudaErrorInvalidValue;
+  if (epi == EPI_QKV16 && p.N != 3 * 512) return cudaErrorInvalidValue;     // the validation modes: C = 512 only
   if (pair_cluster == 2 && cta_group == 2 && passes == 2) {
     if (epi == EPI_F32) return launch_one<2, 256, 2, EPI_F32, 2>(maps, p, num_sms, st);
     if (epi == EPI_GELU_SPLIT) return launch_one<2, 256, 2, EPI_GELU_SPLIT, 2>(maps, p, num_sms, st);

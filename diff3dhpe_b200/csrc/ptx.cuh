@@ -412,6 +412,17 @@ __device__ __forceinline__ uint64_t make_desc_k_sw128(uint32_t smem_addr) {
   d |= static_cast<uint64_t>(2) << 61;
   return d;
 }
+// The same for 64-byte (32 fp16) rows in the 64-byte swizzle (a SWIZZLE_64B TMA box of {32, rows}): 8 rows x 64 B = 512 B
+// between 8-row groups, layout type = 4 (SWIZZLE_64B)
+__device__ __forceinline__ uint64_t make_desc_k_sw64(uint32_t smem_addr) {
+  uint64_t d = 0;
+  d |= static_cast<uint64_t>((smem_addr & 0x3ffffu) >> 4);
+  d |= static_cast<uint64_t>(1) << 16;
+  d |= static_cast<uint64_t>(512 >> 4) << 32;
+  d |= static_cast<uint64_t>(1) << 46;
+  d |= static_cast<uint64_t>(4) << 61;
+  return d;
+}
 
 // Shared-memory descriptor of a tcgen05.cp.32x128b source: 32 rows x 16 bytes stored contiguously (row r at 16 r), i.e.
 // four 8-row x 16-byte core matrices 128 bytes apart, K-major, no swizzle: SBO = 128 B, LBO unused (one core matrix

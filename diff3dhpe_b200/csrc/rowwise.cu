@@ -1,10 +1,11 @@
-// Row-wise (memory-bound) kernels: one warp owns one 512-wide token row, lane l holds columns
-// {128*i + 4*l .. +3 : i = 0..3} so every global access is a fully coalesced 128-bit transaction.
+// Row-wise (memory-bound) kernels: one warp owns one C-wide token row (C = 512 or 256, a template parameter), lane l holds
+// columns {128*i + 4*l .. +3 : i < C / 128} -- N = C / 32 values per lane -- so every global access is a fully coalesced
+// 128-bit transaction.
 //
 //   lift_ln            G-lift : fusion_layer (K=5) + Spatial_pos_embed + block-0 time vector + norm1   (MODEL:250,230-233,113-116,127)
 //   postnorm_add_ln    G-ln   : Spatial_/Temporal_norm + Temporal_pos_embed + next block's time vector + next norm1
 //   ln_split           G-ln   : norm2 -> split fp16 A operand of fc1                                  (MODEL:128)
-//   head_ddim          G-head+ddim : Temporal_norm + head LayerNorm(1e-5) + Linear(512->3) + clamp + DDIM update
+//   head_ddim          G-head+ddim : Temporal_norm + head LayerNorm(1e-5) + Linear(C->3) + clamp + DDIM update
 //                                                                                  (MODEL:245,255; DIFF:256,283-297)
 //   tta_merge, mpjpe   G-tta  : RUN:583-588, LOSS:15-27
 #include <cstdlib>
@@ -28,46 +29,52 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
-__device__ __forceinline__ void load_row(const float* __restrict__ p, int lane, float (&v)[16]) {
+template <int N>
+__device__ __forceinline__ void load_row(const float* __restrict__ p, int lane, float (&v)[N]) {
 #pragma unroll
-  for (int i = 0; i < 4; ++i) {
+  for (int i = 0; i < N / 4; ++i) {
     const float4 t = *reinterpret_cast<const float4*>(p + 128 * i + 4 * lane);
     v[4 * i + 0] = t.x; v[4 * i + 1] = t.y; v[4 * i + 2] = t.z; v[4 * i + 3] = t.w;
   }
 }
-__device__ __forceinline__ void load_row_ldg(const float* __restrict__ p, int lane, float (&v)[16]) {
+template <int N>
+__device__ __forceinline__ void load_row_ldg(const float* __restrict__ p, int lane, float (&v)[N]) {
 #pragma unroll
-  for (int i = 0; i < 4; ++i) {
+  for (int i = 0; i < N / 4; ++i) {
     const float4 t = __ldg(reinterpret_cast<const float4*>(p + 128 * i + 4 * lane));
     v[4 * i + 0] = t.x; v[4 * i + 1] = t.y; v[4 * i + 2] = t.z; v[4 * i + 3] = t.w;
   }
 }
-__device__ __forceinline__ void store_row(float* __restrict__ p, int lane, const float (&v)[16]) {
+template <int N>
+__device__ __forceinline__ void store_row(float* __restrict__ p, int lane, const float (&v)[N]) {
 #pragma unroll
-  for (int i = 0; i < 4; ++i)
+  for (int i = 0; i < N / 4; ++i)
     *reinterpret_cast<float4*>(p + 128 * i + 4 * lane) = make_float4(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
 }
-// a += b  /  a += s * b  over the lane's 16 columns, as 8 packed pairs
-__device__ __forceinline__ void add16(float (&a)[16], const float (&b)[16]) {
+// a += b  /  a += s * b  over the lane's N columns, as N / 2 packed pairs
+template <int N>
+__device__ __forceinline__ void add16(float (&a)[N], const float (&b)[N]) {
 #pragma unroll
-  for (int i = 0; i < 8; ++i)
+  for (int i = 0; i < N / 2; ++i)
     ptx::unpack2(ptx::add2(ptx::pack2(a[2 * i], a[2 * i + 1]), ptx::pack2(b[2 * i], b[2 * i + 1])), a[2 * i], a[2 * i + 1]);
 }
-__device__ __forceinline__ void fma16(float (&a)[16], float s, const float (&b)[16]) {
+template <int N>
+__device__ __forceinline__ void fma16(float (&a)[N], float s, const float (&b)[N]) {
   const ptx::f32x2 s2 = ptx::splat2(s);
 #pragma unroll
-  for (int i = 0; i < 8; ++i)
+  for (int i = 0; i < N / 2; ++i)
     ptx::unpack2(ptx::fma2(s2, ptx::pack2(b[2 * i], b[2 * i + 1]), ptx::pack2(a[2 * i], a[2 * i + 1])), a[2 * i], a[2 * i + 1]);
 }
 
-// GEMM A operand of token row `row` (K = 512) in the handle's operand format (operand.cuh); `second` / `sf` are the BASE
-// pointers of the operand's second array and (FMT_F4C) its scale-factor array.
-template <int FMT>
+// GEMM A operand of token row `row` (K = C = 32 N) in the handle's operand format (operand.cuh); `second` / `sf` are the
+// BASE pointers of the operand's second array and (FMT_F4C) its scale-factor array.
+template <int FMT, int N>
 __device__ __forceinline__ void store_operand(__half* __restrict__ hi, __half* __restrict__ second,
-                                              uint8_t* __restrict__ sf, int64_t row, int lane, const float (&v)[16]) {
+                                              uint8_t* __restrict__ sf, int64_t row, int lane, const float (&v)[N]) {
+  constexpr int kC = 32 * N;
   if (FMT != FMT_F4C) {
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
+    for (int i = 0; i < N / 4; ++i) {
       const float x[4] = {v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]};
       op_store4<FMT>(hi + row * kC, second + row * kC, kC, 128 * i + 4 * lane, x);
     }
@@ -75,13 +82,13 @@ __device__ __forceinline__ void store_operand(__half* __restrict__ hi, __half* _
   }
   // FMT_F4C: the lane's 4 columns of chunk i belong to the 32-column block (4 i + lane / 8).  The scale byte is a
   // monotone function of the block maximum, so the 8 lanes of a block reduce the two BYTES (P: q4(x), k-blocks 0..15;
-  // Q: q4(x - hi), k-blocks 16..31) packed in one register with three shuffles + packed-halfword maxima.
+  // Q: q4(x - hi), k-blocks C/32 .. C/16 - 1) packed in one register with three shuffles + packed-halfword maxima.
   uint8_t* c4 = reinterpret_cast<uint8_t*>(second) + row * kC;
   __half* hrow = hi + row * kC;
-  // scale bytes of (row, k-block 4 i + g) sit at sf_row + 512 i + g (P) and sf_row + 512 (4 + i) + g (Q)
+  // scale bytes of (row, k-block 4 i + g) sit at sf_row + 512 i + g (P) and sf_row + 512 (C / 128 + i) + g (Q)
   uint8_t* sf_row = sf + (static_cast<size_t>(row >> 7) * (kC / 64)) * 512 + 16 * (row & 31) + 4 * ((row & 127) >> 5) + (lane >> 3);
 #pragma unroll
-  for (int i = 0; i < 4; ++i) {
+  for (int i = 0; i < N / 4; ++i) {
     float x[4], l[4];
     const __half2 h01 = __floats2half2_rn(v[4 * i], v[4 * i + 1]), h23 = __floats2half2_rn(v[4 * i + 2], v[4 * i + 3]);
     const float2 f01 = __half22float2(h01), f23 = __half22float2(h23);
@@ -108,25 +115,27 @@ __device__ __forceinline__ void store_operand(__half* __restrict__ hi, __half* _
         static_cast<uint16_t>(op_e2m1x2(l[0], l[1]) | (op_e2m1x2(l[2], l[3]) << 8));
     if ((lane & 7) == 0) {       // lanes 0, 8, 16, 24: four adjacent bytes of one scale-factor atom
       sf_row[512 * i] = static_cast<uint8_t>(bp);
-      sf_row[512 * (4 + i)] = static_cast<uint8_t>(bq);
+      sf_row[512 * (N / 4 + i)] = static_cast<uint8_t>(bq);
     }
   }
 }
 
-// y = (x - mean) * rstd * gamma + beta over 512 columns held by the warp (two-pass variance in registers).  The
+// y = (x - mean) * rstd * gamma + beta over the C columns held by the warp (two-pass variance in registers).  The
 // element-wise work runs on packed fp32 pairs (FADD2 / FFMA2 / FMUL2: two IEEE-rn operations per issue slot): with the
 // block-scaled operand format these kernels are bound by instruction issue, not by HBM.
-__device__ __forceinline__ float ln_center(const float (&x)[16], ptx::f32x2 (&xp)[8]);
+template <int N>
+__device__ __forceinline__ float ln_center(const float (&x)[N], ptx::f32x2 (&xp)[N / 2]);
 __device__ __forceinline__ ptx::f32x2 ln_rstd(float var, float eps);
-__device__ __forceinline__ void layernorm_row(const float (&x)[16], const float* __restrict__ gamma,
-                                              const float* __restrict__ beta, float eps, int lane, float (&y)[16]) {
-  ptx::f32x2 xp[8];
+template <int N>
+__device__ __forceinline__ void layernorm_row(const float (&x)[N], const float* __restrict__ gamma,
+                                              const float* __restrict__ beta, float eps, int lane, float (&y)[N]) {
+  ptx::f32x2 xp[N / 2];
   const float var = ln_center(x, xp);
   // 1 / sqrt(var + eps): MUFU.RSQ + one Newton step (< 1 ulp) -- the IEEE sqrt + division pair cost ~25 instructions with
   // its slow-path calls (ln_rstd)
   const ptx::f32x2 rstd = ln_rstd(var, eps);
 #pragma unroll
-  for (int i = 0; i < 4; ++i) {
+  for (int i = 0; i < N / 4; ++i) {
     const float4 g = __ldg(reinterpret_cast<const float4*>(gamma + 128 * i + 4 * lane));
     const float4 b = __ldg(reinterpret_cast<const float4*>(beta + 128 * i + 4 * lane));
     ptx::unpack2(ptx::fma2(ptx::mul2(xp[2 * i], rstd), ptx::pack2(g.x, g.y), ptx::pack2(b.x, b.y)), y[4 * i], y[4 * i + 1]);
@@ -138,18 +147,25 @@ __device__ __forceinline__ void layernorm_row(const float (&x)[16], const float*
 // one-row kernels (profiles/r02n_full_*.md, r02f_full_postnorm_add_ln.md): l1tex throughput 77-95 % -- each row re-read
 // 2 KB per parameter vector through L1 (24 of postnorm's 36 memory instructions), and at the step's power-capped clock
 // that, not HBM, set their time.  Per-row arithmetic is identical to layernorm_row (results do not depend on the partner).
-__device__ __forceinline__ float ln_center(const float (&x)[16], ptx::f32x2 (&xp)[8]) {      // xp = x - mean; returns var
+template <int N>
+__device__ __forceinline__ float ln_center(const float (&x)[N], ptx::f32x2 (&xp)[N / 2]) {      // xp = x - mean; returns var
+  static_assert(N == 8 || N == 16, "C = 256 or 512");
+  constexpr int kC = 32 * N;
 #pragma unroll
-  for (int i = 0; i < 8; ++i) xp[i] = ptx::pack2(x[2 * i], x[2 * i + 1]);
-  ptx::f32x2 sp = ptx::add2(ptx::add2(ptx::add2(xp[0], xp[1]), ptx::add2(xp[2], xp[3])),
-                            ptx::add2(ptx::add2(xp[4], xp[5]), ptx::add2(xp[6], xp[7])));
+  for (int i = 0; i < N / 2; ++i) xp[i] = ptx::pack2(x[2 * i], x[2 * i + 1]);
+  ptx::f32x2 sp;
+  if constexpr (N == 16)
+    sp = ptx::add2(ptx::add2(ptx::add2(xp[0], xp[1]), ptx::add2(xp[2], xp[3])),
+                   ptx::add2(ptx::add2(xp[4], xp[5]), ptx::add2(xp[6], xp[7])));
+  else
+    sp = ptx::add2(ptx::add2(xp[0], xp[1]), ptx::add2(xp[2], xp[3]));
   float s0, s1;
   ptx::unpack2(sp, s0, s1);
   const float mean = warp_sum(s0 + s1) * (1.0f / kC);
   const ptx::f32x2 nm = ptx::splat2(-mean);
   ptx::f32x2 qp = ptx::splat2(0.f);
 #pragma unroll
-  for (int i = 0; i < 8; ++i) {
+  for (int i = 0; i < N / 2; ++i) {
     xp[i] = ptx::add2(xp[i], nm);
     qp = ptx::fma2(xp[i], xp[i], qp);
   }
@@ -162,15 +178,16 @@ __device__ __forceinline__ ptx::f32x2 ln_rstd(float var, float eps) {
   asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(r0) : "f"(ve));
   return ptx::splat2(r0 * fmaf(-0.5f * ve, r0 * r0, 1.5f));
 }
-// y_r = LN(x_r) (+ add) for r = 0, 1; `add` (optional, a 512-vector common to both rows) is added after beta
-__device__ __forceinline__ void layernorm_2rows(const float (&x0)[16], const float (&x1)[16], const float* __restrict__ gamma,
+// y_r = LN(x_r) (+ add) for r = 0, 1; `add` (optional, a C-vector common to both rows) is added after beta
+template <int N>
+__device__ __forceinline__ void layernorm_2rows(const float (&x0)[N], const float (&x1)[N], const float* __restrict__ gamma,
                                                 const float* __restrict__ beta, const float* __restrict__ add, float eps,
-                                                int lane, float (&y0)[16], float (&y1)[16]) {
-  ptx::f32x2 p0[8], p1[8];
+                                                int lane, float (&y0)[N], float (&y1)[N]) {
+  ptx::f32x2 p0[N / 2], p1[N / 2];
   const float v0 = ln_center(x0, p0), v1 = ln_center(x1, p1);
   const ptx::f32x2 r0 = ln_rstd(v0, eps), r1 = ln_rstd(v1, eps);
 #pragma unroll
-  for (int i = 0; i < 4; ++i) {
+  for (int i = 0; i < N / 4; ++i) {
     const float4 g = __ldg(reinterpret_cast<const float4*>(gamma + 128 * i + 4 * lane));
     const float4 b = __ldg(reinterpret_cast<const float4*>(beta + 128 * i + 4 * lane));
     const ptx::f32x2 g01 = ptx::pack2(g.x, g.y), g23 = ptx::pack2(g.z, g.w), b01 = ptx::pack2(b.x, b.y), b23 = ptx::pack2(b.z, b.w);
@@ -189,7 +206,7 @@ __device__ __forceinline__ void layernorm_2rows(const float (&x0)[16], const flo
   }
 }
 
-template <int FMT>
+template <int C, int FMT>
 __global__ void __launch_bounds__(kWarpsPerCta * 32)
 lift_ln_kernel(const float* __restrict__ x2d, const float* __restrict__ y3, const float* __restrict__ x5,
                const float* __restrict__ wf_t, const float* __restrict__ bf, const float* __restrict__ spos,
@@ -207,13 +224,13 @@ lift_ln_kernel(const float* __restrict__ x2d, const float* __restrict__ y3, cons
     in[0] = __ldg(x2d + t * 2); in[1] = __ldg(x2d + t * 2 + 1);
     in[2] = __ldg(y3 + t * 3); in[3] = __ldg(y3 + t * 3 + 1); in[4] = __ldg(y3 + t * 3 + 2);
   }
-  float v[16], w[16];
+  float v[C / 32], w[C / 32];
   // F.linear: sum_k in_k * W[c][k] + b[c]
 #pragma unroll
-  for (int i = 0; i < 16; ++i) v[i] = 0.f;
+  for (int i = 0; i < C / 32; ++i) v[i] = 0.f;
 #pragma unroll
   for (int k = 0; k < 5; ++k) {
-    load_row_ldg(wf_t + k * kC, lane, w);
+    load_row_ldg(wf_t + k * C, lane, w);
     fma16(v, in[k], w);
   }
   load_row_ldg(bf, lane, w);
@@ -221,7 +238,7 @@ lift_ln_kernel(const float* __restrict__ x2d, const float* __restrict__ y3, cons
   // token indices fit 32 bits (launchers check T < 2^31): 32-bit divisions instead of the 64-bit software routine,
   // which cost these issue-bound kernels ~100 instructions per row
   const uint32_t t32 = static_cast<uint32_t>(t);
-  load_row_ldg(spos + static_cast<size_t>(t32 % static_cast<uint32_t>(J)) * kC, lane, w);
+  load_row_ldg(spos + static_cast<size_t>(t32 % static_cast<uint32_t>(J)) * C, lane, w);
   add16(v, w);
   if (tvec) {
     const float* tv = tvec;
@@ -229,15 +246,15 @@ lift_ln_kernel(const float* __restrict__ x2d, const float* __restrict__ y3, cons
     load_row_ldg(tv, lane, w);
     add16(v, w);
   }
-  store_row(X + t * kC, lane, v);
-  float a[16];
+  store_row(X + t * C, lane, v);
+  float a[C / 32];
   layernorm_row(v, ln1.gamma, ln1.beta, 1e-6f, lane, a);
   store_operand<FMT>(a_hi, a_lo, a_sf, t, lane, a);
 }
 
 // lift_ln on two rows per warp: the five fusion_layer weight rows, its bias, the time vector and the norm1 parameters are
 // loaded once for both tokens (only the Spatial_pos_embed row differs); eval only (one time vector for every clip).
-template <int FMT>
+template <int C, int FMT>
 __global__ void __launch_bounds__(kWarpsPerCta * 32, D3D_ROWS2_MIN_CTAS)
 lift_ln2_kernel(const float* __restrict__ x2d, const float* __restrict__ y3, const float* __restrict__ x5,
                 const float* __restrict__ wf_t, const float* __restrict__ bf, const float* __restrict__ spos,
@@ -258,12 +275,12 @@ lift_ln2_kernel(const float* __restrict__ x2d, const float* __restrict__ y3, con
     in1[0] = __ldg(x2d + t1 * 2); in1[1] = __ldg(x2d + t1 * 2 + 1);
     in1[2] = __ldg(y3 + t1 * 3); in1[3] = __ldg(y3 + t1 * 3 + 1); in1[4] = __ldg(y3 + t1 * 3 + 2);
   }
-  float v0[16], v1[16], w[16];
+  float v0[C / 32], v1[C / 32], w[C / 32];
 #pragma unroll
-  for (int i = 0; i < 16; ++i) { v0[i] = 0.f; v1[i] = 0.f; }
+  for (int i = 0; i < C / 32; ++i) { v0[i] = 0.f; v1[i] = 0.f; }
 #pragma unroll
   for (int k = 0; k < 5; ++k) {
-    load_row_ldg(wf_t + k * kC, lane, w);
+    load_row_ldg(wf_t + k * C, lane, w);
     fma16(v0, in0[k], w);
     fma16(v1, in1[k], w);
   }
@@ -272,24 +289,24 @@ lift_ln2_kernel(const float* __restrict__ x2d, const float* __restrict__ y3, con
   add16(v1, w);
   const uint32_t j0 = static_cast<uint32_t>(t) % static_cast<uint32_t>(J);
   const uint32_t j1 = j0 + 1 == static_cast<uint32_t>(J) ? 0u : j0 + 1;
-  load_row_ldg(spos + static_cast<size_t>(j0) * kC, lane, w);
+  load_row_ldg(spos + static_cast<size_t>(j0) * C, lane, w);
   add16(v0, w);
-  load_row_ldg(spos + static_cast<size_t>(j1) * kC, lane, w);
+  load_row_ldg(spos + static_cast<size_t>(j1) * C, lane, w);
   add16(v1, w);
   if (tvec) {
     load_row_ldg(tvec, lane, w);
     add16(v0, w);
     add16(v1, w);
   }
-  store_row(X + t * kC, lane, v0);
-  if (two) store_row(X + (t + 1) * kC, lane, v1);
-  float a0[16], a1[16];
+  store_row(X + t * C, lane, v0);
+  if (two) store_row(X + (t + 1) * C, lane, v1);
+  float a0[C / 32], a1[C / 32];
   layernorm_2rows(v0, v1, ln1.gamma, ln1.beta, nullptr, 1e-6f, lane, a0, a1);
   store_operand<FMT>(a_hi, a_lo, a_sf, t, lane, a0);
   if (two) store_operand<FMT>(a_hi, a_lo, a_sf, t + 1, lane, a1);
 }
 
-template <int FMT>
+template <int C, int FMT>
 __global__ void __launch_bounds__(kWarpsPerCta * 32)
 postnorm_add_ln_kernel(float* __restrict__ X, LnParams post, const float* __restrict__ tpos,
                        const float* __restrict__ tvec, int64_t tvec_stride, LnParams ln1, __half* __restrict__ a_hi,
@@ -297,11 +314,11 @@ postnorm_add_ln_kernel(float* __restrict__ X, LnParams post, const float* __rest
   const int lane = threadIdx.x & 31;
   const int64_t t = static_cast<int64_t>(blockIdx.x) * kWarpsPerCta + (threadIdx.x >> 5);
   if (t >= T) return;
-  float x[16], z[16], w[16];
-  load_row(X + t * kC, lane, x);
+  float x[C / 32], z[C / 32], w[C / 32];
+  load_row(X + t * C, lane, x);
   layernorm_row(x, post.gamma, post.beta, 1e-6f, lane, z);
   if (tpos) {
-    load_row_ldg(tpos + static_cast<size_t>((static_cast<uint32_t>(t) / static_cast<uint32_t>(J)) % static_cast<uint32_t>(F)) * kC, lane, w);
+    load_row_ldg(tpos + static_cast<size_t>((static_cast<uint32_t>(t) / static_cast<uint32_t>(J)) % static_cast<uint32_t>(F)) * C, lane, w);
     add16(z, w);
   }
   if (tvec) {          // eval: every clip shares t (tvec_stride == 0), no clip index needed
@@ -310,27 +327,27 @@ postnorm_add_ln_kernel(float* __restrict__ X, LnParams post, const float* __rest
     load_row_ldg(tv, lane, w);
     add16(z, w);
   }
-  store_row(X + t * kC, lane, z);
+  store_row(X + t * C, lane, z);
   layernorm_row(z, ln1.gamma, ln1.beta, 1e-6f, lane, x);
   store_operand<FMT>(a_hi, a_lo, a_sf, t, lane, x);
 }
 
-template <int FMT>
+template <int C, int FMT>
 __global__ void __launch_bounds__(kWarpsPerCta * 32)
 ln_split_kernel(const float* __restrict__ X, LnParams ln, float eps, __half* __restrict__ a_hi,
                 __half* __restrict__ a_lo, uint8_t* __restrict__ a_sf, int64_t T) {
   const int lane = threadIdx.x & 31;
   const int64_t t = static_cast<int64_t>(blockIdx.x) * kWarpsPerCta + (threadIdx.x >> 5);
   if (t >= T) return;
-  float x[16], y[16];
-  load_row(X + t * kC, lane, x);
+  float x[C / 32], y[C / 32];
+  load_row(X + t * C, lane, x);
   layernorm_row(x, ln.gamma, ln.beta, eps, lane, y);
   store_operand<FMT>(a_hi, a_lo, a_sf, t, lane, y);
 }
 
 // Two rows per warp (rows 2 w, 2 w + 1 of the launch): the production forms of ln_split / postnorm_add_ln when no
 // per-row additive term is needed (eval: one time vector for every clip; Temporal_pos_embed only after block 0).
-template <int FMT>
+template <int C, int FMT>
 __global__ void __launch_bounds__(kWarpsPerCta * 32, D3D_ROWS2_MIN_CTAS)
 ln_split2_kernel(const float* __restrict__ X, LnParams ln, float eps, __half* __restrict__ a_hi, __half* __restrict__ a_lo,
                  uint8_t* __restrict__ a_sf, int64_t T) {
@@ -338,15 +355,15 @@ ln_split2_kernel(const float* __restrict__ X, LnParams ln, float eps, __half* __
   const int64_t t = (static_cast<int64_t>(blockIdx.x) * kWarpsPerCta + (threadIdx.x >> 5)) * 2;
   if (t >= T) return;
   const bool two = t + 1 < T;
-  float x0[16], x1[16], y0[16], y1[16];
-  load_row(X + t * kC, lane, x0);
-  load_row(X + (two ? t + 1 : t) * kC, lane, x1);
+  float x0[C / 32], x1[C / 32], y0[C / 32], y1[C / 32];
+  load_row(X + t * C, lane, x0);
+  load_row(X + (two ? t + 1 : t) * C, lane, x1);
   layernorm_2rows(x0, x1, ln.gamma, ln.beta, nullptr, eps, lane, y0, y1);
   store_operand<FMT>(a_hi, a_lo, a_sf, t, lane, y0);
   if (two) store_operand<FMT>(a_hi, a_lo, a_sf, t + 1, lane, y1);
 }
 
-template <int FMT>
+template <int C, int FMT>
 __global__ void __launch_bounds__(kWarpsPerCta * 32, D3D_ROWS2_MIN_CTAS)
 postnorm_add_ln2_kernel(float* __restrict__ X, LnParams post, const float* __restrict__ tvec, LnParams ln1,
                         __half* __restrict__ a_hi, __half* __restrict__ a_lo, uint8_t* __restrict__ a_sf, int64_t T) {
@@ -354,28 +371,30 @@ postnorm_add_ln2_kernel(float* __restrict__ X, LnParams post, const float* __res
   const int64_t t = (static_cast<int64_t>(blockIdx.x) * kWarpsPerCta + (threadIdx.x >> 5)) * 2;
   if (t >= T) return;
   const bool two = t + 1 < T;
-  float x0[16], x1[16], z0[16], z1[16];
-  load_row(X + t * kC, lane, x0);
-  load_row(X + (two ? t + 1 : t) * kC, lane, x1);
+  float x0[C / 32], x1[C / 32], z0[C / 32], z1[C / 32];
+  load_row(X + t * C, lane, x0);
+  load_row(X + (two ? t + 1 : t) * C, lane, x1);
   layernorm_2rows(x0, x1, post.gamma, post.beta, tvec, 1e-6f, lane, z0, z1);
-  store_row(X + t * kC, lane, z0);
-  if (two) store_row(X + (t + 1) * kC, lane, z1);
+  store_row(X + t * C, lane, z0);
+  if (two) store_row(X + (t + 1) * C, lane, z1);
   layernorm_2rows(z0, z1, ln1.gamma, ln1.beta, nullptr, 1e-6f, lane, x0, x1);
   store_operand<FMT>(a_hi, a_lo, a_sf, t, lane, x0);
   if (two) store_operand<FMT>(a_hi, a_lo, a_sf, t + 1, lane, x1);
 }
 
+template <int C>
 __global__ void __launch_bounds__(kWarpsPerCta * 32)
 ln_f32_kernel(const float* __restrict__ X, LnParams ln, float eps, float* __restrict__ out, int64_t T) {
   const int lane = threadIdx.x & 31;
   const int64_t t = static_cast<int64_t>(blockIdx.x) * kWarpsPerCta + (threadIdx.x >> 5);
   if (t >= T) return;
-  float x[16], y[16];
-  load_row(X + t * kC, lane, x);
+  float x[C / 32], y[C / 32];
+  load_row(X + t * C, lane, x);
   layernorm_row(x, ln.gamma, ln.beta, eps, lane, y);
-  store_row(out + t * kC, lane, y);
+  store_row(out + t * C, lane, y);
 }
 
+template <int C>
 __global__ void __launch_bounds__(kWarpsPerCta * 32)
 head_ddim_kernel(const float* __restrict__ X, LnParams post, LnParams head_ln, const float* __restrict__ wh,
                  const float* __restrict__ bh, DdimStep s, float* __restrict__ y, const float* __restrict__ noise,
@@ -384,17 +403,17 @@ head_ddim_kernel(const float* __restrict__ X, LnParams post, LnParams head_ln, c
   const int lane = threadIdx.x & 31;
   const int64_t t = static_cast<int64_t>(blockIdx.x) * kWarpsPerCta + (threadIdx.x >> 5);
   if (t >= T) return;
-  float x[16], z[16], h[16], w[16];
-  load_row(X + t * kC, lane, x);
+  float x[C / 32], z[C / 32], h[C / 32], w[C / 32];
+  load_row(X + t * C, lane, x);
   layernorm_row(x, post.gamma, post.beta, 1e-6f, lane, z);
   layernorm_row(z, head_ln.gamma, head_ln.beta, 1e-5f, lane, h);
   float o[3];
 #pragma unroll
   for (int k = 0; k < 3; ++k) {
-    load_row_ldg(wh + k * kC, lane, w);
+    load_row_ldg(wh + k * C, lane, w);
     float d = 0.f;
 #pragma unroll
-    for (int i = 0; i < 16; ++i) d = fmaf(h[i], w[i], d);
+    for (int i = 0; i < C / 32; ++i) d = fmaf(h[i], w[i], d);
     o[k] = warp_sum(d) + __ldg(bh + k);
   }
   if (lane < 3) {
@@ -450,6 +469,7 @@ __device__ __forceinline__ void head_finish(float o0, float o1, float o2, int la
   }
 }
 
+template <int C>
 __global__ void __launch_bounds__(kWarpsPerCta * 32, D3D_ROWS2_MIN_CTAS)
 head_ddim2_kernel(const float* __restrict__ X, LnParams post, LnParams head_ln, const float* __restrict__ wh,
                   const float* __restrict__ bh, DdimStep s, float* __restrict__ y, const float* __restrict__ noise,
@@ -459,18 +479,18 @@ head_ddim2_kernel(const float* __restrict__ X, LnParams post, LnParams head_ln, 
   const int64_t t = (static_cast<int64_t>(blockIdx.x) * kWarpsPerCta + (threadIdx.x >> 5)) * 2;
   if (t >= T) return;
   const bool two = t + 1 < T;
-  float x0[16], x1[16], z0[16], z1[16], w[16];
-  load_row(X + t * kC, lane, x0);
-  load_row(X + (two ? t + 1 : t) * kC, lane, x1);
+  float x0[C / 32], x1[C / 32], z0[C / 32], z1[C / 32], w[C / 32];
+  load_row(X + t * C, lane, x0);
+  load_row(X + (two ? t + 1 : t) * C, lane, x1);
   layernorm_2rows(x0, x1, post.gamma, post.beta, nullptr, 1e-6f, lane, z0, z1);
   layernorm_2rows(z0, z1, head_ln.gamma, head_ln.beta, nullptr, 1e-5f, lane, x0, x1);
   float o0[3], o1[3];
 #pragma unroll
   for (int k = 0; k < 3; ++k) {
-    load_row_ldg(wh + k * kC, lane, w);
+    load_row_ldg(wh + k * C, lane, w);
     float d0 = 0.f, d1 = 0.f;
 #pragma unroll
-    for (int i = 0; i < 16; ++i) { d0 = fmaf(x0[i], w[i], d0); d1 = fmaf(x1[i], w[i], d1); }
+    for (int i = 0; i < C / 32; ++i) { d0 = fmaf(x0[i], w[i], d0); d1 = fmaf(x1[i], w[i], d1); }
     const float bk = __ldg(bh + k);
     o0[k] = warp_sum(d0) + bk;
     o1[k] = warp_sum(d1) + bk;
@@ -695,65 +715,77 @@ cudaError_t launch_sf_rows(const uint8_t* sf, uint8_t* out, int64_t rows, int K,
   sf_rows_kernel<<<flat_grid(n), 256, 0, st>>>(sf, out, n, K);
   return cudaGetLastError();
 }
-cudaError_t launch_lift_ln(const float* x2d, const float* y, const float* x5, const float* wf_t, const float* bf,
+// The (C, FMT) instantiation of a row-wise kernel: every operand format at C = 512, the shipped FMT_F4C at C = 256.
+inline bool rowwise_built(int C, int fmt) { return C == 512 || (C == 256 && fmt == FMT_F4C); }
+#define D3D_ROWWISE_PICK(KERN)                                                                                          \
+  (C == 256 ? KERN<256, FMT_F4C> : fmt == FMT_F4C ? KERN<512, FMT_F4C> : fmt == FMT_F8C ? KERN<512, FMT_F8C> \
+                                                                                 : KERN<512, FMT_SPLIT16>)
+
+cudaError_t launch_lift_ln(int C, const float* x2d, const float* y, const float* x5, const float* wf_t, const float* bf,
                            const float* spos, const float* tvec, int64_t tvec_stride, LnParams ln1, float* X,
                            __half* a_hi, __half* a_lo, uint8_t* a_sf, int fmt, int64_t T, int J, int tokens_per_clip,
                            cudaStream_t st) {
   if (T <= 0) return cudaSuccess;
-  if (T > 0x7fffffffLL) return cudaErrorInvalidValue;
+  if (T > 0x7fffffffLL || !rowwise_built(C, fmt)) return cudaErrorInvalidValue;
   if ((!tvec || tvec_stride == 0) && rows_per_warp() == 2) {
-    auto k2 = fmt == FMT_F4C ? lift_ln2_kernel<FMT_F4C> : fmt == FMT_F8C ? lift_ln2_kernel<FMT_F8C> : lift_ln2_kernel<FMT_SPLIT16>;
+    auto k2 = D3D_ROWWISE_PICK(lift_ln2_kernel);
     k2<<<row_grid((T + 1) / 2), kWarpsPerCta * 32, 0, st>>>(x2d, y, x5, wf_t, bf, spos, tvec, ln1, X, a_hi, a_lo, a_sf, T, J);
     return cudaGetLastError();
   }
-  auto kern = fmt == FMT_F4C ? lift_ln_kernel<FMT_F4C> : fmt == FMT_F8C ? lift_ln_kernel<FMT_F8C> : lift_ln_kernel<FMT_SPLIT16>;
+  auto kern = D3D_ROWWISE_PICK(lift_ln_kernel);
   kern<<<row_grid(T), kWarpsPerCta * 32, 0, st>>>(x2d, y, x5, wf_t, bf, spos, tvec, tvec_stride, ln1, X, a_hi, a_lo, a_sf, T,
                                                  J, tokens_per_clip);
   return cudaGetLastError();
 }
-cudaError_t launch_postnorm_add_ln(float* X, LnParams post, const float* tpos, const float* tvec,
+cudaError_t launch_postnorm_add_ln(int C, float* X, LnParams post, const float* tpos, const float* tvec,
                                    int64_t tvec_stride, LnParams ln1, __half* a_hi, __half* a_lo, uint8_t* a_sf, int fmt,
                                    int64_t T, int J, int F, cudaStream_t st) {
   if (T <= 0) return cudaSuccess;
-  if (T > 0x7fffffffLL) return cudaErrorInvalidValue;
+  if (T > 0x7fffffffLL || !rowwise_built(C, fmt)) return cudaErrorInvalidValue;
   if (!tpos && (!tvec || tvec_stride == 0) && rows_per_warp() == 2) {       // eval: no per-row additive term
-    auto k2 = fmt == FMT_F4C ? postnorm_add_ln2_kernel<FMT_F4C>
-            : fmt == FMT_F8C ? postnorm_add_ln2_kernel<FMT_F8C> : postnorm_add_ln2_kernel<FMT_SPLIT16>;
+    auto k2 = D3D_ROWWISE_PICK(postnorm_add_ln2_kernel);
     k2<<<row_grid((T + 1) / 2), kWarpsPerCta * 32, 0, st>>>(X, post, tvec, ln1, a_hi, a_lo, a_sf, T);
     return cudaGetLastError();
   }
-  auto kern = fmt == FMT_F4C ? postnorm_add_ln_kernel<FMT_F4C>
-            : fmt == FMT_F8C ? postnorm_add_ln_kernel<FMT_F8C> : postnorm_add_ln_kernel<FMT_SPLIT16>;
+  auto kern = D3D_ROWWISE_PICK(postnorm_add_ln_kernel);
   kern<<<row_grid(T), kWarpsPerCta * 32, 0, st>>>(X, post, tpos, tvec, tvec_stride, ln1, a_hi, a_lo, a_sf, T, J, F);
   return cudaGetLastError();
 }
-cudaError_t launch_ln_split(const float* X, LnParams ln, float eps, __half* a_hi, __half* a_lo, uint8_t* a_sf, int fmt,
-                            int64_t T, cudaStream_t st) {
+cudaError_t launch_ln_split(int C, const float* X, LnParams ln, float eps, __half* a_hi, __half* a_lo, uint8_t* a_sf,
+                            int fmt, int64_t T, cudaStream_t st) {
   if (T <= 0) return cudaSuccess;
+  if (!rowwise_built(C, fmt)) return cudaErrorInvalidValue;
   if (rows_per_warp() == 2) {
-    auto k2 = fmt == FMT_F4C ? ln_split2_kernel<FMT_F4C> : fmt == FMT_F8C ? ln_split2_kernel<FMT_F8C> : ln_split2_kernel<FMT_SPLIT16>;
+    auto k2 = D3D_ROWWISE_PICK(ln_split2_kernel);
     k2<<<row_grid((T + 1) / 2), kWarpsPerCta * 32, 0, st>>>(X, ln, eps, a_hi, a_lo, a_sf, T);
     return cudaGetLastError();
   }
-  auto kern = fmt == FMT_F4C ? ln_split_kernel<FMT_F4C> : fmt == FMT_F8C ? ln_split_kernel<FMT_F8C> : ln_split_kernel<FMT_SPLIT16>;
+  auto kern = D3D_ROWWISE_PICK(ln_split_kernel);
   kern<<<row_grid(T), kWarpsPerCta * 32, 0, st>>>(X, ln, eps, a_hi, a_lo, a_sf, T);
   return cudaGetLastError();
 }
-cudaError_t launch_ln_f32(const float* x, LnParams ln, float eps, float* out, int64_t T, cudaStream_t st) {
+#undef D3D_ROWWISE_PICK
+cudaError_t launch_ln_f32(int C, const float* x, LnParams ln, float eps, float* out, int64_t T, cudaStream_t st) {
   if (T <= 0) return cudaSuccess;
-  ln_f32_kernel<<<row_grid(T), kWarpsPerCta * 32, 0, st>>>(x, ln, eps, out, T);
+  if (!width_supported(C)) return cudaErrorInvalidValue;
+  auto kern = C == 256 ? ln_f32_kernel<256> : ln_f32_kernel<512>;
+  kern<<<row_grid(T), kWarpsPerCta * 32, 0, st>>>(x, ln, eps, out, T);
   return cudaGetLastError();
 }
-cudaError_t launch_head_ddim(const float* X, LnParams post, LnParams head_ln, const float* wh, const float* bh,
+cudaError_t launch_head_ddim(int C, const float* X, LnParams post, LnParams head_ln, const float* wh, const float* bh,
                              DdimStep s, float* y, const float* noise, float* out3, float* trace_y, float* trace_x0,
                              int trace_stride, int trace_idx, int64_t T, cudaStream_t st) {
   if (T <= 0) return cudaSuccess;
-  if (rows_per_warp() == 2)
-    head_ddim2_kernel<<<row_grid((T + 1) / 2), kWarpsPerCta * 32, 0, st>>>(X, post, head_ln, wh, bh, s, y, noise, out3, trace_y,
-                                                                          trace_x0, trace_stride, trace_idx, T);
-  else
-    head_ddim_kernel<<<row_grid(T), kWarpsPerCta * 32, 0, st>>>(X, post, head_ln, wh, bh, s, y, noise, out3, trace_y,
-                                                               trace_x0, trace_stride, trace_idx, T);
+  if (!width_supported(C)) return cudaErrorInvalidValue;
+  if (rows_per_warp() == 2) {
+    auto kern = C == 256 ? head_ddim2_kernel<256> : head_ddim2_kernel<512>;
+    kern<<<row_grid((T + 1) / 2), kWarpsPerCta * 32, 0, st>>>(X, post, head_ln, wh, bh, s, y, noise, out3, trace_y, trace_x0,
+                                                             trace_stride, trace_idx, T);
+  } else {
+    auto kern = C == 256 ? head_ddim_kernel<256> : head_ddim_kernel<512>;
+    kern<<<row_grid(T), kWarpsPerCta * 32, 0, st>>>(X, post, head_ln, wh, bh, s, y, noise, out3, trace_y, trace_x0,
+                                                   trace_stride, trace_idx, T);
+  }
   return cudaGetLastError();
 }
 cudaError_t launch_tta_merge(const float* y, const float* yf, const int32_t* perm, float scale, float* out,

@@ -1,5 +1,5 @@
 // G-temb: sinusoidal time embedding and the tiny time MLPs (MODEL:29-36, 169-174, 104-116).
-// At eval every clip of a DDIM step shares one t (DIFF:254), so the whole [S, 2*depth, 512] table of
+// At eval every clip of a DDIM step shares one t (DIFF:254), so the whole [S, 2*depth, C] table of
 // per-block time vectors is computed once per (weights, schedule); the same kernels serve the general
 // per-sample-t path of forward_denoise.  Work is O(R * 10 MFLOP): fp32 CUDA cores, one warp per output.
 #include "kernels.cuh"
@@ -7,18 +7,20 @@
 namespace d3d {
 namespace {
 
+template <int C>
 __global__ void sincos_kernel(const float* __restrict__ t, int R, float* __restrict__ out) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;      // over R * 256
-  if (i >= R * 256) return;
-  const int r = i / 256, k = i % 256;
-  // freq_k = exp(k * -(ln(1e4)/255)) evaluated like torch does in fp32: the product k * (-step) is rounded to
+  constexpr int kHalf = C / 2;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;      // over R * C / 2
+  if (i >= R * kHalf) return;
+  const int r = i / kHalf, k = i % kHalf;
+  // freq_k = exp(k * -(ln(1e4)/(half_dim - 1))) evaluated like torch does in fp32: the product k * (-step) is rounded to
   // fp32, exp is correctly rounded from double; arg = t * freq in fp32; sin/cos correctly rounded from double.
-  const float step = static_cast<float>(9.210340371976184 / 255.0);   // math.log(10000) / (half_dim - 1)
+  const float step = static_cast<float>(9.210340371976184 / (kHalf - 1.0));   // math.log(10000) / (half_dim - 1)
   const float e = __fmul_rn(static_cast<float>(k), -step);
   const float freq = static_cast<float>(exp(static_cast<double>(e)));
   const float arg = __fmul_rn(t[r], freq);
-  out[r * 512 + k] = static_cast<float>(sin(static_cast<double>(arg)));
-  out[r * 512 + 256 + k] = static_cast<float>(cos(static_cast<double>(arg)));
+  out[r * C + k] = static_cast<float>(sin(static_cast<double>(arg)));
+  out[r * C + kHalf + k] = static_cast<float>(cos(static_cast<double>(arg)));
 }
 
 // per-sample timesteps of forward_denoise (int64 on the device, MODEL:33 multiplies them into fp32) -> fp32
@@ -64,9 +66,11 @@ cudaError_t launch_t_to_f32(const int64_t* t, int R, float* out, cudaStream_t st
   return cudaGetLastError();
 }
 
-cudaError_t launch_sincos(const float* t, int R, float* out, cudaStream_t st) {
+cudaError_t launch_sincos(int C, const float* t, int R, float* out, cudaStream_t st) {
   if (R <= 0) return cudaSuccess;
-  sincos_kernel<<<(R * 256 + 255) / 256, 256, 0, st>>>(t, R, out);
+  if (!width_supported(C)) return cudaErrorInvalidValue;
+  if (C == 256) sincos_kernel<256><<<(R * 128 + 255) / 256, 256, 0, st>>>(t, R, out);
+  else sincos_kernel<512><<<(R * 256 + 255) / 256, 256, 0, st>>>(t, R, out);
   return cudaGetLastError();
 }
 

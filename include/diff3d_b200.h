@@ -73,10 +73,12 @@ enum {
 typedef struct d3d_config {
   int32_t num_frame;     /* F: 27 / 81 / 243 (any 1..256)           */
   int32_t num_joints;    /* J: 17                                     */
-  int32_t embed_dim;     /* C: 512 (kernels are specialised for 512)  */
+  int32_t embed_dim;     /* C: 512 or 256 (the kernels are instantiated
+                            for both widths; 256 runs D3D_GEMM_TC_F4C +
+                            D3D_ATTN_DEFAULT with 17 joints only)     */
   int32_t depth;         /* spatial/temporal block pairs: 8           */
-  int32_t num_heads;     /* 8 (head_dim 64)                           */
-  int32_t mlp_hidden;    /* int(C * mlp_ratio): 1024                  */
+  int32_t num_heads;     /* 8 (head_dim C / 8: 64 or 32)              */
+  int32_t mlp_hidden;    /* int(C * mlp_ratio) = 2 C: 1024 or 512     */
   int32_t with_time_emb; /* 0/1 (MODEL:163-177)                       */
   int32_t max_clips;     /* workspace capacity in clips (B)           */
   int32_t gemm_mode;     /* D3D_GEMM_*                                */
@@ -196,8 +198,9 @@ D3D_API int d3d_mpjpe_accumulate(d3d_handle* h, const float* pred_dev, const flo
 D3D_API int64_t d3d_launch_count(const d3d_handle* h);
 
 /* Device bytes the handle owns (packed weights, activation workspace, time tables, sampler state): everything is
- * allocated in d3d_create / d3d_set_schedule, nothing on the hot path (SURVEY.md 8b `d3d_workspace_bytes`).  16 KB per
- * token of max_clips * num_frame * num_joints + ~100 MB of weights: 34 GB for 512 clips of 243 frames. */
+ * allocated in d3d_create / d3d_set_schedule, nothing on the hot path (SURVEY.md 8b `d3d_workspace_bytes`).  About 32 C
+ * bytes (16 KB at C = 512, 8 KB at C = 256) per token of max_clips * num_frame * num_joints + the weights (~100 MB at
+ * C = 512): 34 GB for 512 clips of 243 frames at C = 512. */
 D3D_API int64_t d3d_workspace_bytes(const d3d_handle* h);
 
 /* Per-kernel-class device timing.  Between d3d_profile_begin and d3d_profile_end every kernel of the sampler /
@@ -228,7 +231,7 @@ D3D_API int d3d_op_linear(d3d_handle* h, const float* a_dev, const float* w_dev,
 D3D_API int d3d_op_linear_bench(d3d_handle* h, int64_t M, int32_t N, int32_t K, int32_t act, int32_t gemm_mode,
                         int32_t iters, float* ms_per_launch);
 
-/* LayerNorm over the last dim (512): out = (x-mean)*rstd*gamma+beta (MODEL:184,218).  The per-row arithmetic is the
+/* LayerNorm over the last dim (C): out = (x-mean)*rstd*gamma+beta (MODEL:184,218).  The per-row arithmetic is the
  * one of the hot path's row-wise kernels (two-pass variance, rsqrt + one Newton step, packed fp32 pairs), so `out` is
  * bit for bit the fp32 LayerNorm those kernels quantise into a GEMM operand. */
 D3D_API int d3d_op_layernorm(d3d_handle* h, const float* x_dev, const float* gamma_dev, const float* beta_dev, float eps,
